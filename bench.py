@@ -17,6 +17,7 @@ shard's result recomputed on rank 0's GPU alone.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          # our CUDA path
   python bench.py --impl reference ...                         # CPU restatement of the reference, same workload
+  python bench.py ... --dump-outputs DIR                       # also save the last timed step's H, b, sum as DIR/*.npy
 Multi-GPU: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 Prints ONE JSON line on rank 0.
 """
@@ -79,7 +80,21 @@ def parse():
     ap.add_argument("--strong-total", type=int, default=-1,
                     help="N>1: second timed region, this many correspondences in total sharded contiguously over the "
                          "ranks (BASELINE configs[3]); default 1e9 when N>1, 0 disables")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (H, b, sum r^T r of the headline workload) as "
+                         "DIR/H.npy, DIR/b.npy, DIR/sum_rtr.npy (float64), so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(directory, H, b, s):
+    """--dump-outputs: the arrays a caller of the timed path receives from its last step.  The inputs are the seeded
+    generator's rows, so the same arguments give the same inputs in every run."""
+    os.makedirs(directory, exist_ok=True)
+    for name, v in (("H", H), ("b", b), ("sum_rtr", s)):
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def workload_config(n_per_gpu: int, n_total: int) -> dict:
@@ -242,10 +257,9 @@ def run_reference(args):
     if rank != 0:
         return
     from oracle import oracle_py as orc
-    orc.build()
     cores = orc.hardware_concurrency() or (os.cpu_count() or 1)
     n_full = args.n
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     # a quick probe decides whether the full per-GPU workload fits the time budget
     probe_n = min(n_full, 2_000_000)
     ps, pt = orc.generate_p2p(SEED, probe_n, X_GT, **GEN)
@@ -261,6 +275,8 @@ def run_reference(args):
     if warmup:
         orc.time_linearize(cost, x0, nthreads=cores, reps=warmup)
     t, H, b, s = orc.time_linearize(cost, x0, nthreads=cores, reps=steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, H, b, s)
     ms = t / steps * 1e3
     value = n / (t / steps) / 1e9
     sample = (f"{n} correspondences per step (fp64 AoS, the first rows of rank 0's shard"
@@ -504,6 +520,8 @@ def run_ours(args):
     sampler.mark()
     sampler.stop()
     H, b, s = ctx.result(6)
+    if rank == 0 and args.dump_outputs:  # every rank holds the same exchanged result
+        dump_outputs(args.dump_outputs, H, b, s)
     # diagnostics for N > 1: every rank's own pass time with the exchange switched off (no lock-step coupling);
     # the gap between max(local) and the coupled step is what the collective + straggling cost
     local_ms = None
@@ -702,7 +720,6 @@ def run_ours(args):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         from oracle import oracle_py as orc
-        orc.build()
         m = min(args.cpu_sample, n)
         src = store.download(0, np.float64, 0, m)
         tgt = store.download(1, np.float64, 0, m)

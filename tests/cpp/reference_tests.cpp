@@ -2,7 +2,9 @@
 // call sequences (moptimizer::CostFunction*{,Dynamic}, CostComputation, LevenbergMarquadtDynamic) with the
 // builtin device models in place of the test-defined host models.  Each TEST cites the reference test.
 #include <cmath>
+#include <cstdlib>
 #include <memory>
+#include <string>
 #include <vector>
 
 #include "fixtures.h"
@@ -430,8 +432,16 @@ TEST(Registration, UpdateHookReassociatesCorrespondences) {
 
 TEST(Ingest, TextCloudFeedsTheDeviceStore) {
   P2PFixture f;
-  const char* path = "/tmp/mopt_cpp_cloud.txt";
-  FILE* out = std::fopen(path, "w");
+  // a file of its own: a fixed name in a shared temporary directory may belong to another user or another run
+  const char* tmpdir = std::getenv("TMPDIR");
+  std::string tmpl = std::string(tmpdir && *tmpdir ? tmpdir : "/tmp") + "/mopt_cpp_cloud_XXXXXX";
+  std::vector<char> name(tmpl.begin(), tmpl.end());
+  name.push_back('\0');
+  const int fd = mkstemp(name.data());
+  FILE* out = fd >= 0 ? fdopen(fd, "w") : nullptr;
+  EXPECT_TRUE(out != nullptr);
+  if (out == nullptr) return;
+  const char* path = name.data();
   for (int i = 0; i < f.n; ++i)
     std::fprintf(out, "%.8f %.8f %.8f %d %d %d\n", f.src[i * 3], f.src[i * 3 + 1], f.src[i * 3 + 2], i % 256, 7, 0);
   std::fclose(out);

@@ -42,6 +42,56 @@ def test_reference_arm_other_ranks_stay_silent():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_reference_arm_dump_outputs(tmp_path):
+    """--dump-outputs writes the last timed step's H, b and sum r^T r; the seeded inputs make two runs agree."""
+    import numpy as np
+    dumps = []
+    for k in range(2):
+        d = tmp_path / f"run{k}"
+        r = run_bench("--impl", "reference", "--steps", "2", "--warmup", "0", "--n", "30000", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+        assert sorted(os.listdir(d)) == ["H.npy", "b.npy", "sum_rtr.npy"]
+        out = {name: np.load(d / f"{name}.npy") for name in ("H", "b", "sum_rtr")}
+        assert out["H"].shape == (6, 6) and out["b"].shape == (6,) and out["sum_rtr"].shape == ()
+        assert all(v.dtype == np.float64 for v in out.values())
+        assert out["H"][0, 0] == line["check"]["H00"] and out["b"][0] == line["check"]["b0"]
+        assert float(out["sum_rtr"]) == line["check"]["sum_rtr"]
+        dumps.append(out)
+    assert all(np.array_equal(dumps[0][k], dumps[1][k]) for k in dumps[0])
+
+
+def test_steps_must_be_positive():
+    r = run_bench("--impl", "reference", "--steps", "0", "--n", "1000")
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
+@pytest.mark.gpu
+def test_cuda_arm_dump_outputs(tmp_path):
+    """The CUDA arm's dump is the result of the timed pass: the same rows linearized again give the same H, b, sum."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from moptimizer_0_b200 import capi
+    from tests.common import rel_err
+    n, steps = 1_000_003, 7
+    r = run_bench("--steps", str(steps), "--warmup", "1", "--prewarm-steps", "10", "--n", str(n), "--no-cpu-baseline",
+                  "--no-e2e", "--no-configs", "--no-peaks", "--no-lm", "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+    assert line["steps"] == steps and line["gpu_launches"] == steps
+    H, b, s = (np.load(tmp_path / f"{name}.npy") for name in ("H", "b", "sum_rtr"))
+    ctx = capi.Context(0)
+    st = capi.Store(ctx, capi.MODEL_POINT2POINT, n, capi.F32)
+    st.generate(seed=bench.SEED, gt=bench.X_GT, **bench.GEN)
+    prob = capi.make_problem(capi.MODEL_POINT2POINT, capi.JAC_ANALYTICAL, capi.F32, loss=capi.LOSS_HUBER,
+                             loss_param=bench.HUBER_K, variant=capi.P2P_EXACT)
+    He, be, se = ctx.linearize(st, prob, np.zeros(6))
+    st.close()
+    ctx.close()
+    assert rel_err(H, He) < 1e-12 and rel_err(b, be) < 1e-12 and abs(float(s) - se) <= 1e-12 * se
+
+
 def test_cuda_arm_refuses_to_run_without_a_gpu():
     import torch
     if torch.cuda.is_available():
