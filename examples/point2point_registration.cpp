@@ -51,6 +51,10 @@ int main(int argc, char** argv) {
     for (int i = 0; i < 6; ++i) err = std::fmax(err, std::fabs(x0[i] - x_gt[i]));
     std::printf("status %d after %d iterations, x = (%.5f %.5f %.5f %.5f %.5f %.5f), max |x - x_gt| = %.2e\n", int(status),
                 lm.getExecutedIterations(), x0[0], x0[1], x0[2], x0[3], x0[4], x0[5], err);
+    // registration quality at the solution: correspondences within 3 noise sigmas (0.03) of their target
+    const mopt_eval_stats fit = cost.evaluateStatistics(x0, 0.03);
+    std::printf("fitness %.4f (%lld of %ld residuals within 0.03), inlier RMSE %.5f\n", double(fit.n_inliers) / double(n),
+                (long long)fit.n_inliers, n, fit.n_inliers ? std::sqrt(fit.inlier_sum_sq / double(fit.n_inliers)) : 0.0);
     return err < 1e-3 ? 0 : 1;
   } catch (const moptimizer::Exception& e) {
     std::printf("moptimizer::Exception: %s\n", e.what());

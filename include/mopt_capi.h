@@ -268,6 +268,38 @@ MOPT_API int mopt_compute_cost(mopt_ctx* ctx, mopt_store* store, const mopt_prob
 MOPT_API int mopt_linearize_async(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x);
 MOPT_API int mopt_ctx_result(mopt_ctx* ctx, int num_parameters, double* H, double* b, double* sum);
 
+/* ---- per-residual evaluation ------------------------------------------------------------------ */
+/* Fit statistics of one cost term over a range of its store (mopt_evaluate).  Counts and sums add across the
+ * ranks of a sharded problem and max_sq combines by maximum: each rank evaluates its own store only. */
+typedef struct mopt_eval_stats {
+  int64_t n_valid;        /* elements of the range whose residual exists (not masked, see mopt_evaluate) */
+  int64_t n_inliers;      /* valid elements with r^T r <= inlier_threshold^2 */
+  double sum_sq;          /* sum of r^T r over valid elements: mopt_compute_cost's value over the same range */
+  double inlier_sum_sq;   /* sum of r^T r over inliers */
+  double max_sq;          /* max r^T r over valid elements (0 if none) */
+  double reserved[3];
+} mopt_eval_stats;
+
+/* CostComputation::computeCost's loop body (linearization.h:36-47) with each element's result kept:
+ * for the elements [first, first + count) of `store` at x, optionally write the residual r_i (count x O,
+ * row-major: element i's O components are contiguous) and the loss weight w_i = loss(r_i^T r_i), both in
+ * `out_dtype`, to DEVICE memory on the context's device.  `residuals`, `weights` and `stats` may each be NULL,
+ * but not all three.  Returns after the context stream is synchronised.
+ *   - r_i is the model residual in problem.compute_dtype arithmetic at setup(x); w_i is the IRLS weight the pass
+ *     kernels apply.  The covariance, jacobian, variant and manifold fields have no effect.
+ *   - Elements without a correspondence (point2point stores with an attached target index, see
+ *     mopt_store_reassociate) get NaN in every residual component and weight 0, and enter no statistic.
+ *   - Evaluation never re-associates: a store with a target index is evaluated with the correspondences it holds
+ *     now.  Call mopt_store_reassociate(store, x) first to evaluate at fresh correspondences.
+ *   - Statistics are accumulated in fp64 and reduced in a fixed order: identical bits from run to run, whichever
+ *     outputs are written.  inlier_threshold = +inf counts every valid element as an inlier.
+ *   - Sharded contexts: this rank's store only, no collective (see mopt_eval_stats).
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for a range outside the store, out_dtype not MOPT_F32 /
+ * MOPT_F64, residuals or weights with count 0, or all three outputs NULL. */
+MOPT_API int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x,
+                           int64_t first, int64_t count, double inlier_threshold, int out_dtype,
+                           void* residuals, void* weights, mopt_eval_stats* stats);
+
 /* End-to-end convenience: upload host AoS data (group A and B) into `store` and linearize, with the
  * host->device copies chunked and overlapped with the device work. */
 MOPT_API int mopt_upload_and_linearize(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const void* host_a,

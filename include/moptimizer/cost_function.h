@@ -52,6 +52,24 @@ class CostFunctionBase {
   /// is not a builtin device model or the loss is not one the kernels implement: there is no host fallback.
   virtual void deviceProblem(mopt_problem* problem, device::Store::Ptr* store) const = 0;
 
+  /// New: fit statistics of this cost term at x over all its residuals (mopt_evaluate without per-element outputs):
+  /// valid residuals, inliers (r^T r <= inlier_threshold^2), sum r^T r, its inlier part and max r^T r.  Fitness is
+  /// n_inliers / residual count, inlier RMSE sqrt(inlier_sum_sq / n_inliers).  Correspondences are not re-associated:
+  /// call update(x) first for fresh ones.  Per-element residuals and weights live in device memory only, so they
+  /// are read through the C ABI (mopt_evaluate on deviceProblem()'s store) by a caller that owns device buffers.
+  mopt_eval_stats evaluateStatistics(const Scalar* x, double inlier_threshold) const {
+    mopt_problem p;
+    device::Store::Ptr st;
+    deviceProblem(&p, &st);
+    double xd[MOPT_MAX_PARAMETERS] = {0};
+    for (int i = 0; i < p.num_parameters && x; ++i) xd[i] = double(x[i]);
+    mopt_eval_stats stats;
+    device::check(mopt_evaluate(st->context()->get(), st->get(), &p, xd, 0, st->size(), inlier_threshold, MOPT_F64,
+                                nullptr, nullptr, &stats),
+                  "mopt_evaluate");
+    return stats;
+  }
+
  protected:
   void fillDeviceProblem(int num_parameters, int num_outputs, int jacobian, mopt_problem* p,
                          device::Store::Ptr* store) const {

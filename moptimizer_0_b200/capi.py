@@ -46,7 +46,7 @@ EXPORTS = [
     "mopt_nn_index_create", "mopt_nn_index_destroy", "mopt_store_set_target", "mopt_store_reassociate",
     "mopt_ctx_peer_handle", "mopt_ctx_open_peers", "mopt_ctx_set_exchange_enabled",
     "mopt_user_model_compile", "mopt_user_model_release", "mopt_user_model_log",
-    "mopt_measure_peaks", "mopt_measure_h2d",
+    "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate",
 ]
 MODEL_USER_BASE = 1000
 PEER_HANDLE_BYTES = 64
@@ -99,6 +99,14 @@ class Peaks(C.Structure):
                 ("issue_gwarp_inst_per_s", C.c_double), ("hbm_read_gbs", C.c_double), ("reserved", C.c_double * 4)]
 
 
+class EvalStats(C.Structure):
+    _fields_ = [("n_valid", C.c_int64), ("n_inliers", C.c_int64), ("sum_sq", C.c_double),
+                ("inlier_sum_sq", C.c_double), ("max_sq", C.c_double), ("reserved", C.c_double * 3)]
+
+
+mopt_eval_stats = EvalStats  # the C name
+
+
 class MoptError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"mopt error {code}: {msg}")
@@ -137,6 +145,8 @@ def lib():
         L.mopt_linearize_async.argtypes = [vp, vp, C.POINTER(Problem), dp]
         L.mopt_ctx_result.argtypes = [vp, C.c_int, dp, dp, dp]
         L.mopt_measure_peaks.argtypes = [vp, C.POINTER(Peaks)]
+        L.mopt_evaluate.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_double, C.c_int, vp, vp,
+                                    C.POINTER(EvalStats)]
         L.mopt_measure_h2d.argtypes = [vp, C.c_uint64, C.c_double, dp]
         L.mopt_upload_and_linearize.argtypes = [vp, vp, C.POINTER(Problem), vp, vp, C.c_int, i64, dp, dp, dp, dp]
         L.mopt_lm_minimize.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), C.POINTER(LmOptions), dp,
@@ -227,6 +237,7 @@ class Context:
     """One GPU (mopt_ctx).  `sharded=(rank, world, unique_id_bytes)` joins a NCCL communicator."""
 
     def __init__(self, device: int = 0, sharded=None):
+        self.device = device
         self._h = C.c_void_p()
         if sharded is None:
             check(lib().mopt_ctx_create(device, C.byref(self._h)))
@@ -305,6 +316,40 @@ class Context:
         check(lib().mopt_compute_cost(self._h, store.handle, C.byref(problem), _dp(xs), C.byref(s)))
         return s.value
 
+    def evaluate(self, store: "Store", problem: Problem, x, first: int = 0, count: Optional[int] = None,
+                 inlier_threshold: float = float("inf"), residuals: bool = True, weights: bool = True,
+                 out_dtype: int = F32, out=None) -> "EvalResult":
+        """Per-residual evaluation (mopt_evaluate) of the elements [first, first + count) at x: residuals (count, O)
+        and loss weights (count,) as CUDA tensors on this context's device, plus fit statistics.  `out` =
+        (residuals, weights) supplies the output tensors (either may be None); they must be contiguous, on the
+        context's device, of `out_dtype` and of those shapes.  Never re-associates: call store_reassociate first
+        for fresh correspondences.  Elements without a correspondence get NaN residuals and weight 0."""
+        import torch
+        count = store.n - first if count is None else int(count)
+        O = problem.num_outputs
+        tdt = torch.float32 if out_dtype == F32 else torch.float64
+        dev = torch.device("cuda", self.device)
+        r_t = w_t = None
+        if out is not None:
+            r_t, w_t = out
+            for t, shape, name in ((r_t, (count, O), "residuals"), (w_t, (count,), "weights")):
+                if t is None:
+                    continue
+                if t.device != dev or t.dtype != tdt or tuple(t.shape) != shape or not t.is_contiguous():
+                    raise ValueError(f"out {name}: need a contiguous {tdt} tensor of shape {shape} on {dev}, got "
+                                     f"{t.dtype} {tuple(t.shape)} on {t.device}")
+        else:
+            if residuals:
+                r_t = torch.empty((count, O), dtype=tdt, device=dev)
+            if weights:
+                w_t = torch.empty((count,), dtype=tdt, device=dev)
+        xs = np.ascontiguousarray(np.asarray(x if len(x) else [0.0], dtype=np.float64))
+        st = EvalStats()
+        check(lib().mopt_evaluate(self._h, store.handle, C.byref(problem), _dp(xs), int(first), count,
+                                  float(inlier_threshold), out_dtype, r_t.data_ptr() if r_t is not None else None,
+                                  w_t.data_ptr() if w_t is not None else None, C.byref(st)))
+        return EvalResult(st, count, r_t, w_t)
+
     def linearize_async(self, store: "Store", problem: Problem, xs: np.ndarray):
         check(lib().mopt_linearize_async(self._h, store.handle, C.byref(problem), _dp(xs)))
 
@@ -347,6 +392,35 @@ class Context:
             rep = self._lm_report = LmReport()
         check(lib().mopt_lm_minimize(self._h, n, hs, ps, C.byref(opt), _dp(x), C.byref(rep)))
         return LmResult(x, rep)
+
+
+class EvalResult:
+    """Context.evaluate: `residuals` (count, O) / `weights` (count,) CUDA tensors (None when not requested),
+    `stats` (mopt_eval_stats as a dict) and the registration / calibration figures derived from it."""
+
+    def __init__(self, st: EvalStats, count: int, residuals, weights):
+        self.stats = {"n_valid": st.n_valid, "n_inliers": st.n_inliers, "sum_sq": st.sum_sq,
+                      "inlier_sum_sq": st.inlier_sum_sq, "max_sq": st.max_sq}
+        self.count = count
+        self.residuals = residuals
+        self.weights = weights
+
+    @property
+    def fitness(self) -> float:
+        """Fraction of the evaluated elements that are inliers (n_inliers / count)."""
+        return self.stats["n_inliers"] / self.count if self.count else 0.0
+
+    @property
+    def inlier_rmse(self) -> float:
+        """sqrt(inlier_sum_sq / n_inliers): RMS residual norm over the inliers."""
+        n = self.stats["n_inliers"]
+        return float(np.sqrt(self.stats["inlier_sum_sq"] / n)) if n else 0.0
+
+    @property
+    def rms(self) -> float:
+        """sqrt(sum_sq / n_valid): RMS residual norm over every valid element."""
+        n = self.stats["n_valid"]
+        return float(np.sqrt(self.stats["sum_sq"] / n)) if n else 0.0
 
 
 class LmResult:

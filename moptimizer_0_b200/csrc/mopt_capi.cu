@@ -318,6 +318,28 @@ int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int 
   return launch_dense(L, p->model, p->jacobian != MOPT_JAC_ANALYTICAL, st->dtype, p->compute_dtype, a);
 }
 
+// Per-residual evaluation (mopt_evaluate): the builtin or run-time compiled evaluate_kernel of the model, on set 0 of
+// slot 0 (staged by setup_slot), reducing its statistics through the same partials / ticket as the passes.
+int launch_eval(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int out_dtype, const EvalArgs& ev) {
+  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
+  if (p->model >= MOPT_MODEL_USER_BASE)
+    return launch_user_evaluate(L, ctx->device, p->model, st->dtype, p->compute_dtype, out_dtype, a, ev);
+  return launch_evaluate(L, p->model, st->dtype, p->compute_dtype, out_dtype, a, ev);
+}
+
+// An output of mopt_evaluate must be device memory the context's device can write.
+int check_device_output(const mopt_ctx* ctx, const void* ptr, const char* what) {
+  if (!ptr) return MOPT_OK;
+  cudaPointerAttributes attr;
+  const cudaError_t e = cudaPointerGetAttributes(&attr, ptr);
+  if (e != cudaSuccess) (void)cudaGetLastError();
+  MOPT_REQUIRE(e == cudaSuccess && (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged) &&
+                   attr.device == ctx->device,
+               std::string(what) + " must be device memory on the context's device");
+  return MOPT_OK;
+}
+
 int allreduce_trial(mopt_ctx* ctx, int P, int mode_override) {
   if (ctx->world <= 1 || !ctx->exchange_enabled) return MOPT_OK;
   if (ctx->peers_open) {
@@ -477,6 +499,7 @@ int ctx_alloc(mopt_ctx* ctx) {
   MOPT_CUDA_TRY(cudaMemset(ctx->d_gen, 0, 32 * sizeof(unsigned long long)));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_xerr_dev, sizeof(int)));
   MOPT_CUDA_TRY(cudaMemset(ctx->d_xerr_dev, 0, sizeof(int)));
+  MOPT_CUDA_TRY(cudaMalloc(&ctx->d_eval_stats, sizeof(double) * (kEvalSums + 1)));
   ctx->flags_capacity = 4096;
   if (const char* e = getenv("MOPT_LM_FLAG_RING")) {  // test knob: a small ring makes an ordinary solve wrap it
     const int v = atoi(e);
@@ -576,6 +599,7 @@ int mopt_ctx_destroy(mopt_ctx* ctx) try {
   cudaFree(ctx->d_xbuf);
   cudaFree(ctx->d_xerr_dev);
   cudaFree(ctx->d_gen);
+  cudaFree(ctx->d_eval_stats);
   if (ctx->h_xerr) cudaFreeHost(ctx->h_xerr);
   cudaFree(ctx->d_partials); cudaFree(ctx->d_ticket); cudaFree(ctx->d_trial);
   cudaFree(ctx->d_slots); cudaFree(ctx->d_lm);
@@ -677,6 +701,50 @@ int mopt_compute_cost(mopt_ctx* ctx, mopt_store* store, const mopt_problem* prob
   MOPT_TRY(validate_problem(store, problem, false));
   MOPT_TRY(enqueue_pass(ctx, store, problem, x, PASS_COST));
   return fetch_result(ctx, problem->num_parameters, nullptr, nullptr, sum);
+}
+MOPT_ABI_CATCH
+
+int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x, int64_t first,
+                  int64_t count, double inlier_threshold, int out_dtype, void* residuals, void* weights,
+                  mopt_eval_stats* stats) try {
+  MOPT_REQUIRE(ctx && store && store->ctx == ctx, "store does not belong to this context");
+  MOPT_TRY(validate_problem(store, problem, false));
+  MOPT_REQUIRE(first >= 0 && count >= 0 && first <= store->n && count <= store->n - first,
+               "the range [first, first + count) must lie inside the store");
+  MOPT_REQUIRE(out_dtype == MOPT_F32 || out_dtype == MOPT_F64, "out_dtype must be MOPT_F32 or MOPT_F64");
+  MOPT_REQUIRE(residuals || weights || stats, "residuals, weights and stats are all NULL: nothing to evaluate");
+  MOPT_REQUIRE(count > 0 || (!residuals && !weights), "residuals or weights requested for an empty range");
+  MOPT_REQUIRE(problem->num_parameters == 0 || x, "null parameter vector");
+  MOPT_REQUIRE(!(inlier_threshold < 0.0), "inlier_threshold must not be negative");
+  MOPT_CUDA_TRY(cudaSetDevice(ctx->device));
+  MOPT_TRY(check_device_output(ctx, residuals, "residuals"));
+  MOPT_TRY(check_device_output(ctx, weights, "weights"));
+  if (count == 0) {
+    std::memset(stats, 0, sizeof(*stats));
+    return MOPT_OK;
+  }
+  MOPT_TRY(setup_slot(ctx, 0, problem, x));
+  EvalArgs ev;
+  ev.first = first;
+  ev.count = count;
+  ev.r = residuals;
+  ev.w = weights;
+  ev.thr2 = inlier_threshold * inlier_threshold;
+  ev.stats = ctx->d_eval_stats;
+  MOPT_TRY(launch_eval(ctx, store, problem, out_dtype, ev));
+  double* h = ctx->h_result->v;  // pinned bounce buffer (idle between calls)
+  MOPT_CUDA_TRY(cudaMemcpyAsync(h, ctx->d_eval_stats, sizeof(double) * (kEvalSums + 1), cudaMemcpyDeviceToHost,
+                                ctx->stream));
+  MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  if (stats) {
+    std::memset(stats, 0, sizeof(*stats));
+    stats->n_valid = int64_t(h[0]);
+    stats->n_inliers = int64_t(h[1]);
+    stats->sum_sq = h[2];
+    stats->inlier_sum_sq = h[3];
+    stats->max_sq = h[4];
+  }
+  return MOPT_OK;
 }
 MOPT_ABI_CATCH
 

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include "mopt_common.cuh"
+#include "mopt_eval.cuh"
 #include "mopt_lm.cuh"
 #include "mopt_lm_mono.cuh"
 #include "mopt_models.cuh"
@@ -54,6 +55,7 @@ struct mopt_ctx {
   unsigned long long* d_gen = nullptr;           // persistent LM kernel: the 24 tagged words that carry (R, t) and act as its grid barrier (publish_rt)
   unsigned long long mono_gen = 0;               // barrier targets handed out so far (monotonic over the context's life)
   int* d_xerr_dev = nullptr;                     // device-resident copy, read by the kernels that follow a failed exchange
+  double* d_eval_stats = nullptr;                // mopt_evaluate: the statistics written by the evaluation kernel's last CTA
 };
 
 struct mopt_store {
@@ -97,9 +99,15 @@ int enqueue_reassociate(mopt_store* st, const ParamBlock* pb, const LmState* gat
 // mopt_pass_wide.cu
 int launch_wide(const PassLaunch& L, int model, int store_dtype, int compute_dtype, const PassArgs& a);
 
+// mopt_eval.cu: per-residual evaluation of a builtin model (mopt_evaluate)
+int launch_evaluate(const PassLaunch& L, int model, int store_dtype, int compute_dtype, int out_dtype,
+                    const PassArgs& a, const EvalArgs& ev);
+
 // mopt_rtc.cu: run-time compiled user models (ids >= MOPT_MODEL_USER_BASE)
 int launch_user(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
                 const PassArgs& a);
+int launch_user_evaluate(const PassLaunch& L, int device, int model, int store_dtype, int compute_dtype, int out_dtype,
+                         const PassArgs& a, const EvalArgs& ev);
 int launch_user_setup(cudaStream_t stream, int device, int model, CostSlot* slot, const double* x_dev,
                       const double* x_host, int P);
 int user_model_rot_offset(int model);
