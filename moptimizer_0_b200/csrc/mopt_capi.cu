@@ -4,7 +4,6 @@
 
 #include <cmath>
 #include <atomic>
-#include <chrono>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -89,11 +88,9 @@ __global__ void lm_init_kernel(LmState* st, CostSlot* slots, LmInit in) {
   lm_init_warp(st, slots, in, &s_sh, threadIdx.x);
 }
 
-__device__ long long g_step_prof[8];  // MOPT_LM_MONO_TRACE=1: clock64 stamps of the last solving lm_step_kernel
-
 // One optimizer transition between passes; also publishes the done flag of this slot to the host.
-__global__ void lm_step_kernel(LmState* st, const PassResult* trial, CostSlot* slots, int* flag, const int* xerr, int prof,
-                               int P, int scalar_f32) {
+__global__ void lm_step_kernel(LmState* st, const PassResult* trial, CostSlot* slots, int* flag, const int* xerr, int P,
+                               int scalar_f32) {
   __shared__ LmStepShared s_sh;
   const int lane = threadIdx.x;
   if (*reinterpret_cast<const volatile int*>(xerr)) {  // a peer exchange timed out: `trial` is not a total
@@ -103,13 +100,8 @@ __global__ void lm_step_kernel(LmState* st, const PassResult* trial, CostSlot* s
     }
     return;
   }
-  long long stamps[16] = {0};
-  const int done = lm_step_warp(st, trial, slots, &s_sh, lane, P, scalar_f32 != 0, LmStepIo{}, prof ? stamps : nullptr);
-  if (lane == 0) {
-    *flag = done;
-    if (prof && stamps[3] - stamps[2] > 1000)  // a transition that solved
-      for (int i = 0; i < 6; ++i) g_step_prof[i] = stamps[i];
-  }
+  const int done = lm_step_warp(st, trial, slots, &s_sh, lane, P, scalar_f32 != 0, LmStepIo{});
+  if (lane == 0) *flag = done;
 }
 
 // The same solve through the warp-cooperative LDL^T (mopt_ldlt_solve with cooperative = 1; for tests).
@@ -855,13 +847,11 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
   }
 
   // Small single-cost point2point problems on one GPU: the whole loop in ONE cooperative launch (mopt_lm_mono.cuh);
-  // MOPT_LM_MONO=0 in the environment keeps the launch-per-trial path (A/B), MOPT_LM_MONO_MAX overrides the size limit.
+  // up to 2^22 residuals.  MOPT_LM_MONO=0 in the environment keeps the launch-per-trial path (A/B).
   {
     static const int64_t mono_max = [] {
       const char* e = getenv("MOPT_LM_MONO");
-      if (e && e[0] == '0') return int64_t(0);
-      const char* m = getenv("MOPT_LM_MONO_MAX");
-      return (m && m[0]) ? int64_t(atoll(m)) : int64_t(1) << 22;
+      return (e && e[0] == '0') ? int64_t(0) : int64_t(1) << 22;
     }();
     const mopt_problem& p0 = problems[0];
     const bool moment_path = p0.model == MOPT_MODEL_POINT2POINT &&
@@ -876,8 +866,6 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
       m.host_st = ctx->d_lm_host;
       m.host_flag = ctx->d_flags;  // word 0 of the mapped flag ring (idle: this path and the launch-per-trial path exclude each other)
       reinterpret_cast<volatile int*>(ctx->h_flags)[0] = 0;
-      static const int generic_p = [] { const char* e = getenv("MOPT_LM_GENERIC_P"); return (e && e[0] == '1') ? 1 : 0; }();
-      m.generic_p = generic_p;
       ctx->h_lm->done = 0;
       m.slots = ctx->d_slots;
       m.rt_words = ctx->d_gen;
@@ -886,66 +874,25 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
       m.init = in;  // prepare() + the first setup(x0) run inside the kernel too (CTA 0, before the first pass)
       m.gen_base = ctx->mono_gen;
       ctx->mono_gen += (unsigned long long)(m.max_slots) + 2ull;
-      m.dbg = nullptr;
-      static const bool trace = [] { const char* e = getenv("MOPT_LM_MONO_TRACE"); return e && e[0] == '1'; }();
-      unsigned long long* d_dbg = nullptr;
-      if (trace) {  // diagnostics: where a trial's time goes inside the persistent kernel (printed to stderr)
-        MOPT_CUDA_TRY(cudaMalloc(&d_dbg, sizeof(unsigned long long) * 512));
-        MOPT_CUDA_TRY(cudaMemsetAsync(d_dbg, 0, sizeof(unsigned long long) * 512, ctx->stream));
-        m.dbg = d_dbg;
-      }
       const bool qrot = p0.jacobian == MOPT_JAC_ANALYTICAL && (p0.variant == MOPT_P2P_EXACT || p0.variant == MOPT_P2P_LEFT);
-      const auto h0 = std::chrono::steady_clock::now();
       MOPT_TRY(launch_p2p_lm_mono(L, stores[0]->dtype, p0.compute_dtype, p0.loss, qrot, a, m));
-      const auto h1 = std::chrono::steady_clock::now();
       // The kernel's last act is to set the mapped flag (after a system-scope fence behind the state and the trace):
       // spinning on it sees the end ~5 us before cudaStreamSynchronize would return (kernel teardown + driver
-      // wake-up).  The stream is queried now and then so that a failed launch cannot hang the caller; with the
-      // trace on, the stream is drained as before (the stamps are read back).
-      if (trace) {
-        MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-      } else {
-        for (int spins = 0;; ++spins) {
-          if (reinterpret_cast<volatile int*>(ctx->h_flags)[0] != 0) break;
-          if ((spins & 4095) == 4095) {
-            const cudaError_t q = cudaStreamQuery(ctx->stream);
-            if (q == cudaSuccess) break;  // finished (the flag is set by now, or the state says why not)
-            if (q != cudaErrorNotReady) MOPT_CUDA_TRY(q);
-          }
-        }
-        std::atomic_thread_fence(std::memory_order_acquire);
-      }
-      const auto h2 = std::chrono::steady_clock::now();
-      if (d_dbg) {
-        std::fprintf(stderr, "mono host: launch call %.1f us, wait for the kernel %.1f us\n",
-                     std::chrono::duration<double, std::micro>(h1 - h0).count(),
-                     std::chrono::duration<double, std::micro>(h2 - h1).count());
-        unsigned long long h[512];
-        MOPT_CUDA_TRY(cudaMemcpy(h, d_dbg, sizeof(h), cudaMemcpyDeviceToHost));
-        cudaFree(d_dbg);
-        std::fprintf(stderr, "mono kernel: init %.2f us, loop %.2f us (CTA 0), last data CTA leaves %+.2f us after CTA 0\n",
-                     (h[501] - h[500]) * 1e-3, (h[502] - h[501]) * 1e-3, (double(h[503]) - double(h[502])) * 1e-3);
-        for (int s = 0; s < 64 && h[s * 4 + 3]; ++s)
-          std::fprintf(stderr, "mono trial %2d: pass %6.2f us  step %6.2f us  open %5.2f us  (next begins +%6.2f us)\n", s,
-                       (h[s * 4 + 1] - h[s * 4]) * 1e-3, (h[s * 4 + 2] - h[s * 4 + 1]) * 1e-3, (h[s * 4 + 3] - h[s * 4 + 2]) * 1e-3,
-                       h[(s + 1) * 4] ? (double(h[(s + 1) * 4]) - double(h[s * 4 + 3])) * 1e-3 : 0.0);
-        for (int s = 0; s < 15 && h[256 + s * 16 + 5]; ++s) {
-          const unsigned long long* q = h + 256 + s * 16;
-          std::fprintf(stderr, "mono step %2d (cycles): stage-in %llu  state machine %llu  solve+propose %llu  setup %llu  write-back %llu",
-                       s, q[1] - q[0], q[2] - q[1], q[3] - q[2], q[4] - q[3], q[5] - q[4]);
-          if (q[10] > q[6] && q[6] > q[2])
-            std::fprintf(stderr, "  | build A %llu  factor %llu  forward %llu  D %llu  backward %llu  propose %llu", q[6] - q[2],
-                         q[7] - q[6], q[8] - q[7], q[9] - q[8], q[10] - q[9], q[3] - q[10]);
-          if (q[11] > q[3]) std::fprintf(stderr, "  | barrier opened %llu cycles into the setup", q[11] - q[3]);
-          std::fprintf(stderr, "\n");
+      // wake-up).  The stream is queried now and then so that a failed launch cannot hang the caller.
+      for (int spins = 0;; ++spins) {
+        if (reinterpret_cast<volatile int*>(ctx->h_flags)[0] != 0) break;
+        if ((spins & 4095) == 4095) {
+          const cudaError_t q = cudaStreamQuery(ctx->stream);
+          if (q == cudaSuccess) break;  // finished (the flag is set by now, or the state says why not)
+          if (q != cudaErrorNotReady) MOPT_CUDA_TRY(q);
         }
       }
+      std::atomic_thread_fence(std::memory_order_acquire);
       return finish_lm(ctx, P, x, report, /*on_host=*/true);
     }
   }
 
   MOPT_TRY(launch_init());
-  static const bool step_prof = [] { const char* e = getenv("MOPT_LM_MONO_TRACE"); return e && e[0] == '1'; }();
   // Passes are enqueued in batches, always one batch ahead of the one whose done flag is being
   // awaited, so the device never idles on the host; every rank reads the flag of the same slot,
   // so all ranks stop after the same number of (collective-bearing) slots.
@@ -965,7 +912,7 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
         MOPT_TRY(launch_pass(ctx, stores[c], &problems[c], c, c > 0 ? 1 : 0, -1, c == n_costs - 1));
       MOPT_TRY(allreduce_trial(ctx, P, -1));
       lm_step_kernel<<<1, 32, 0, ctx->stream>>>(ctx->d_lm, ctx->d_trial, ctx->d_slots, ctx->d_flags + slot_index(enq),
-                                                ctx->d_xerr_dev, step_prof ? 1 : 0, in.P, in.scalar_f32);
+                                                ctx->d_xerr_dev, in.P, in.scalar_f32);
       MOPT_CUDA_TRY(cudaGetLastError());
       MOPT_TRY(user_setups());
       *last_slot = enq;
@@ -985,12 +932,6 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
     cur_last = next_last;
   }
   MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  if (step_prof) {
-    long long q[8];
-    MOPT_CUDA_TRY(cudaMemcpyFromSymbol(q, g_step_prof, sizeof(q)));
-    std::fprintf(stderr, "lm_step_kernel (cycles): stage-in %lld  state machine %lld  solve+propose %lld  setup %lld  write-back %lld\n",
-                 q[1] - q[0], q[2] - q[1], q[3] - q[2], q[4] - q[3], q[5] - q[4]);
-  }
 
   return finish_lm(ctx, P, x, report);
 }

@@ -225,11 +225,6 @@ __host__ __device__ __forceinline__ double fast_rcp(double x) { return 1.0 / x; 
 __host__ __device__ __forceinline__ bool all_abs_below(float x, float t) { return fabsf(x) < t; }
 __host__ __device__ __forceinline__ bool all_abs_below(double x, float t) { return fabs(x) < double(t); }
 
-// TMA bulk prefetch of `bytes` (multiple of 16, 16-byte aligned source) into L2.
-__device__ __forceinline__ void l2_prefetch_bulk(const void* p, unsigned bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
 template <typename ST>
 struct VecOf;
 template <>

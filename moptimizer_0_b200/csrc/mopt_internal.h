@@ -113,6 +113,32 @@ int launch_user_setup(cudaStream_t stream, int device, int model, CostSlot* slot
 int user_model_rot_offset(int model);
 bool user_model_has_setup(int model);
 
-int pick_grid(const void* kernel, int threads, const PassLaunch& L, int64_t work_items);
+// Persistent grid of a streaming kernel: resident CTAs per SM (at most L.ctas_per_sm when that is set) times the SMs,
+// capped at kMaxGrid and at one CTA per `threads` work items, never below 1.  The summation order of a pass follows
+// the grid, so every launcher of a pass kernel sizes it here.
+inline int pick_grid(const void* kernel, int threads, const PassLaunch& L, int64_t work_items, size_t dyn_smem = 0) {
+  int occ = 1;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, dyn_smem) != cudaSuccess || occ < 1) occ = 1;
+  int per_sm = (L.ctas_per_sm > 0) ? (L.ctas_per_sm < occ ? L.ctas_per_sm : occ) : occ;
+  int64_t g = int64_t(per_sm) * L.num_sms;
+  if (g > kMaxGrid) g = kMaxGrid;
+  const int64_t need = (work_items + threads - 1) / threads;
+  if (need < g) g = need;
+  if (g < 1) g = 1;
+  return int(g);
+}
+
+// Opt kernel K in to `bytes` of dynamic shared memory.  Function attributes are per device, so this runs once on each.
+template <auto K>
+int allow_dyn_smem(size_t bytes) {
+  static bool configured[64] = {false};
+  int dev = 0;
+  MOPT_CUDA_TRY(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= 64 || !configured[dev]) {
+    MOPT_CUDA_TRY(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, int(bytes)));
+    if (dev >= 0 && dev < 64) configured[dev] = true;
+  }
+  return MOPT_OK;
+}
 
 }  // namespace mopt

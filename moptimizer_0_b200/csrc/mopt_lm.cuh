@@ -131,8 +131,7 @@ __device__ inline void lm_finish(LmState* st, int status) {
 // cycles per 6 x 6 solve on a B200 against ~5 000 now.  A (n x n, column-major, overwritten), tmp, y and tr live in
 // shared memory; n <= 16.  NC > 0: the size is known at compile time (the loops unroll).
 template <typename S, int NC = 0>
-__device__ inline void ldlt_solve_warp(int n_rt, S* A, const S* rhs, S* out, S* tmp, S* y, int* tr, int lane,
-                                       long long* prof = nullptr) {
+__device__ inline void ldlt_solve_warp(int n_rt, S* A, const S* rhs, S* out, S* tmp, S* y, int* tr, int lane) {
   const int n = NC > 0 ? NC : n_rt;
   unsigned long long perm = 0xFEDCBA9876543210ull;
   auto PH = [&](int i) { return int((perm >> (4 * i)) & 15ull); };
@@ -176,7 +175,6 @@ __device__ inline void ldlt_solve_warp(int n_rt, S* A, const S* rhs, S* out, S* 
     if (valid && lane > k && lane < n) MOPT_A(PH(lane), pk) /= akk;
     __syncwarp();
   }
-  if (prof && lane == 0) prof[7] = clock64();
   if (lane == 0) {
     for (int i = 0; i < n; ++i) y[i] = rhs[i];
     for (int k = 0; k < n; ++k) { const S t = y[k]; y[k] = y[tr[k]]; y[tr[k]] = t; }
@@ -188,14 +186,12 @@ __device__ inline void ldlt_solve_warp(int n_rt, S* A, const S* rhs, S* out, S* 
     }
   }
   __syncwarp();
-  if (prof && lane == 0) prof[8] = clock64();
   if (lane < n) {  // D^+ with tolerance numeric_limits::min(): one division per lane
     const S tol = (sizeof(S) == 4) ? S(1.17549435e-38) : S(2.2250738585072014e-308);
     const S dd = MOPT_A(PH(lane), PH(lane));
     y[lane] = (fabs(dd) > tol) ? y[lane] / dd : S(0);
   }
   __syncwarp();
-  if (prof && lane == 0) prof[9] = clock64();
   if (lane == 0) {
     for (int r = n - 1; r >= 0; --r) {
       const int pr = PH(r);
@@ -207,7 +203,6 @@ __device__ inline void ldlt_solve_warp(int n_rt, S* A, const S* rhs, S* out, S* 
     for (int i = 0; i < n; ++i) out[i] = y[i];
   }
   __syncwarp();
-  if (prof && lane == 0) prof[10] = clock64();
 #undef MOPT_A
 }
 
@@ -220,8 +215,7 @@ struct LmSolveScratch {
 // Solve (H + lambda diag(H)) delta = -b (levenberg_marquadt_dyn.cpp:65,78-80), xi = x (+) delta (:83), executed by
 // one full warp: the lanes build the damped matrix and factor it together.
 template <typename S, int PC = 0>
-__device__ inline void lm_solve_propose_warp(LmState* st, const CostDev& cost0, LmSolveScratch* sc, int lane,
-                                             long long* prof = nullptr) {
+__device__ inline void lm_solve_propose_warp(LmState* st, const CostDev& cost0, LmSolveScratch* sc, int lane) {
   const int P = PC > 0 ? PC : st->P;
   S* A = reinterpret_cast<S*>(sc->A);
   S* nb = reinterpret_cast<S*>(sc->nb);
@@ -234,8 +228,7 @@ __device__ inline void lm_solve_propose_warp(LmState* st, const CostDev& cost0, 
   }
   if (lane < P) nb[lane] = -S(st->cur.v[P * (P + 1) / 2 + lane]);
   __syncwarp();
-  if (prof && lane == 0) prof[6] = clock64();
-  ldlt_solve_warp<S, PC>(P, A, nb, d, reinterpret_cast<S*>(sc->tmp), reinterpret_cast<S*>(sc->y), sc->tr, lane, prof);
+  ldlt_solve_warp<S, PC>(P, A, nb, d, reinterpret_cast<S*>(sc->tmp), reinterpret_cast<S*>(sc->y), sc->tr, lane);
   if (cost0.manifold == MOPT_MANIFOLD_SO3_LEFT) {
     if (lane == 0) {
       for (int i = 0; i < P; ++i) st->delta[i] = double(d[i]);
@@ -406,7 +399,6 @@ struct LmStepIo {
   unsigned long long* rt_words = nullptr;
   unsigned long long gen_target = 0;
   int* opened = nullptr;
-  bool generic_p = false;  // A/B: run the P = 6 case through the generic-size code (loops instead of unrolled)
   LmState* host_state = nullptr;  // mapped host memory: the trace and the final state are written there as well,
   int* host_flag = nullptr;       // then this word is set (after a system-scope fence): the host may stop waiting
 };
@@ -445,9 +437,8 @@ static __device__ __noinline__ void lm_init_warp(LmState* st, CostSlot* slots, c
 // Returns the state's `done` flag after the transition.
 template <typename S, int PC>
 __device__ inline int lm_step_warp_t(LmState* gst, const PassResult* gtrial, CostSlot* slots, LmStepShared* sh, int lane,
-                                     int P_rt, const LmStepIo& io, long long* prof = nullptr) {
+                                     int P_rt, const LmStepIo& io) {
   LmState* st = reinterpret_cast<LmState*>(sh->hot);
-  if (prof && lane == 0) prof[0] = clock64();
   const int npk = packed_size(PC > 0 ? PC : P_rt);
   {
     const double* g = reinterpret_cast<const double*>(gst);
@@ -482,7 +473,6 @@ __device__ inline int lm_step_warp_t(LmState* gst, const PassResult* gtrial, Cos
     }
   }
   __syncwarp();
-  if (prof && lane == 0) prof[1] = clock64();
   const CostDev& cost0 = io.cost0 ? *io.cost0 : slots[0].cost;
   int act = 0;
   if (lane == 0) act = lm_step_thread<S, PC>(st, &sh->trial, cost0, io.host_state ? io.host_state->trials : gst->trials);
@@ -493,21 +483,18 @@ __device__ inline int lm_step_warp_t(LmState* gst, const PassResult* gtrial, Cos
     __syncwarp();
     act &= ~kLmCopyTrial;
   }
-  if (prof && lane == 0) prof[2] = clock64();
   if (act == 2) {  // damped solve + proposal, the lanes sharing the factorization
-    lm_solve_propose_warp<S, PC>(st, cost0, &sh->sc, lane, prof);
+    lm_solve_propose_warp<S, PC>(st, cost0, &sh->sc, lane);
     __syncwarp();
   }
-  if (prof && lane == 0) prof[3] = clock64();
   if (act) {
     const int nc = st->n_costs;
-    const SetupEarlyOpen eo{io.rt_words, (io.gen_target << 2) | (unsigned long long)(st->pass_mode), io.opened, prof};
+    const SetupEarlyOpen eo{io.rt_words, (io.gen_target << 2) | (unsigned long long)(st->pass_mode), io.opened};
     for (int c = 0; c < nc; ++c)
       setup_cost(c == 0 ? cost0 : slots[c].cost, st->x_eval, &slots[c].pb, lane, 32, sh->sc.tmp,
                  (io.rt_words != nullptr && nc == 1) ? &eo : nullptr);
   }
   __syncwarp();
-  if (prof && lane == 0) prof[4] = clock64();
   if (io.store_state || st->done) {
     double* g = reinterpret_cast<double*>(gst);
     for (int i = lane; i < kLmHotWords; i += 32) g[i] = sh->hot[i];
@@ -520,7 +507,6 @@ __device__ inline int lm_step_warp_t(LmState* gst, const PassResult* gtrial, Cos
     }
   }
   __syncwarp();
-  if (prof && lane == 0) prof[5] = clock64();
   return st->done;
 }
 // P and the Scalar of the LM arithmetic are launch-time constants of a minimize() call: the callers pass them as
@@ -528,13 +514,13 @@ __device__ inline int lm_step_warp_t(LmState* gst, const PassResult* gtrial, Cos
 // __noinline__: one copy per translation unit instead of one per kernel instantiation (the persistent LM kernel alone
 // has 18; inlined, that translation unit took six minutes to compile).
 static __device__ __noinline__ int lm_step_warp(LmState* st, const PassResult* trial, CostSlot* slots, LmStepShared* sh, int lane,
-                                                int P, bool f32, const LmStepIo& io, long long* prof = nullptr) {
-  if (P == 6 && !io.generic_p) {  // the 6-DoF registration case with unrolled loops
-    return f32 ? lm_step_warp_t<float, 6>(st, trial, slots, sh, lane, P, io, prof)
-               : lm_step_warp_t<double, 6>(st, trial, slots, sh, lane, P, io, prof);
+                                                int P, bool f32, const LmStepIo& io) {
+  if (P == 6) {  // the 6-DoF registration case with unrolled loops
+    return f32 ? lm_step_warp_t<float, 6>(st, trial, slots, sh, lane, P, io)
+               : lm_step_warp_t<double, 6>(st, trial, slots, sh, lane, P, io);
   }
-  return f32 ? lm_step_warp_t<float, 0>(st, trial, slots, sh, lane, P, io, prof)
-             : lm_step_warp_t<double, 0>(st, trial, slots, sh, lane, P, io, prof);
+  return f32 ? lm_step_warp_t<float, 0>(st, trial, slots, sh, lane, P, io)
+             : lm_step_warp_t<double, 0>(st, trial, slots, sh, lane, P, io);
 }
 
 #endif  // __CUDACC__

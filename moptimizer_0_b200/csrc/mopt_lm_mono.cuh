@@ -25,10 +25,8 @@ struct MonoArgs {
   unsigned long long* rt_words; // 24 tagged words: (R, t) of the next pass + its control word = the grid barrier (publish_rt)
   unsigned long long gen_base;  // barrier targets of this launch start here (monotonic over the context's life)
   int max_slots;
-  int generic_p;                // A/B switch (MOPT_LM_GENERIC_P=1): LmStepIo::generic_p
   int loss, qrot;               // mopt_loss_kind / "the moments are taken in q = R p" of the pass, chosen at run time here
   LmInit init;                  // prepare() arguments: CTA 0 initialises the state before the first pass
-  unsigned long long* dbg;  // optional (MOPT_LM_MONO_TRACE=1): 4 globaltimer stamps per trial from the last CTA
 };
 
 #ifdef __CUDACC__
@@ -38,7 +36,7 @@ struct MonoArgs {
 // transition once per entry, and with a kernel per (loss, form) this translation unit took six minutes to build.
 template <typename ST, typename CT, int THREADS, int UNROLL, int FLUSH_ROUNDS>
 __device__ __forceinline__ void p2p_mono_pass(const PassArgs& a, int mode, int loss, bool qrot, const double* rt) {
-#define MOPT_MONO_BODY(L, Q) p2p_moment_body<ST, CT, L, Q, THREADS, UNROLL, FLUSH_ROUNDS, 0, false, false, true>(a, mode, rt)
+#define MOPT_MONO_BODY(L, Q) p2p_moment_body<ST, CT, L, Q, THREADS, UNROLL, FLUSH_ROUNDS, false, true>(a, mode, rt)
   switch (loss) {
     case MOPT_LOSS_NONE: qrot ? MOPT_MONO_BODY(MOPT_LOSS_NONE, true) : MOPT_MONO_BODY(MOPT_LOSS_NONE, false); break;
     case MOPT_LOSS_GEMAN_MCCLURE:
@@ -91,7 +89,6 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_lm_mono_kernel(const PassAr
     publish_rt(m.rt_words, (target << 2) | (unsigned long long)(mode), v, lane);
   };
   const bool master = blockIdx.x == 0;
-  if (m.dbg && master && threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); m.dbg[500] = t; }
   // prepare() + the first setup(x0): CTA 0, everyone else waits (no separate init kernel, no launch gap)
   if (master) {
     for (int i = threadIdx.x; i < int(sizeof(CostDev) / 4); i += THREADS)
@@ -108,7 +105,6 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_lm_mono_kernel(const PassAr
     if (threadIdx.x == 0) s_mode = mode;
   }
   __syncthreads();
-  if (m.dbg && master && threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); m.dbg[501] = t; }
   for (int slot = 0; slot < m.max_slots; ++slot) {
     const int mode = s_mode;  // written before the __syncthreads that ends the previous iteration
     if (mode == PASS_SKIP) break;
@@ -121,12 +117,9 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_lm_mono_kernel(const PassAr
         if (threadIdx.x == 0) s_mode = next;
       }
     } else {
-      unsigned long long t_begin = 0, t_pass = 0, t_step = 0, t_open = 0;
-      if (m.dbg && threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_begin));
       p2p_master_tail<THREADS>(a, mode, &s_sh.trial);
       if (threadIdx.x == 0) s_opened = 0;
       __syncthreads();  // the pass result complete (assembled by the whole CTA, in shared memory)
-      if (m.dbg && threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_pass));
       if (threadIdx.x < 32) {
         LmStepIo io;
         io.load_state = false;
@@ -138,26 +131,14 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_lm_mono_kernel(const PassAr
         io.opened = &s_opened;
         io.host_state = m.host_st;
         io.host_flag = m.host_flag;
-        io.generic_p = m.generic_p != 0;
-        lm_step_warp(m.st, &s_sh.trial, m.slots, &s_sh, threadIdx.x, m.init.P, m.init.scalar_f32 != 0, io,
-                     (m.dbg && slot < 15) ? reinterpret_cast<long long*>(m.dbg) + 256 + slot * 16 : nullptr);
+        lm_step_warp(m.st, &s_sh.trial, m.slots, &s_sh, threadIdx.x, m.init.P, m.init.scalar_f32 != 0, io);
         __syncwarp();
         const int next = reinterpret_cast<const LmState*>(s_sh.hot)->pass_mode;
         if (!s_opened) publish_from_pb(target, next);  // generic set-ups, and the final "stop"
         if (threadIdx.x == 0) s_mode = next;
       }
-      if (m.dbg && threadIdx.x == 0) {
-        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_step));
-        t_open = t_step;
-        if (slot < 64) { m.dbg[slot * 4 + 0] = t_begin; m.dbg[slot * 4 + 1] = t_pass; m.dbg[slot * 4 + 2] = t_step; m.dbg[slot * 4 + 3] = t_open; }
-      }
     }
     __syncthreads();
-  }
-  if (m.dbg && threadIdx.x == 0 && (master || blockIdx.x == gridDim.x - 1)) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    m.dbg[master ? 502 : 503] = t;
   }
 }
 

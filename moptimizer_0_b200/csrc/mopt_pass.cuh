@@ -438,8 +438,7 @@ __device__ __forceinline__ void p2p_master_tail(const PassArgs& a, int mode, Pas
 // FUSED: model->setup(x) runs inside the kernel (PassArgs::x; host-driven analytical passes), `pb` is not read.
 // The pass itself, callable from the one-pass kernel below and from the persistent LM kernel (mopt_lm_mono.cuh).
 // Returns true in the last CTA once `out` holds the packed result.
-template <typename ST, typename CT, int LOSS, bool QROT, int THREADS, int UNROLL, int FLUSH_ROUNDS, int PF, bool SWP,
-          bool FUSED, bool COHERENT>
+template <typename ST, typename CT, int LOSS, bool QROT, int THREADS, int UNROLL, int FLUSH_ROUNDS, bool FUSED, bool COHERENT>
 __device__ __forceinline__ bool p2p_moment_body(const PassArgs& a, const int mode, const double* rt = nullptr) {
   // COHERENT: a data CTA of the persistent LM kernel, whose CTA 0 takes no residuals (grid_reduce_shared); (R, t)
   // comes in `rt` (shared memory, received with the barrier: publish_rt) instead of the ParamBlock
@@ -509,67 +508,10 @@ __device__ __forceinline__ bool p2p_moment_body(const PassArgs& a, const int mod
     }
   };
 
-  // L2 bulk prefetch (TMA, cp.async.bulk.prefetch.L2): one thread per CTA asks for the CTA's 6 x (THREADS*16 B)
-  // slices of round `rr`, PF rounds ahead of the demand loads, so the register-limited number of loads in
-  // flight no longer bounds the DRAM queue depth.
-  auto prefetch_round = [&](int64_t rr) {
-    if (PF > 0 && threadIdx.x == 0 && rr < full_rounds) {
-      const int64_t e0 = (int64_t(bid) * THREADS + rr * stride) * VEC;
-      constexpr unsigned bytes = THREADS * VEC * sizeof(ST);
-      l2_prefetch_bulk(sx + e0, bytes); l2_prefetch_bulk(sy + e0, bytes); l2_prefetch_bulk(sz + e0, bytes);
-      l2_prefetch_bulk(tx + e0, bytes); l2_prefetch_bulk(ty + e0, bytes); l2_prefetch_bulk(tz + e0, bytes);
-    }
-  };
-  if (PF > 0)
-    for (int64_t rr = 0; rr < PF; ++rr) prefetch_round(rr);
-
   int since_flush = 0;
   int64_t r = 0;
-  if constexpr (SWP) {
-    // Software-pipelined variant: the loads of round r+1 are issued before round r is consumed, so every
-    // warp keeps 6 x 16-byte loads in flight through its whole compute phase (two register buffers, A / B).
-    auto load_round = [&](CT (&buf)[6][VEC], int64_t rr) {
-      const int64_t g = g0 + rr * stride;
-      load_vec<ST, CT>(sx, g, buf[0]); load_vec<ST, CT>(sy, g, buf[1]); load_vec<ST, CT>(sz, g, buf[2]);
-      load_vec<ST, CT>(tx, g, buf[3]); load_vec<ST, CT>(ty, g, buf[4]); load_vec<ST, CT>(tz, g, buf[5]);
-    };
-    auto consume = [&](const CT (&buf)[6][VEC]) {
-      if (mode == PASS_COST) {
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) p2p_cost_only<CT>(masked, R, t, buf[0][e], buf[1][e], buf[2][e], buf[3][e], buf[4][e], buf[5][e], acc);
-      } else {
-#pragma unroll
-        for (int e = 0; e < VEC; ++e)
-          p2p_moments<CT, LOSS, QROT>(masked, R, t, lossp, buf[0][e], buf[1][e], buf[2][e], buf[3][e], buf[4][e], buf[5][e], acc);
-      }
-    };
-    if (full_rounds > 0) {
-      CT A[6][VEC], B[6][VEC];
-      load_round(A, 0);
-      for (;;) {
-        if (r + 1 < full_rounds) load_round(B, r + 1);
-        consume(A);
-        if (r + 1 >= full_rounds) { r += 1; break; }
-        if (r + 2 < full_rounds) load_round(A, r + 2);
-        consume(B);
-        r += 2;
-        if (kFp32Acc) {
-          since_flush += 2;
-          if (since_flush >= FLUSH_ROUNDS) {
-            flush();
-            since_flush = 0;
-          }
-        }
-        if (r >= full_rounds) break;
-      }
-    }
-  }
   // UNROLL grid-stride rounds per iteration: 6*UNROLL independent 16-byte loads in flight per thread
   for (; r + (UNROLL - 1) < full_rounds; r += UNROLL) {
-    if (PF > 0) {
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u) prefetch_round(r + PF + u);
-    }
     CT px[UNROLL][VEC], py[UNROLL][VEC], pz[UNROLL][VEC], qx[UNROLL][VEC], qy[UNROLL][VEC], qz[UNROLL][VEC];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
@@ -616,12 +558,12 @@ __device__ __forceinline__ bool p2p_moment_body(const PassArgs& a, const int mod
 }
 
 template <typename ST, typename CT, int LOSS, bool QROT, int THREADS, int MINB, int UNROLL = 2, int FLUSH_ROUNDS = 8,
-          int PF = 0, bool SWP = false, bool FUSED = false>
+          bool FUSED = false>
 __global__ void __launch_bounds__(THREADS, MINB) p2p_moment_kernel(const PassArgs a) {
   const int mode = a.mode_override >= 0 ? a.mode_override : *a.mode_ptr;
   if (mode == PASS_SKIP) return;
   if (peer_failed(a)) return;
-  p2p_moment_body<ST, CT, LOSS, QROT, THREADS, UNROLL, FLUSH_ROUNDS, PF, SWP, FUSED, false>(a, mode);
+  p2p_moment_body<ST, CT, LOSS, QROT, THREADS, UNROLL, FLUSH_ROUNDS, FUSED, false>(a, mode);
 }
 
 // =============================================================================================

@@ -1,6 +1,4 @@
 // Instantiations + dispatch of the generic dense pass kernel (mopt_pass.cuh).
-#include <cstdlib>
-
 #include "mopt_internal.h"
 #include "mopt_pass_dense_f2.cuh"
 
@@ -28,49 +26,20 @@ int launch_shape(const PassLaunch& L, const PassArgs& a) {
 }
 
 // Second generation for fp32 finite differences of models with an affine first stage (mopt_pass_dense_f2.cuh): two
-// observations per thread in packed fp32.  MOPT_DENSE_F2_SHAPE in the environment selects the launch shape (A/B).
-template <class M, int THREADS, int MINB>
-int launch_f2_shape(const PassLaunch& L, const PassArgs& a) {
-  auto kern = dense_f2_kernel<M, THREADS, MINB>;
-  PassLaunch L2 = L;
-  L2.ctas_per_sm = 0;
-  const int grid = pick_grid(reinterpret_cast<const void*>(kern), THREADS, L2, a.n / 4);
-  kern<<<grid, THREADS, 0, L.stream>>>(a);
-  MOPT_CUDA_TRY(cudaGetLastError());
-  return MOPT_OK;
-}
+// observations per thread in packed fp32, 256 threads x 2 CTAs per SM.
 template <class M>
 int launch_f2(const PassLaunch& L, const PassArgs& a) {
-  static const int shape = [] {
-    const char* e = getenv("MOPT_DENSE_F2_SHAPE");
-    return (e && e[0]) ? atoi(e) : 0;
-  }();
-  switch (shape) {
-    case 1: return launch_f2_shape<M, 256, 1>(L, a);
-    case 2: return launch_f2_shape<M, 128, 3>(L, a);
-    case 3: return launch_f2_shape<M, 128, 4>(L, a);
-    case 4: return launch_f2_shape<M, 256, 3>(L, a);
-    case 5: return launch_f2_shape<M, 256, 4>(L, a);
-    case 6: return launch_f2_shape<M, 256, 6>(L, a);
-    default: return launch_f2_shape<M, 256, 2>(L, a);
-  }
+  auto kern = dense_f2_kernel<M, kThreads, 2>;
+  PassLaunch L2 = L;
+  L2.ctas_per_sm = 0;
+  const int grid = pick_grid(reinterpret_cast<const void*>(kern), kThreads, L2, a.n / 4);
+  kern<<<grid, kThreads, 0, L.stream>>>(a);
+  MOPT_CUDA_TRY(cudaGetLastError());
+  return MOPT_OK;
 }
 
 template <class M, typename ST, typename CT, bool NUMERIC>
 int launch_one(const PassLaunch& L, const PassArgs& a) {
-#ifdef MOPT_TUNE_DENSE
-  // tuning build: register-cap / CTA-shape variants of the fp32 finite-difference kernels, selected with
-  // mopt_ctx_set_launch(ctas_per_sm, threads)
-  if constexpr (NUMERIC && sizeof(ST) == 4 && M::P >= 4) {
-    if (L.threads == 128) {
-      if (L.ctas_per_sm == 6) return launch_shape<M, ST, CT, NUMERIC, 128, 6>(L, a);
-      return launch_shape<M, ST, CT, NUMERIC, 128, 4>(L, a);
-    }
-    if (L.ctas_per_sm == 2) return launch_shape<M, ST, CT, NUMERIC, 256, 2>(L, a);
-    if (L.ctas_per_sm == 3) return launch_shape<M, ST, CT, NUMERIC, 256, 3>(L, a);
-    if (L.ctas_per_sm == 4) return launch_shape<M, ST, CT, NUMERIC, 256, 4>(L, a);
-  }
-#endif
   // Finite-difference kernels of the 6-parameter models want all 1 + 2P parameter sets in registers (247-255
   // registers, one 256-thread CTA per SM, issue slots 34 % busy).  Capping them at 80 registers (3 CTAs per SM)
   // turns the hoisted sets into L1-resident local loads and triples the warps that hide the division / MUFU

@@ -3,18 +3,6 @@
 
 namespace mopt {
 
-int pick_grid(const void* kernel, int threads, const PassLaunch& L, int64_t work_items) {
-  int occ = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, 0) != cudaSuccess || occ < 1) occ = 1;
-  int per_sm = (L.ctas_per_sm > 0) ? (L.ctas_per_sm < occ ? L.ctas_per_sm : occ) : occ;
-  int64_t g = int64_t(per_sm) * L.num_sms;
-  if (g > kMaxGrid) g = kMaxGrid;
-  const int64_t need = (work_items + threads - 1) / threads;
-  if (need < g) g = need;
-  if (g < 1) g = 1;
-  return int(g);
-}
-
 namespace {
 
 // Launch shapes (profiles/r1_tune_p2p.txt): the fp32 kernel is bound by bytes in flight, not by its ALU
@@ -31,7 +19,7 @@ struct ShapeF64 {
 
 template <typename ST, typename CT, int LOSS, bool QROT, class S, bool FUSED>
 int launch_fused(const PassLaunch& L, const PassArgs& a) {
-  auto kern = p2p_moment_kernel<ST, CT, LOSS, QROT, S::THREADS, S::MINB, S::UNROLL, S::FLUSH, 0, false, FUSED>;
+  auto kern = p2p_moment_kernel<ST, CT, LOSS, QROT, S::THREADS, S::MINB, S::UNROLL, S::FLUSH, FUSED>;
   const int64_t groups = a.n / VecOf<ST>::N;
   // small problems: keep CTAs at 256 threads' worth of work granularity by capping the grid, never below 1
   const int grid = pick_grid(reinterpret_cast<const void*>(kern), S::THREADS, L, groups);

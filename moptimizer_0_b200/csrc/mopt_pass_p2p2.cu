@@ -18,15 +18,9 @@ struct ShapeGen2 {
 // ---- second generation (fp32 store, fp32 compute) ----------------------------------------------------------
 template <int LOSS, bool QROT, bool MASKED, bool FUSED, class S>
 int launch_gen2_one(const PassLaunch& L, const PassArgs& a0) {
-  auto kern = p2p_moment2_kernel<LOSS, QROT, MASKED, FUSED, S::THREADS, 1, S::STAGES, S::U, S::FLUSH, 0>;
+  constexpr auto kern = p2p_moment2_kernel<LOSS, QROT, MASKED, FUSED, S::THREADS, 1, S::STAGES, S::U, S::FLUSH>;
   constexpr size_t smem = p2p2_ring_bytes(S::THREADS, S::STAGES, S::U);
-  static bool configured[64] = {false};  // function attributes are per device
-  int dev = 0;
-  MOPT_CUDA_TRY(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    MOPT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
+  MOPT_TRY(allow_dyn_smem<kern>(smem));
   PassArgs a = a0;
   // the bulk copies need 16-byte aligned sources; anything else streams through the kernel's direct-load path
   for (int k = 0; k < 6; ++k)

@@ -127,11 +127,10 @@ __device__ __forceinline__ void p2p_cost_x2(const float (&R)[9], const float (&t
 // Shared-memory footprint of the ring: STAGES x 6 streams x (U * THREADS) float4.
 constexpr size_t p2p2_ring_bytes(int threads, int stages, int u) { return size_t(stages) * 6 * size_t(u) * threads * 16; }
 
-// STAGES == 0: no ring, 16-byte streaming loads straight into registers (small problems, unaligned stores, A/B).
-// U: float4 groups per thread per stream per round.  PF (STAGES == 0 only): L2 bulk prefetch distance in rounds.
-template <int LOSS, bool QROT, bool MASKED, bool FUSED, int THREADS, int MINB, int STAGES, int U, int FLUSH_ROUNDS,
-          int PF = 0>
+// U: float4 groups per thread per stream per round.
+template <int LOSS, bool QROT, bool MASKED, bool FUSED, int THREADS, int MINB, int STAGES, int U, int FLUSH_ROUNDS>
 __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassArgs a) {
+  static_assert(STAGES > 0, "p2p_moment2_kernel: the ring needs at least one stage");
   const int mode = a.mode_override >= 0 ? a.mode_override : *a.mode_ptr;
   if (mode == PASS_SKIP) return;
   if (peer_failed(a)) return;
@@ -141,8 +140,8 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
   __shared__ double s_warp[NW * 32];
   __shared__ double s_tot[32];
   __shared__ double s_set0[FUSED ? 12 : 1];
-  __shared__ __align__(8) uint64_t s_full[STAGES > 0 ? STAGES : 1];
-  __shared__ __align__(8) uint64_t s_empty[STAGES > 0 ? STAGES : 1];
+  __shared__ __align__(8) uint64_t s_full[STAGES];
+  __shared__ __align__(8) uint64_t s_empty[STAGES];
   extern __shared__ __align__(128) unsigned char p2p2_ring[];
   float4* ring = reinterpret_cast<float4*>(p2p2_ring);  // [STAGES][6][CHUNK]
 
@@ -156,17 +155,15 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
       p2p_fused_set0(a.cost, xl, s_set0);
     }
   }
-  if constexpr (STAGES > 0) {
-    if (threadIdx.x == 0) {
+  if (threadIdx.x == 0) {
 #pragma unroll
-      for (int s = 0; s < STAGES; ++s) {
-        mbar_init(&s_full[s], 1);
-        mbar_init(&s_empty[s], NW);
-      }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(&s_full[s], 1);
+      mbar_init(&s_empty[s], NW);
     }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if constexpr (FUSED || STAGES > 0) __syncthreads();
+  __syncthreads();
 
   const float* __restrict__ sp[6];
 #pragma unroll
@@ -174,7 +171,7 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
 
   const int64_t ngroups = a.n / 4;
   const int64_t stride = int64_t(gridDim.x) * CHUNK;   // groups per round over the whole grid
-  const int64_t full_rounds = (STAGES > 0 && a.no_ring) ? 0 : ngroups / stride;
+  const int64_t full_rounds = a.no_ring ? 0 : ngroups / stride;
 
   // producer (thread 0): the CTA's 6 x CHUNK x 16 B slices of round rr into stage rr % STAGES
   auto issue_to = [&](int64_t rr, int s) {
@@ -184,19 +181,8 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
     for (int k = 0; k < 6; ++k)
       bulk_g2s(ring + (size_t(s) * 6 + k) * CHUNK, reinterpret_cast<const float4*>(sp[k]) + g, CHUNK * 16u, &s_full[s]);
   };
-  if constexpr (STAGES > 0) {
-    if (threadIdx.x == 0)
-      for (int rr = 0; rr < STAGES && rr < full_rounds; ++rr) issue_to(rr, rr);
-  }
-  auto prefetch_round = [&](int64_t rr) {  // STAGES == 0: TMA bulk prefetch into L2, PF rounds ahead of the demand loads
-    if (PF > 0 && threadIdx.x == 0 && rr < full_rounds) {
-      const int64_t g = rr * stride + int64_t(blockIdx.x) * CHUNK;
-#pragma unroll
-      for (int k = 0; k < 6; ++k) l2_prefetch_bulk(reinterpret_cast<const float4*>(sp[k]) + g, CHUNK * 16u);
-    }
-  };
-  if constexpr (STAGES == 0 && PF > 0)
-    for (int64_t rr = 0; rr < PF; ++rr) prefetch_round(rr);
+  if (threadIdx.x == 0)
+    for (int rr = 0; rr < STAGES && rr < full_rounds; ++rr) issue_to(rr, rr);
 
   float R[9], t[3];
 #pragma unroll
@@ -245,51 +231,33 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
   };
 
   int since_flush = 0;
-  if constexpr (STAGES > 0) {
-    // stage index and phase parity advance incrementally (no 64-bit division per round)
-    int s = 0;
-    unsigned ph = 0;
-    const float4* st = ring + threadIdx.x;
-    for (int64_t r = 0; r < full_rounds; ++r) {
-      mbar_wait(&s_full[s], ph);
-      float4 v[U][6];
+  // stage index and phase parity advance incrementally (no 64-bit division per round)
+  int s = 0;
+  unsigned ph = 0;
+  const float4* st = ring + threadIdx.x;
+  for (int64_t r = 0; r < full_rounds; ++r) {
+    mbar_wait(&s_full[s], ph);
+    float4 v[U][6];
 #pragma unroll
-      for (int u = 0; u < U; ++u)
+    for (int u = 0; u < U; ++u)
 #pragma unroll
-        for (int k = 0; k < 6; ++k) v[u][k] = st[(s * 6 + k) * CHUNK + u * THREADS];
-      // the stage is in registers: hand it back (one arrival per warp), thread 0 refills it for round r + STAGES
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&s_empty[s]);
-      if (threadIdx.x == 0 && r + STAGES < full_rounds) {
-        mbar_wait(&s_empty[s], ph);
-        issue_to(r + STAGES, s);
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) consume(v[u]);
-      if (++since_flush >= FLUSH_ROUNDS) {
-        flush();
-        since_flush = 0;
-      }
-      if (++s == STAGES) {
-        s = 0;
-        ph ^= 1u;
-      }
+      for (int k = 0; k < 6; ++k) v[u][k] = st[(s * 6 + k) * CHUNK + u * THREADS];
+    // the stage is in registers: hand it back (one arrival per warp), thread 0 refills it for round r + STAGES
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&s_empty[s]);
+    if (threadIdx.x == 0 && r + STAGES < full_rounds) {
+      mbar_wait(&s_empty[s], ph);
+      issue_to(r + STAGES, s);
     }
-  } else {
-    for (int64_t r = 0; r < full_rounds; ++r) {
-      if (PF > 0) prefetch_round(r + PF);
-      const int64_t g = r * stride + int64_t(blockIdx.x) * CHUNK + threadIdx.x;
-      float4 v[U][6];
 #pragma unroll
-      for (int u = 0; u < U; ++u)
-#pragma unroll
-        for (int k = 0; k < 6; ++k) v[u][k] = ld_stream(reinterpret_cast<const float4*>(sp[k]) + g + u * THREADS);
-#pragma unroll
-      for (int u = 0; u < U; ++u) consume(v[u]);
-      if (++since_flush >= FLUSH_ROUNDS) {
-        flush();
-        since_flush = 0;
-      }
+    for (int u = 0; u < U; ++u) consume(v[u]);
+    if (++since_flush >= FLUSH_ROUNDS) {
+      flush();
+      since_flush = 0;
+    }
+    if (++s == STAGES) {
+      s = 0;
+      ph ^= 1u;
     }
   }
   {  // ragged remainder (< one grid round of groups) + scalar tail (n % 4 residuals)

@@ -1,6 +1,4 @@
 // Instantiations + dispatch of the wide pass kernel (mopt_pass.cuh): models with more than 32 packed sums.
-#include <cstdlib>
-
 #include "mopt_internal.h"
 #include "mopt_pass_wide_tc.cuh"
 
@@ -11,67 +9,29 @@ constexpr int kThreads = 256;
 
 template <class M, typename ST, typename CT, bool AFFINE_FD>
 int launch_one(const PassLaunch& L, const PassArgs& a) {
-  auto kern = wide_pass_kernel<M, ST, CT, kThreads, true, AFFINE_FD>;
+  constexpr auto kern = wide_pass_kernel<M, ST, CT, kThreads, true, AFFINE_FD>;
   constexpr size_t smem = wide_smem_bytes<M, CT, kThreads>();
-  // function attributes are per device: opt in to the large dynamic shared-memory tile once on each
-  static bool configured[64] = {false};
-  int dev = 0;
-  MOPT_CUDA_TRY(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    MOPT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
-  int occ = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kThreads, smem) != cudaSuccess || occ < 1) occ = 1;
-  int64_t grid = int64_t(occ) * L.num_sms;
-  const int64_t need = (a.n + kThreads - 1) / kThreads;  // one residual per lane per sweep
-  if (need < grid) grid = need;
-  if (grid < 1) grid = 1;
-  if (grid > kMaxGrid) grid = kMaxGrid;
-  kern<<<int(grid), kThreads, smem, L.stream>>>(a);
+  MOPT_TRY(allow_dyn_smem<kern>(smem));  // the large dynamic shared-memory tile
+  PassLaunch L2 = L;
+  L2.ctas_per_sm = 0;
+  const int grid = pick_grid(reinterpret_cast<const void*>(kern), kThreads, L2, a.n, smem);  // one residual per lane per sweep
+  kern<<<grid, kThreads, smem, L.stream>>>(a);
   MOPT_CUDA_TRY(cudaGetLastError());
   return MOPT_OK;
 }
 
 // Second generation, fp32 only: packed-fp32 finite differences + Gram matrix on the tensor cores (mopt_pass_wide_tc.cuh).
-template <class M, int FLUSH>
-int launch_tc_flush(const PassLaunch& L, const PassArgs& a) {
-  constexpr int kTcThreads = 256;
-  auto kern = wide_tc_kernel<M, kTcThreads, 2, FLUSH>;
-  constexpr size_t smem = wide_tc_smem_bytes(M::O, M::SETN, M::P, kTcThreads);
-  static bool configured[64] = {false};
-  int dev = 0;
-  MOPT_CUDA_TRY(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    MOPT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
-  int occ = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kTcThreads, smem) != cudaSuccess || occ < 1) occ = 1;
-  if (L.ctas_per_sm > 0 && L.ctas_per_sm < occ) occ = L.ctas_per_sm;
-  int64_t grid = int64_t(occ) * L.num_sms;
-  const int64_t need = (a.n + 2 * kTcThreads - 1) / (2 * kTcThreads);  // two observations per lane per sweep
-  if (need < grid) grid = need;
-  if (grid < 1) grid = 1;
-  if (grid > kMaxGrid) grid = kMaxGrid;
-  static const bool prefetch = [] {  // MOPT_WIDE_TC_PREFETCH=0: load the observations where they are used (A/B)
-    const char* e = getenv("MOPT_WIDE_TC_PREFETCH");
-    return !(e && e[0] == '0');
-  }();
-  PassArgs aa = a;
-  aa.no_ring = prefetch ? 0 : 1;  // (the field belongs to the point2point ring kernel; unused by this one otherwise)
-  kern<<<int(grid), kTcThreads, smem, L.stream>>>(aa);
-  MOPT_CUDA_TRY(cudaGetLastError());
-  return MOPT_OK;
-}
-
 template <class M>
 int launch_tc(const PassLaunch& L, const PassArgs& a) {
-  static const int flush = [] {  // experiment knob: MOPT_WIDE_TC_FLUSH=1 / 2 folds the fp32 accumulators into fp64 more often than every 4 groups
-    const char* e = getenv("MOPT_WIDE_TC_FLUSH");
-    return (e && e[0]) ? atoi(e) : 4;
-  }();
-  return flush >= 4 ? launch_tc_flush<M, 4>(L, a) : (flush >= 2 ? launch_tc_flush<M, 2>(L, a) : launch_tc_flush<M, 1>(L, a));
+  constexpr int kTcThreads = 256;
+  constexpr auto kern = wide_tc_kernel<M, kTcThreads, 2>;
+  constexpr size_t smem = wide_tc_smem_bytes(M::O, M::SETN, M::P, kTcThreads);
+  MOPT_TRY(allow_dyn_smem<kern>(smem));
+  // two observations per lane per sweep
+  const int grid = pick_grid(reinterpret_cast<const void*>(kern), kTcThreads, L, (a.n + 1) / 2, smem);
+  kern<<<grid, kTcThreads, smem, L.stream>>>(a);
+  MOPT_CUDA_TRY(cudaGetLastError());
+  return MOPT_OK;
 }
 
 template <class M>

@@ -107,7 +107,7 @@ __host__ __device__ constexpr size_t wide_tc_smem_bytes(int O, int setn, int P, 
   return size_t(4) * (size_t(threads / 32) * wide_tc_cols(P) * wide_tc_row(O) + size_t(1 + 2 * P) * ((setn + 3) / 4 * 4) + P) + 16;
 }
 
-template <class M, int THREADS, int MINB, int FLUSH_GROUPS = 4>
+template <class M, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a) {
   const int mode = a.mode_override >= 0 ? a.mode_override : *a.mode_ptr;
   if (mode == PASS_SKIP) return;
@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a
   constexpr int NW = THREADS / 32;
   constexpr int ROW = wide_tc_row(O);
   constexpr int KSTEPS = 8 * O;                 // k-steps of 8 residual rows over the warp's 64 observations
-  // FLUSH_GROUPS: the fp32 accumulators are folded into fp64 every FLUSH_GROUPS * 64 observations
+  constexpr int FLUSH_GROUPS = 4;               // the fp32 accumulators are folded into fp64 every 4 * 64 observations
   constexpr int NSETS = 1 + 2 * P;
   constexpr int SETN = (M::SETN + 3) / 4 * 4;
   constexpr int S1P = WideStage<M>::PARAMS;
@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a
   F2 e_next[NS];
   {
     const int64_t g_first = int64_t(blockIdx.x) * NW + warp;
-    if (g_first < ngroups && !a.no_ring) load_obs(g_first, e_next);
+    if (g_first < ngroups) load_obs(g_first, e_next);
   }
   for (int64_t g = int64_t(blockIdx.x) * NW + warp; g < ngroups; g += wstride) {
     const int64_t i0 = g * 64 + 2 * lane;
@@ -216,7 +216,6 @@ __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a
     F2 e[NS];
 #pragma unroll
     for (int s = 0; s < NS; ++s) e[s] = e_next[s];
-    if (a.no_ring) load_obs(g, e);  // A/B switch (MOPT_WIDE_TC_PREFETCH=0): load at the point of use
     F2 r[O], tmp[NTMP], s0[SETN];
     load_set(0, s0);
     if constexpr (S1P < P) {
@@ -275,7 +274,7 @@ __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a
 #pragma unroll
       for (int o = 0; o < O; ++o) *reinterpret_cast<float2*>(my + (kWideTcCols - 1) * ROW + o * 64) = (sw * r[o]).v;
       __syncwarp();
-      if (g + wstride < ngroups && !a.no_ring) load_obs(g + wstride, e_next);
+      if (g + wstride < ngroups) load_obs(g + wstride, e_next);
       // ---- 2. Gram matrix of the tile on the tensor cores: C += X^T X, 3 x TF32 ------------------------------
       // The tensor core's fp32 accumulation truncates: a chain of n dependent MMAs on one accumulator biases a sum of
       // same-signed products (the diagonal of H) low by ~n * 2^-25 relative (measured: 5.3e-6 / 3.2e-6 / 2.3e-6 of
@@ -313,7 +312,7 @@ __global__ void __launch_bounds__(THREADS, MINB) wide_tc_kernel(const PassArgs a
           for (int q = 0; q < 4; ++q) cs[t][q] += ps[t][q];
       }
       __syncwarp();
-    } else if (g + wstride < ngroups && !a.no_ring) {
+    } else if (g + wstride < ngroups) {
       load_obs(g + wstride, e_next);  // cost-only pass: no tensor-core phase to put the loads in front of
     }
     if (++since_flush >= FLUSH_GROUPS) {

@@ -279,8 +279,7 @@ __device__ inline void setup_p2p_affine(const CostDev& c, const double* x, doubl
 struct SetupEarlyOpen {
   unsigned long long* rt_words;
   unsigned long long value;  // (barrier target << 2) | PassMode
-  int* opened;      // shared memory
-  long long* prof;  // optional clock64 stamps (slot 11: published)
+  int* opened;  // shared memory
 };
 __device__ inline void setup_p2p_analytical_warp(const CostDev& c, const double* x, ParamBlock* pb, int lane, double* Jl,
                                                  const SetupEarlyOpen* early);
@@ -403,10 +402,7 @@ __device__ inline void setup_p2p_analytical_warp(const CostDev& c, const double*
     for (int i = 1; i < 9; ++i) v = (idx == i) ? R[i] : v;
     v = (idx == 9) ? xs[0] : (idx == 10 ? xs[1] : (idx == 11 ? xs[2] : v));
     publish_rt(early->rt_words, early->value, v, lane);
-    if (lane == 0) {
-      *early->opened = 1;
-      if (early->prof) early->prof[11] = clock64();
-    }
+    if (lane == 0) *early->opened = 1;
   }
 #pragma unroll
   for (int i = 0; i < 9; ++i) J[i] = (i % 4 == 0) ? 1.0 : 0.0;

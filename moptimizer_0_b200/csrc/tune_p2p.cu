@@ -120,9 +120,9 @@ float time_sustained(Env& E, F launch) {
   return t / g_sustained_reps;
 }
 
-template <int THREADS, int MINB, int UNROLL, int FLUSH, int PF = 0, bool SWP = false, int LOSS = MOPT_LOSS_HUBER>
+template <int THREADS, int MINB, int UNROLL, int FLUSH, int LOSS = MOPT_LOSS_HUBER>
 void run_variant(Env& E, int ctas_per_sm, int mode = PASS_LINEARIZE) {
-  auto kern = p2p_moment_kernel<float, float, LOSS, true, THREADS, MINB, UNROLL, FLUSH, PF, SWP>;
+  auto kern = p2p_moment_kernel<float, float, LOSS, true, THREADS, MINB, UNROLL, FLUSH>;
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, 0));
   cudaFuncAttributes fa;
@@ -136,20 +136,20 @@ void run_variant(Env& E, int ctas_per_sm, int mode = PASS_LINEARIZE) {
   const float ms = time_launch(E, [&] { kern<<<grid, THREADS, 0, E.stream>>>(a); });
   const float sus = time_sustained(E, [&] { kern<<<grid, THREADS, 0, E.stream>>>(a); });
   const double gbs = 24.0 * double(a.n) / (ms * 1e-3) / 1e9;
-  std::printf("moment%s threads=%3d minb=%d unroll=%d flush=%2d pf=%2d ctas/sm=%d regs=%3d occ=%d  %8.1f us  %7.1f GB/s  %6.1f Gres/s",
-              SWP ? "/swp" : "    ", THREADS, MINB, UNROLL, FLUSH, PF, per_sm, fa.numRegs, occ, ms * 1e3, gbs, gbs / 24.0);
+  std::printf("moment threads=%3d minb=%d unroll=%d flush=%2d ctas/sm=%d regs=%3d occ=%d  %8.1f us  %7.1f GB/s  %6.1f Gres/s",
+              THREADS, MINB, UNROLL, FLUSH, per_sm, fa.numRegs, occ, ms * 1e3, gbs, gbs / 24.0);
   if (sus > 0.f) std::printf("   sustained %8.1f us %6.1f Gres/s", sus * 1e3, double(a.n) / (sus * 1e-3) / 1e9);
   std::printf("\n");
   std::fflush(stdout);
 }
 
 
-// second-generation kernel (mopt_pass_p2p2.cuh): packed fp32 + TMA bulk-copy ring (STAGES > 0) or direct loads
-template <int THREADS, int MINB, int STAGES, int U, int FLUSH, int PF = 0, int LOSS = MOPT_LOSS_HUBER, bool FUSED = false>
+// second-generation kernel (mopt_pass_p2p2.cuh): packed fp32 + TMA bulk-copy ring
+template <int THREADS, int MINB, int STAGES, int U, int FLUSH, int LOSS = MOPT_LOSS_HUBER, bool FUSED = false>
 void run_variant2(Env& E, int ctas_per_sm, int mode = PASS_LINEARIZE) {
-  auto kern = p2p_moment2_kernel<LOSS, true, false, FUSED, THREADS, MINB, STAGES, U, FLUSH, PF>;
+  auto kern = p2p_moment2_kernel<LOSS, true, false, FUSED, THREADS, MINB, STAGES, U, FLUSH>;
   const size_t smem = p2p2_ring_bytes(THREADS, STAGES, U);
-  if (smem > 0) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, smem));
   cudaFuncAttributes fa;
@@ -166,8 +166,8 @@ void run_variant2(Env& E, int ctas_per_sm, int mode = PASS_LINEARIZE) {
   const float ms = time_launch(E, [&] { kern<<<grid, THREADS, smem, E.stream>>>(a); });
   const float sus = time_sustained(E, [&] { kern<<<grid, THREADS, smem, E.stream>>>(a); });
   const double gbs = 24.0 * double(a.n) / (ms * 1e-3) / 1e9;
-  std::printf("moment2 threads=%4d minb=%d stages=%d u=%d flush=%2d pf=%2d ctas/sm=%d regs=%3d smem=%6zu  %8.1f us  %7.1f GB/s  %6.1f Gres/s",
-              THREADS, MINB, STAGES, U, FLUSH, PF, per_sm, fa.numRegs, smem, ms * 1e3, gbs, gbs / 24.0);
+  std::printf("moment2 threads=%4d minb=%d stages=%d u=%d flush=%2d ctas/sm=%d regs=%3d smem=%6zu  %8.1f us  %7.1f GB/s  %6.1f Gres/s",
+              THREADS, MINB, STAGES, U, FLUSH, per_sm, fa.numRegs, smem, ms * 1e3, gbs, gbs / 24.0);
   if (sus > 0.f) std::printf("   sustained %8.1f us %6.1f Gres/s", sus * 1e3, double(a.n) / (sus * 1e-3) / 1e9);
   std::printf("\n");
   std::fflush(stdout);
@@ -183,7 +183,7 @@ void print_result(Env& E, const char* tag) {
 // fp64-compute variants (the reference's default Scalar is double): ST = float or double streams
 template <typename ST, int THREADS, int MINB, int UNROLL, int FLUSH>
 void run_variant64(Env& E, const PassArgs& a64, int ctas_per_sm) {
-  auto kern = p2p_moment_kernel<ST, double, MOPT_LOSS_HUBER, true, THREADS, MINB, UNROLL, FLUSH, 0, false>;
+  auto kern = p2p_moment_kernel<ST, double, MOPT_LOSS_HUBER, true, THREADS, MINB, UNROLL, FLUSH>;
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, THREADS, 0));
   cudaFuncAttributes fa;
@@ -272,9 +272,9 @@ int main(int argc, char** argv) {
     CK(cudaStreamSynchronize(E.stream));
     PassArgs a = E.a;
     auto k1 = p2p_moment_kernel<float, float, MOPT_LOSS_HUBER, true, 1024, 1, 1, 16>;
-    auto k2 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 512, 1, 2, 2, 16, 0>;
-    auto k3 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 384, 1, 2, 2, 16, 0>;
-    auto k4 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 512, 1, 4, 1, 32, 0>;
+    auto k2 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 512, 1, 2, 2, 16>;
+    auto k3 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 384, 1, 2, 2, 16>;
+    auto k4 = p2p_moment2_kernel<MOPT_LOSS_HUBER, true, false, false, 512, 1, 4, 1, 32>;
     const size_t s2 = p2p2_ring_bytes(512, 2, 2), s3 = p2p2_ring_bytes(384, 2, 2), s4 = p2p2_ring_bytes(512, 4, 1);
     CK(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, int(s2)));
     CK(cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, int(s3)));
@@ -324,10 +324,9 @@ int main(int argc, char** argv) {
       run_variant2<256, 2, 2, 1, 32>(E, 2);
       run_variant2<256, 2, 2, 2, 16>(E, 2);
       run_variant2<192, 2, 2, 2, 16>(E, 2);
-      run_variant2<512, 1, 0, 1, 32, 1>(E, 1);    // direct loads + L2 bulk prefetch
       run_variant2<512, 1, 2, 2, 16>(E, 1, PASS_COST);
       run_variant2<384, 1, 2, 2, 16>(E, 1, PASS_COST);
-      run_variant2<512, 1, 2, 2, 16, 0, MOPT_LOSS_NONE>(E, 1);
+      run_variant2<512, 1, 2, 2, 16, MOPT_LOSS_NONE>(E, 1);
     }
     return 0;
   }
@@ -376,7 +375,7 @@ int main(int argc, char** argv) {
     for (int rep = 0; rep < 3; ++rep) {
       run_ceiling<256, 4>(E, 3);
       run_variant<1024, 1, 1, 16>(E, 1);
-      run_variant<1024, 1, 1, 16, 0, false, MOPT_LOSS_NONE>(E, 1);
+      run_variant<1024, 1, 1, 16, MOPT_LOSS_NONE>(E, 1);
       run_variant<1024, 1, 1, 16>(E, 1, PASS_COST);
       run_variant<256, 2, 2, 16>(E, 2);
       run_variant<256, 2, 2, 16>(E, 2, PASS_COST);
@@ -390,19 +389,5 @@ int main(int argc, char** argv) {
   run_variant<256, 2, 2, 8>(E, 2);   // shipped shape
   run_variant<256, 2, 2, 16>(E, 2);
   run_variant<1024, 1, 1, 16>(E, 1);
-  run_variant<256, 2, 2, 16, 2>(E, 2);
-  // software-pipelined variants
-  run_variant<256, 2, 1, 16, 0, true>(E, 2);
-  run_variant<256, 2, 1, 32, 0, true>(E, 2);
-  run_variant<256, 3, 1, 16, 0, true>(E, 3);
-  run_variant<512, 1, 1, 16, 0, true>(E, 1);
-  run_variant<512, 2, 1, 16, 0, true>(E, 2);
-  run_variant<128, 4, 1, 16, 0, true>(E, 4);
-  run_variant<128, 5, 1, 16, 0, true>(E, 5);
-  run_variant<128, 6, 1, 16, 0, true>(E, 6);
-  run_variant<1024, 1, 1, 16, 0, true>(E, 1);
-  run_variant<256, 2, 1, 16, 2, true>(E, 2);
-  run_variant<256, 2, 1, 16, 4, true>(E, 2);
-  run_variant<256, 3, 1, 16, 2, true>(E, 3);
   return 0;
 }

@@ -1,6 +1,6 @@
 """Exp-curve fit, 10 M samples, central / forward fp32: dense_f2_kernel with the model's series-form difference quotient
-(MOPT_DENSE_F2_SHAPE selects the launch shape) against the literal form (MOPT_FLAG_GENERIC_KERNEL) — time per pass and
-H, b against fp64 compute with the analytical Jacobian."""
+against the literal form (MOPT_FLAG_GENERIC_KERNEL) — time per pass and H, b against fp64 compute with the analytical
+Jacobian."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -15,7 +15,7 @@ st.generate(seed=1, gt=[0.3, 0.1], lo=(0, 0, 0), hi=(5, 0, 0), n_total=n, noise_
 x = np.array([0.25, 0.15])
 H, b, s = ctx.linearize(st, capi.make_problem(capi.MODEL_EXP_CURVE, capi.JAC_ANALYTICAL, capi.F64), x)
 for jac, jn in ((capi.JAC_CENTRAL, "central"), (capi.JAC_FORWARD, "forward")):
-    for tag, flags in (("series form, shape %s" % os.environ.get("MOPT_DENSE_F2_SHAPE", "0"), 0), ("literal form", capi.FLAG_GENERIC_KERNEL)):
+    for tag, flags in (("series form", 0), ("literal form", capi.FLAG_GENERIC_KERNEL)):
         prob = capi.make_problem(capi.MODEL_EXP_CURVE, jac, capi.F32, flags=flags)
         H32, b32, s32 = ctx.linearize(st, prob, x)
         for _ in range(20): ctx.linearize_async(st, prob, x)

@@ -1,5 +1,5 @@
-"""Camera calibration, 6 extrinsics, 50 M observations, central / forward fp32: dense_f2_kernel (MOPT_DENSE_F2_SHAPE
-selects the launch shape) against dense_pass_kernel (set_launch(.., 1024)) — time per pass and H, b against fp64 compute."""
+"""Camera calibration, 6 extrinsics, 50 M observations, central / forward fp32: dense_f2_kernel against
+dense_pass_kernel (set_launch(.., 1024)) — time per pass and H, b against fp64 compute."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -19,7 +19,7 @@ st.generate(seed=3, gt=M.reshape(-1), lo=(2.0, -1.0, -0.5), hi=(5.0, 1.0, 1.0), 
 x = np.array([0.01, -0.01, 0.02, 0.005, 0.003, -0.004])
 for jac, jn in ((capi.JAC_CENTRAL, "central"), (capi.JAC_FORWARD, "forward")):
     H, b, s = ctx.linearize(st, capi.make_problem(capi.MODEL_PINHOLE, jac, capi.F64, consts=consts, flags=capi.FLAG_STABLE_FD), x)
-    for tag, threads in (("dense_f2 shape %s" % os.environ.get("MOPT_DENSE_F2_SHAPE", "0"), 0), ("dense_pass", 1024)):
+    for tag, threads in (("dense_f2", 0), ("dense_pass", 1024)):
         ctx.set_launch(0, threads)
         prob = capi.make_problem(capi.MODEL_PINHOLE, jac, capi.F32, consts=consts)
         H32, b32, s32 = ctx.linearize(st, prob, x)

@@ -1,6 +1,5 @@
 """tst/point2point's cloud (29 310 points, fp64): a few device LM solves, for ncu (launch list / lm_step_kernel source
-page) and for MOPT_LM_MONO_TRACE=1 (per-trial timeline of the persistent kernel on stderr); prints the wall time of
-every solve."""
+page); prints the wall time of every solve."""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -1,6 +1,5 @@
 """n x n calibration case, 50 M observations: the tensor-core Gram kernel against the first-generation kernel and the
-fp64-compute path — time per pass and error of H, b in the scale sqrt(H_ii H_jj).  MOPT_WIDE_TC_FLUSH selects how often
-the fp32 MMA accumulators are folded into fp64 (1, 2 or 4 groups of 64 observations)."""
+fp64-compute path — time per pass and error of H, b in the scale sqrt(H_ii H_jj)."""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -36,7 +35,7 @@ def run(tag, threads, loss=capi.LOSS_NONE, lp=0.0):
     else:
         print(f"{tag}: {ms:.3f} ms (Huber)", flush=True)
     return H32, b32
-run("tensor-core kernel (flush=%s)" % os.environ.get("MOPT_WIDE_TC_FLUSH", "1"), 0)
+run("tensor-core kernel", 0)
 run("first-generation kernel", 1024)
 h1, b1 = run("tensor-core kernel, Huber(2 px)", 0, capi.LOSS_HUBER, 2.0)
 h2, b2 = run("first-generation kernel, Huber(2 px)", 1024, capi.LOSS_HUBER, 2.0)
