@@ -55,6 +55,13 @@ int main(int argc, char** argv) {
     const mopt_eval_stats fit = cost.evaluateStatistics(x0, 0.03);
     std::printf("fitness %.4f (%lld of %ld residuals within 0.03), inlier RMSE %.5f\n", double(fit.n_inliers) / double(n),
                 (long long)fit.n_inliers, n, fit.n_inliers ? std::sqrt(fit.inlier_sum_sq / double(fit.n_inliers)) : 0.0);
+    // how certain the pose is: standard deviations from s^2 H^-1, s^2 estimated from the fit
+    double cov[36];
+    mopt_cov_report rep;
+    lm.computeCovariance(x0, MOPT_COV_SCALED, cov, &rep);
+    std::printf("std (t, omega) = (%.2e %.2e %.2e %.2e %.2e %.2e), rank %d, sigma^2 %.3e\n", std::sqrt(cov[0]),
+                std::sqrt(cov[7]), std::sqrt(cov[14]), std::sqrt(cov[21]), std::sqrt(cov[28]), std::sqrt(cov[35]),
+                rep.rank, rep.sigma2);
     return err < 1e-3 ? 0 : 1;
   } catch (const moptimizer::Exception& e) {
     std::printf("moptimizer::Exception: %s\n", e.what());

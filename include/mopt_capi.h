@@ -300,6 +300,69 @@ MOPT_API int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem*
                            int64_t first, int64_t count, double inlier_threshold, int out_dtype,
                            void* residuals, void* weights, mopt_eval_stats* stats);
 
+/* ---- parameter covariance at a solution ------------------------------------------------------- */
+/* How certain is x?  Two calls: mopt_covariance_terms streams the stores on the device and returns ADDITIVE terms;
+ * mopt_covariance_from_terms (host only) turns terms into a P x P covariance.  The caller of a sharded problem sums
+ * the terms of its ranks between the two calls (every field but num_parameters adds), as it does with
+ * mopt_eval_stats: the device part is rank-local and runs no collective. */
+typedef enum mopt_cov_estimator {
+  MOPT_COV_UNSCALED = 0, /* H^+: the cost terms' covariance matrices (setCovariance) already are the inverse noise covariances */
+  MOPT_COV_SCALED = 1,   /* s^2 H^+, s^2 = wsse / (m - rank): noise level estimated from the fit (scipy curve_fit's pcov) */
+  MOPT_COV_SANDWICH = 2  /* H^+ G H^+ (HC0): robust to a mis-specified noise model, heteroscedasticity and IRLS weights */
+} mopt_cov_estimator;
+
+typedef struct mopt_cov_terms { /* every field adds across cost terms and across the ranks of a sharded problem */
+  int32_t num_parameters;       /* P (not added: must agree) */
+  int32_t reserved0;
+  int64_t n_valid;              /* elements that have a residual (ICP elements without a correspondence excluded) */
+  int64_t m;                    /* residual components: sum over cost terms of n_valid * O */
+  double H[MOPT_MAX_PARAMETERS * MOPT_MAX_PARAMETERS]; /* sum w J^T C J, P x P column-major: what mopt_linearize returns */
+  double G[MOPT_MAX_PARAMETERS * MOPT_MAX_PARAMETERS]; /* sum g g^T, g = w J^T C r, P x P column-major */
+  double b[MOPT_MAX_PARAMETERS]; /* sum g: mopt_linearize's b */
+  double wsse;                  /* sum w r^T C r */
+  double sum_sq;                /* sum r^T r: mopt_linearize's sum */
+  double reserved[4];
+} mopt_cov_terms;               /* H and G fill their first P*P entries (leading dimension P); the rest is 0 */
+
+typedef struct mopt_cov_report {
+  int32_t rank;                 /* eigenvalues of the scaled H kept (see mopt_covariance_from_terms) */
+  int32_t reserved0;
+  int64_t dof;                  /* m - rank */
+  double sigma2;                /* s^2 = wsse / dof (computed for every estimator, used by MOPT_COV_SCALED) */
+  double eig_min, eig_max;      /* smallest kept / largest eigenvalue of the Jacobi-scaled H */
+  double reserved[3];
+} mopt_cov_report;
+
+/* Terms at x of n_costs cost terms sharing x (same P), on the device.  x is a host pointer.
+ *   - H, b, sum_sq come from the linearization pass kernels, accumulated over the cost terms in order as
+ *     mopt_lm_minimize does; for one cost term on an unsharded context they are bit-identical to mopt_linearize's.
+ *   - G, wsse and n_valid come from one more streaming sweep per cost term (score_gram_kernel).  Its Jacobian of
+ *     each residual is the one the linearization of the same problem and flags uses (the affine point2point form, the
+ *     common-denominator finite differences of the camera models and of the exp curve where those are selected, the
+ *     per-residual differences or the model's f_df otherwise), so that G and H describe the same linearization.
+ *     Sums in fp64 (fp32 compute: fp32 partials folded into fp64 as the passes do), reduced in a fixed order:
+ *     identical bits from run to run.
+ *   - Never re-associates (as mopt_evaluate): a store with a target index is taken with the correspondences it holds.
+ *   - Sharded contexts: this rank's stores only, no collective.  Returns after the context stream is synchronised.
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for n_costs outside [1, MOPT_MAX_COSTS], a store of another
+ * context, a null x, a model without parameters or cost terms whose P differ. */
+MOPT_API int mopt_covariance_terms(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, const mopt_problem* problems,
+                                   const double* x, mopt_cov_terms* out);
+/* Host only, needs no GPU: the P x P column-major covariance of x (in the tangent space at x for
+ * MOPT_MANIFOLD_SO3_LEFT) from terms.
+ *   - Pseudo-inverse: D = diag(H)^(-1/2) (0 for a zero diagonal entry: that parameter is unobservable), S = D H D,
+ *     symmetric eigendecomposition of S by cyclic Jacobi in fp64, eigenvalues lambda > rcond * lambda_max kept,
+ *     H^+ = D S^+ D with S^+ the truncated inverse.  For a full-rank H this is H^-1 up to rounding.  rcond = 0
+ *     selects 1e-10; problems with fp32 compute and a near-null direction want about 1e-6.
+ *   - MOPT_COV_UNSCALED returns H^+, MOPT_COV_SCALED sigma2 H^+ (sigma2 = wsse / dof, dof = m - rank),
+ *     MOPT_COV_SANDWICH H^+ G H^+ with no small-sample factor.  The bread is the Gauss-Newton H the LM iterates with;
+ *     for robust losses that is the usual IRLS approximation of the M-estimator's sandwich.
+ *   - `report` may be NULL.
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for num_parameters outside [1, MOPT_MAX_PARAMETERS], an unknown
+ * estimator, a negative rcond, non-finite terms or dof <= 0. */
+MOPT_API int mopt_covariance_from_terms(const mopt_cov_terms* terms, int estimator, double rcond, double* cov,
+                                        mopt_cov_report* report);
+
 /* End-to-end convenience: upload host AoS data (group A and B) into `store` and linearize, with the
  * host->device copies chunked and overlapped with the device work. */
 MOPT_API int mopt_upload_and_linearize(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const void* host_a,

@@ -70,6 +70,21 @@ class CostFunctionBase {
     return stats;
   }
 
+  /// New: additive covariance terms of this cost at x (mopt_covariance_terms): H, b, sum r^T r of the linearization,
+  /// the score Gram matrix G, wsse and the counts.  Terms of several costs, or of the ranks of a sharded problem,
+  /// add field by field before mopt_covariance_from_terms.  Correspondences are not re-associated.
+  mopt_cov_terms covarianceTerms(const Scalar* x) const {
+    mopt_problem p;
+    device::Store::Ptr st;
+    deviceProblem(&p, &st);
+    double xd[MOPT_MAX_PARAMETERS] = {0};
+    for (int i = 0; i < p.num_parameters && x; ++i) xd[i] = double(x[i]);
+    mopt_store* raw = st->get();
+    mopt_cov_terms terms;
+    device::check(mopt_covariance_terms(st->context()->get(), 1, &raw, &p, xd, &terms), "mopt_covariance_terms");
+    return terms;
+  }
+
  protected:
   void fillDeviceProblem(int num_parameters, int num_outputs, int jacobian, mopt_problem* p,
                          device::Store::Ptr* store) const {

@@ -55,21 +55,44 @@ class Optimizer {
   virtual OptimizationStatus step(Scalar* x0) = 0;
   virtual OptimizationStatus minimize(Scalar* x0) = 0;
 
+  /// New: the P x P covariance of x (column-major; tangent space at x for MOPT_MANIFOLD_SO3_LEFT) from every cost
+  /// added, with `estimator` a mopt_cov_estimator (MOPT_COV_SCALED: s^2 H^-1 as scipy's curve_fit reports it).
+  /// Built from the same device problems minimize() gathers, but without cost->update(x): the correspondences the
+  /// stores hold now are used.  Rank-deficient problems get the truncated pseudo-inverse (report->rank).
+  void computeCovariance(const Scalar* x, int estimator, Scalar* cov, mopt_cov_report* report = nullptr) const {
+    checkCosts();
+    std::vector<mopt_problem> problems;
+    std::vector<device::Store::Ptr> stores;
+    std::vector<mopt_store*> raw;
+    gatherDeviceProblems(x, &problems, &stores, &raw, /*update=*/false);
+    const int P = problems[0].num_parameters;
+    double xd[MOPT_MAX_PARAMETERS] = {0};
+    for (int i = 0; i < P; ++i) xd[i] = double(x[i]);
+    mopt_cov_terms terms;
+    device::check(mopt_covariance_terms(stores[0]->context()->get(), int(raw.size()), raw.data(), problems.data(), xd,
+                                        &terms),
+                  "mopt_covariance_terms");
+    double out[MOPT_MAX_PARAMETERS * MOPT_MAX_PARAMETERS];
+    device::check(mopt_covariance_from_terms(&terms, estimator, 0.0, out, report), "mopt_covariance_from_terms");
+    for (int i = 0; i < P * P; ++i) cov[i] = Scalar(out[i]);
+  }
+
  protected:
   virtual bool hasConverged() = 0;
   virtual void prepare(Scalar* x0) = 0;
 
-  /// cost->update(x0) for every cost (levenberg_marquadt_dyn.cpp:54), then their device descriptions.  Throws if a
-  /// cost is not device-backed, if there are more than MOPT_MAX_COSTS, or if they live on different contexts.
+  /// cost->update(x0) for every cost (levenberg_marquadt_dyn.cpp:54; skipped with update = false), then their device
+  /// descriptions.  Throws if a cost is not device-backed, if there are more than MOPT_MAX_COSTS, or if they live on
+  /// different contexts.
   void gatherDeviceProblems(const Scalar* x0, std::vector<mopt_problem>* problems, std::vector<device::Store::Ptr>* stores,
-                            std::vector<mopt_store*>* raw) const {
+                            std::vector<mopt_store*>* raw, bool update = true) const {
     const size_t n = costs_.size();
     if (n > size_t(MOPT_MAX_COSTS)) throw Exception("Optimizer: too many cost functions for the device path");
     problems->resize(n);
     stores->resize(n);
     raw->resize(n);
     for (size_t i = 0; i < n; ++i) {
-      costs_[i]->update(x0);
+      if (update) costs_[i]->update(x0);
       costs_[i]->deviceProblem(&(*problems)[i], &(*stores)[i]);
       (*raw)[i] = (*stores)[i]->get();
       if ((*stores)[i]->context() != (*stores)[0]->context())

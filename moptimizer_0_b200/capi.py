@@ -28,6 +28,7 @@ FLAG_STABLE_FD = 2
 FLAG_REFERENCE_FLOAT_GUARD = 4
 LM_STAGNATION_STOP = 1
 LOSS_NONE, LOSS_GEMAN_MCCLURE, LOSS_HUBER = range(3)
+COV_UNSCALED, COV_SCALED, COV_SANDWICH = range(3)
 STATUS = ["CONVERGED", "MAXIMUM_ITERATIONS_REACHED", "SMALL_DELTA", "NUMERIC_ERROR", "FATAL_ERROR"]
 MODEL_SHAPE = {  # model -> (P, O, ncomp_a, ncomp_b)
     MODEL_POINT2POINT: (6, 3, 3, 3), MODEL_EXP_CURVE: (2, 1, 1, 1), MODEL_MICHAELIS_MENTEN: (2, 1, 1, 1),
@@ -46,7 +47,7 @@ EXPORTS = [
     "mopt_nn_index_create", "mopt_nn_index_destroy", "mopt_store_set_target", "mopt_store_reassociate",
     "mopt_ctx_peer_handle", "mopt_ctx_open_peers", "mopt_ctx_set_exchange_enabled",
     "mopt_user_model_compile", "mopt_user_model_release", "mopt_user_model_log",
-    "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate",
+    "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate", "mopt_covariance_terms", "mopt_covariance_from_terms",
 ]
 MODEL_USER_BASE = 1000
 PEER_HANDLE_BYTES = 64
@@ -107,6 +108,91 @@ class EvalStats(C.Structure):
 mopt_eval_stats = EvalStats  # the C name
 
 
+class CovTermsStruct(C.Structure):
+    _fields_ = [("num_parameters", C.c_int32), ("reserved0", C.c_int32), ("n_valid", C.c_int64), ("m", C.c_int64),
+                ("H", C.c_double * (MAX_PARAMETERS * MAX_PARAMETERS)),
+                ("G", C.c_double * (MAX_PARAMETERS * MAX_PARAMETERS)), ("b", C.c_double * MAX_PARAMETERS),
+                ("wsse", C.c_double), ("sum_sq", C.c_double), ("reserved", C.c_double * 4)]
+
+
+class CovReport(C.Structure):
+    _fields_ = [("rank", C.c_int32), ("reserved0", C.c_int32), ("dof", C.c_int64), ("sigma2", C.c_double),
+                ("eig_min", C.c_double), ("eig_max", C.c_double), ("reserved", C.c_double * 3)]
+
+
+mopt_cov_terms, mopt_cov_report = CovTermsStruct, CovReport  # the C names
+
+
+class CovTerms:
+    """mopt_cov_terms with numpy views: `H`, `G` (P x P), `b` (P) and the scalars.  Terms add (`+`): sum the terms of
+    cost groups, or of the ranks of a sharded problem, before covariance_from_terms."""
+
+    def __init__(self, raw: Optional[CovTermsStruct] = None):
+        self.raw = raw if raw is not None else CovTermsStruct()
+
+    @property
+    def P(self) -> int:
+        return self.raw.num_parameters
+
+    def _mat(self, name):
+        P = self.P
+        return np.ctypeslib.as_array(getattr(self.raw, name))[:P * P].reshape(P, P).T  # column-major
+
+    H = property(lambda self: self._mat("H"))
+    G = property(lambda self: self._mat("G"))
+    b = property(lambda self: np.ctypeslib.as_array(self.raw.b)[:self.P])
+    n_valid = property(lambda self: self.raw.n_valid)
+    m = property(lambda self: self.raw.m)
+    wsse = property(lambda self: self.raw.wsse)
+    sum_sq = property(lambda self: self.raw.sum_sq)
+
+    def __add__(self, other: "CovTerms") -> "CovTerms":
+        if self.P != other.P:
+            raise ValueError(f"terms of different parameter counts ({self.P} and {other.P})")
+        out = CovTermsStruct()
+        out.num_parameters = self.P
+        out.n_valid, out.m = self.n_valid + other.n_valid, self.m + other.m
+        for name in ("H", "G", "b"):
+            np.ctypeslib.as_array(getattr(out, name))[:] = (np.ctypeslib.as_array(getattr(self.raw, name)) +
+                                                            np.ctypeslib.as_array(getattr(other.raw, name)))
+        out.wsse, out.sum_sq = self.wsse + other.wsse, self.sum_sq + other.sum_sq
+        return CovTerms(out)
+
+    @staticmethod
+    def from_arrays(H, G, b, wsse: float, sum_sq: float, n_valid: int, m: int) -> "CovTerms":
+        """Terms assembled on the host (e.g. after summing ranks with torch.distributed.all_reduce)."""
+        H, G, b = (np.asarray(v, dtype=np.float64) for v in (H, G, b))
+        P = b.shape[0]
+        t = CovTermsStruct()
+        t.num_parameters, t.n_valid, t.m, t.wsse, t.sum_sq = P, int(n_valid), int(m), float(wsse), float(sum_sq)
+        np.ctypeslib.as_array(t.H)[:P * P] = H.T.reshape(-1)
+        np.ctypeslib.as_array(t.G)[:P * P] = G.T.reshape(-1)
+        np.ctypeslib.as_array(t.b)[:P] = b
+        return CovTerms(t)
+
+
+class Covariance:
+    """Context.covariance / covariance_from_terms: `cov` (P x P), `std` (sqrt of its diagonal), and the report."""
+
+    def __init__(self, cov: np.ndarray, rep: CovReport):
+        self.cov = cov
+        self.rank, self.dof, self.sigma2 = rep.rank, rep.dof, rep.sigma2
+        self.eig_min, self.eig_max = rep.eig_min, rep.eig_max
+
+    @property
+    def std(self) -> np.ndarray:
+        return np.sqrt(np.diag(self.cov))
+
+
+def covariance_from_terms(terms: CovTerms, estimator: int = COV_SCALED, rcond: float = 0.0) -> Covariance:
+    """mopt_covariance_from_terms (host only): the covariance of x from (summed) terms."""
+    P = terms.P
+    cov = np.zeros(P * P if P > 0 else 1, dtype=np.float64)
+    rep = CovReport()
+    check(lib().mopt_covariance_from_terms(C.byref(terms.raw), int(estimator), float(rcond), _dp(cov), C.byref(rep)))
+    return Covariance(cov[:P * P].reshape(P, P).T.copy(), rep)
+
+
 class MoptError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"mopt error {code}: {msg}")
@@ -147,6 +233,10 @@ def lib():
         L.mopt_measure_peaks.argtypes = [vp, C.POINTER(Peaks)]
         L.mopt_evaluate.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_double, C.c_int, vp, vp,
                                     C.POINTER(EvalStats)]
+        L.mopt_covariance_terms.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), dp,
+                                            C.POINTER(CovTermsStruct)]
+        L.mopt_covariance_from_terms.argtypes = [C.POINTER(CovTermsStruct), C.c_int, C.c_double, dp,
+                                                 C.POINTER(CovReport)]
         L.mopt_measure_h2d.argtypes = [vp, C.c_uint64, C.c_double, dp]
         L.mopt_upload_and_linearize.argtypes = [vp, vp, C.POINTER(Problem), vp, vp, C.c_int, i64, dp, dp, dp, dp]
         L.mopt_lm_minimize.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), C.POINTER(LmOptions), dp,
@@ -349,6 +439,23 @@ class Context:
                                   float(inlier_threshold), out_dtype, r_t.data_ptr() if r_t is not None else None,
                                   w_t.data_ptr() if w_t is not None else None, C.byref(st)))
         return EvalResult(st, count, r_t, w_t)
+
+    def covariance_terms(self, stores: Sequence["Store"], problems: Sequence[Problem], x) -> CovTerms:
+        """mopt_covariance_terms: additive covariance terms (H, G, b, wsse, sum_sq, n_valid, m) of the cost terms at x,
+        this context's stores only.  Never re-associates."""
+        n = len(stores)
+        hs = (C.c_void_p * n)(*[s.handle for s in stores])
+        ps = (Problem * n)(*problems)
+        xs = np.ascontiguousarray(np.asarray(x, dtype=np.float64))
+        out = CovTermsStruct()
+        check(lib().mopt_covariance_terms(self._h, n, hs, ps, _dp(xs), C.byref(out)))
+        return CovTerms(out)
+
+    def covariance(self, stores: Sequence["Store"], problems: Sequence[Problem], x, estimator: int = COV_SCALED,
+                   rcond: float = 0.0) -> Covariance:
+        """Covariance of x (`.cov`, `.std`, `.rank`, `.dof`, `.sigma2`) from this context's stores: the terms on the
+        device, then mopt_covariance_from_terms."""
+        return covariance_from_terms(self.covariance_terms(stores, problems, x), estimator, rcond)
 
     def linearize_async(self, store: "Store", problem: Problem, xs: np.ndarray):
         check(lib().mopt_linearize_async(self._h, store.handle, C.byref(problem), _dp(xs)))

@@ -274,6 +274,15 @@ bool can_fuse_setup(const mopt_ctx* ctx, const mopt_problem* p, const mopt_store
          p->manifold == MOPT_MANIFOLD_ADDITIVE;
 }
 
+PassLaunch pass_launch(const mopt_ctx* ctx, const mopt_problem* p) {
+  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
+  // finite differences over a common denominator (AFFINE_FD): the default with fp32 compute, opt-in with fp64
+  L.affine_fd = (p->compute_dtype == MOPT_F32) ? !(p->flags & MOPT_FLAG_GENERIC_KERNEL)
+                                               : ((p->flags & MOPT_FLAG_STABLE_FD) && !(p->flags & MOPT_FLAG_GENERIC_KERNEL));
+  L.identity_cov = !p->has_covariance;
+  return L;
+}
+
 int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int slot, int accumulate, int mode_override,
                 bool push, const XArg* fused_x = nullptr) {
   PassArgs a = make_args(ctx, st, slot, accumulate, mode_override);
@@ -291,11 +300,7 @@ int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int 
     a.peer.err_dev = ctx->d_xerr_dev;
     a.peer.seq = ++ctx->xseq;
   }
-  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
-  // finite differences over a common denominator (AFFINE_FD): the default with fp32 compute, opt-in with fp64
-  L.affine_fd = (p->compute_dtype == MOPT_F32) ? !(p->flags & MOPT_FLAG_GENERIC_KERNEL)
-                                               : ((p->flags & MOPT_FLAG_STABLE_FD) && !(p->flags & MOPT_FLAG_GENERIC_KERNEL));
-  L.identity_cov = !p->has_covariance;
+  const PassLaunch L = pass_launch(ctx, p);
   if (p->model >= MOPT_MODEL_USER_BASE)
     return launch_user(L, ctx->device, p->model, p->jacobian != MOPT_JAC_ANALYTICAL, st->dtype, p->compute_dtype, a);
   if (p->model == MOPT_MODEL_POINT2POINT && p->jacobian == MOPT_JAC_ANALYTICAL)
@@ -308,6 +313,25 @@ int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int 
     return launch_p2p_moment(L, st->dtype, p->compute_dtype, p->loss, false, a);
   if (p->model == MOPT_MODEL_PINHOLE_DISTORT) return launch_wide(L, p->model, st->dtype, p->compute_dtype, a);
   return launch_dense(L, p->model, p->jacobian != MOPT_JAC_ANALYTICAL, st->dtype, p->compute_dtype, a);
+}
+
+// Score Gram sums (mopt_covariance_terms) of cost term `slot`, staged by setup_slot, into `out`: the Jacobian form
+// launch_pass selects for the same problem (launch_cov picks the common-denominator differences where
+// pass_launch's affine_fd and the model allow them, as launch_dense / launch_wide do).
+int launch_cov_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int slot, double* out) {
+  const PassArgs a = make_args(ctx, st, slot, 0, PASS_LINEARIZE);
+  const PassLaunch L = pass_launch(ctx, p);
+  const bool numeric = p->jacobian != MOPT_JAC_ANALYTICAL;
+  CovArgs cv;
+  cv.out = out;
+  cv.qrot = (!numeric && (p->variant == MOPT_P2P_EXACT || p->variant == MOPT_P2P_LEFT)) ? 1 : 0;
+  if (p->model >= MOPT_MODEL_USER_BASE)
+    return launch_user_cov(L, ctx->device, p->model, numeric, st->dtype, p->compute_dtype, a, cv);
+  int form = numeric ? COV_JAC_FD : COV_JAC_ANALYTICAL;
+  if (p->model == MOPT_MODEL_POINT2POINT &&
+      (!numeric || (!(p->flags & MOPT_FLAG_GENERIC_KERNEL) && !(st->dtype == MOPT_F64 && p->compute_dtype == MOPT_F32))))
+    form = COV_JAC_P2P_AFFINE;
+  return launch_cov(L, p->model, form, st->dtype, p->compute_dtype, a, cv);
 }
 
 // Per-residual evaluation (mopt_evaluate): the builtin or run-time compiled evaluate_kernel of the model, on set 0 of
@@ -492,6 +516,8 @@ int ctx_alloc(mopt_ctx* ctx) {
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_xerr_dev, sizeof(int)));
   MOPT_CUDA_TRY(cudaMemset(ctx->d_xerr_dev, 0, sizeof(int)));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_eval_stats, sizeof(double) * (kEvalSums + 1)));
+  MOPT_CUDA_TRY(cudaMalloc(&ctx->d_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw));
+  MOPT_CUDA_TRY(cudaHostAlloc(&ctx->h_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw, cudaHostAllocDefault));
   ctx->flags_capacity = 4096;
   if (const char* e = getenv("MOPT_LM_FLAG_RING")) {  // test knob: a small ring makes an ordinary solve wrap it
     const int v = atoi(e);
@@ -592,6 +618,8 @@ int mopt_ctx_destroy(mopt_ctx* ctx) try {
   cudaFree(ctx->d_xerr_dev);
   cudaFree(ctx->d_gen);
   cudaFree(ctx->d_eval_stats);
+  cudaFree(ctx->d_cov_sums);
+  if (ctx->h_cov_sums) cudaFreeHost(ctx->h_cov_sums);
   if (ctx->h_xerr) cudaFreeHost(ctx->h_xerr);
   cudaFree(ctx->d_partials); cudaFree(ctx->d_ticket); cudaFree(ctx->d_trial);
   cudaFree(ctx->d_slots); cudaFree(ctx->d_lm);
@@ -736,6 +764,59 @@ int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem,
     stats->inlier_sum_sq = h[3];
     stats->max_sq = h[4];
   }
+  return MOPT_OK;
+}
+MOPT_ABI_CATCH
+
+int mopt_covariance_terms(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, const mopt_problem* problems,
+                          const double* x, mopt_cov_terms* out) try {
+  MOPT_REQUIRE(ctx && stores && problems && out, "null argument");
+  MOPT_REQUIRE(x, "null parameter vector");
+  MOPT_REQUIRE(n_costs >= 1 && n_costs <= MOPT_MAX_COSTS, "n_costs must lie in [1, MOPT_MAX_COSTS]");
+  const int P = problems[0].num_parameters;
+  for (int c = 0; c < n_costs; ++c) {
+    MOPT_REQUIRE(stores[c] && stores[c]->ctx == ctx, "store does not belong to this context");
+    MOPT_REQUIRE(problems[c].num_parameters == P, "all cost terms must share the parameter vector");
+    MOPT_REQUIRE(problems[c].manifold == problems[0].manifold, "all cost terms must use the same manifold");
+    MOPT_TRY(validate_problem(stores[c], &problems[c], true));  // also: a model without parameters
+  }
+  MOPT_TRY(check_exchange_alive(ctx));
+  MOPT_CUDA_TRY(cudaSetDevice(ctx->device));
+  XArg xa;
+  std::memset(&xa, 0, sizeof(xa));
+  for (int i = 0; i < P; ++i) xa.v[i] = x[i];
+  for (int c = 0; c < n_costs; ++c) {
+    const mopt_problem* p = &problems[c];
+    // the ParamBlock of slot c (sets, steps, point2point affine Jacobian pieces): read by the score Gram kernel
+    // even where the linearization pass derives them itself (fused set-up)
+    MOPT_TRY(setup_slot(ctx, c, p, x));
+    // H, b, sum r^T r: the pass mopt_linearize (one cost) / mopt_lm_minimize (several) runs, rank-local
+    if (can_fuse_setup(ctx, p, stores[c])) MOPT_TRY(launch_pass(ctx, stores[c], p, c, c > 0 ? 1 : 0, PASS_LINEARIZE, false, &xa));
+    else MOPT_TRY(launch_pass(ctx, stores[c], p, c, c > 0 ? 1 : 0, PASS_LINEARIZE, false));
+    MOPT_TRY(launch_cov_pass(ctx, stores[c], p, c, ctx->d_cov_sums + size_t(c) * kMaxRaw));
+  }
+  MOPT_CUDA_TRY(cudaMemcpyAsync(ctx->h_result, ctx->d_trial, sizeof(double) * packed_size(P), cudaMemcpyDeviceToHost,
+                                ctx->stream));
+  MOPT_CUDA_TRY(cudaMemcpyAsync(ctx->h_cov_sums, ctx->d_cov_sums, sizeof(double) * size_t(n_costs) * kMaxRaw,
+                                cudaMemcpyDeviceToHost, ctx->stream));
+  MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  mopt_cov_terms t;
+  std::memset(&t, 0, sizeof(t));
+  t.num_parameters = P;
+  unpack_result(*ctx->h_result, P, t.H, t.b, &t.sum_sq);
+  const int nh = P * (P + 1) / 2;
+  double Gp[kMaxP * (kMaxP + 1) / 2] = {0.0};
+  for (int c = 0; c < n_costs; ++c) {  // cost terms in order, as the passes accumulate H
+    const double* v = ctx->h_cov_sums + size_t(c) * kMaxRaw;
+    for (int k = 0; k < nh; ++k) Gp[k] += v[k];
+    t.wsse += v[nh];
+    const int64_t nv = int64_t(v[nh + 1]);
+    t.n_valid += nv;
+    t.m += nv * problems[c].num_outputs;
+  }
+  for (int i = 0; i < P; ++i)
+    for (int j = i; j < P; ++j) t.G[i + j * P] = t.G[j + i * P] = Gp[tri_index(P, i, j)];
+  *out = t;
   return MOPT_OK;
 }
 MOPT_ABI_CATCH

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include "mopt_common.cuh"
+#include "mopt_cov.cuh"
 #include "mopt_eval.cuh"
 #include "mopt_lm.cuh"
 #include "mopt_lm_mono.cuh"
@@ -56,6 +57,8 @@ struct mopt_ctx {
   unsigned long long mono_gen = 0;               // barrier targets handed out so far (monotonic over the context's life)
   int* d_xerr_dev = nullptr;                     // device-resident copy, read by the kernels that follow a failed exchange
   double* d_eval_stats = nullptr;                // mopt_evaluate: the statistics written by the evaluation kernel's last CTA
+  double* d_cov_sums = nullptr;                  // mopt_covariance_terms: [MOPT_MAX_COSTS][kMaxRaw] score Gram totals
+  double* h_cov_sums = nullptr;                  // pinned host copy of the same
 };
 
 struct mopt_store {
@@ -103,11 +106,17 @@ int launch_wide(const PassLaunch& L, int model, int store_dtype, int compute_dty
 int launch_evaluate(const PassLaunch& L, int model, int store_dtype, int compute_dtype, int out_dtype,
                     const PassArgs& a, const EvalArgs& ev);
 
+// mopt_cov.cu: score Gram sums of a builtin model (mopt_covariance_terms); `form` is a CovJac
+int launch_cov(const PassLaunch& L, int model, int form, int store_dtype, int compute_dtype, const PassArgs& a,
+               const CovArgs& cv);
+
 // mopt_rtc.cu: run-time compiled user models (ids >= MOPT_MODEL_USER_BASE)
 int launch_user(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
                 const PassArgs& a);
 int launch_user_evaluate(const PassLaunch& L, int device, int model, int store_dtype, int compute_dtype, int out_dtype,
                          const PassArgs& a, const EvalArgs& ev);
+int launch_user_cov(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
+                    const PassArgs& a, const CovArgs& cv);
 int launch_user_setup(cudaStream_t stream, int device, int model, CostSlot* slot, const double* x_dev,
                       const double* x_host, int P);
 int user_model_rot_offset(int model);
