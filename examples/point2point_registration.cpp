@@ -55,6 +55,10 @@ int main(int argc, char** argv) {
     const mopt_eval_stats fit = cost.evaluateStatistics(x0, 0.03);
     std::printf("fitness %.4f (%lld of %ld residuals within 0.03), inlier RMSE %.5f\n", double(fit.n_inliers) / double(n),
                 (long long)fit.n_inliers, n, fit.n_inliers ? std::sqrt(fit.inlier_sum_sq / double(fit.n_inliers)) : 0.0);
+    // the distribution of the correspondence distances |r| and the robust noise scale, which outliers do not inflate
+    const mopt_quantiles qd = cost.residualQuantiles(x0, {0.5, 0.9});
+    std::printf("correspondence distance: median %.5f, 90th percentile %.5f, robust sigma %.5f\n", std::sqrt(qd.value[0]),
+                std::sqrt(qd.value[1]), qd.robust_sigma);
     // how certain the pose is: standard deviations from s^2 H^-1, s^2 estimated from the fit
     double cov[36];
     mopt_cov_report rep;

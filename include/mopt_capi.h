@@ -300,6 +300,50 @@ MOPT_API int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem*
                            int64_t first, int64_t count, double inlier_threshold, int out_dtype,
                            void* residuals, void* weights, mopt_eval_stats* stats);
 
+/* ---- residual quantiles ----------------------------------------------------------------------- */
+#define MOPT_MAX_QUANTILES 8
+/* Exact order statistics of the keys e_i = r_i^T r_i of one cost term over a range of its store
+ * (mopt_residual_quantiles).  Unlike the counts and sums of mopt_eval_stats, quantiles do NOT combine across the
+ * ranks of a sharded problem: each rank gets the quantiles of its own store. */
+typedef struct mopt_quantiles {
+  int64_t n_ranked;                 /* valid elements of the range whose e_i is not NaN: the sample */
+  int64_t n_nan;                    /* valid elements whose e_i is NaN (not ranked) */
+  double lo[MOPT_MAX_QUANTILES];    /* e_(j),   j = floor(h), h = (n_ranked - 1) * q  (0-based order statistics) */
+  double hi[MOPT_MAX_QUANTILES];    /* e_(j+1), clamped to e_(n_ranked - 1) */
+  double value[MOPT_MAX_QUANTILES]; /* numpy's method="linear" interpolation of lo, hi */
+  double median;                    /* value at q = 0.5, always computed */
+  double robust_sigma;              /* sqrt(median / chi2_median(O)) */
+  double reserved[4];
+} mopt_quantiles;
+
+/* Quantiles of e_i = r_i^T r_i over the elements [first, first + count) of `store` at x, for n_q levels q[0..n_q)
+ * (host arrays), plus the median and the median-based robust scale.  Exact: every lo / hi is one element's e_i.
+ * Returns after the context stream is synchronised.
+ *   - The key.  r_i is the residual mopt_evaluate computes (the model residual in problem.compute_dtype at
+ *     setup(x)).  e_i is summed in the compute dtype in component order, every product and sum rounded separately
+ *     (no fused multiply-add): e = r_0 r_0, then e = e + r_o r_o for o = 1 .. O-1.  mopt_evaluate's residuals written
+ *     with out_dtype = compute_dtype reproduce it exactly; it can differ in the last bit from the FMA-formed r^T r
+ *     behind mopt_eval_stats and the loss weight.  The covariance, loss, jacobian, variant and manifold fields
+ *     have no effect.
+ *   - The sample.  Elements without a correspondence (as in mopt_evaluate) are excluded.  A valid element whose
+ *     e_i is NaN (NaN data) is counted in n_nan and not ranked; +inf is ranked and sorts last.  Never
+ *     re-associates correspondences.
+ *   - Quantiles (q in [0, 1]).  lo, hi and value are what np.quantile(e.astype(np.float64), q) (method "linear")
+ *     takes and returns: h = (n_ranked - 1) q in fp64, j = floor(h), t = h - j, value = lo + (hi - lo) t, or
+ *     hi - (hi - lo)(1 - t) when t >= 0.5.  One difference: value = lo when t = 0 (numpy gives NaN for a finite lo
+ *     next to hi = +inf).
+ *   - robust_sigma = sqrt(median / m_O), m_O the median of the chi-square distribution with O degrees of freedom
+ *     (O = problem.num_outputs): 1.4826 median|r| for O = 1, and a consistent estimate of the per-component sigma
+ *     for isotropic Gaussian noise.
+ *   - An empty sample (n_ranked = 0) returns MOPT_OK with the counts set and every value NaN.
+ *   - Results are exact element values: identical from run to run, whatever the grid or mopt_ctx_set_launch.
+ *   - Sharded contexts: this rank's store only, no collective (see mopt_quantiles).
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for a store of another context, a problem the store does not
+ * accept, a range outside the store, n_q outside [0, MOPT_MAX_QUANTILES], a q that is NaN or outside [0, 1], a
+ * null q with n_q > 0, a null out, or a null x for a model with parameters. */
+MOPT_API int mopt_residual_quantiles(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x,
+                                     int64_t first, int64_t count, int n_q, const double* q, mopt_quantiles* out);
+
 /* ---- parameter covariance at a solution ------------------------------------------------------- */
 /* How certain is x?  Two calls: mopt_covariance_terms streams the stores on the device and returns ADDITIVE terms;
  * mopt_covariance_from_terms (host only) turns terms into a P x P covariance.  The caller of a sharded problem sums

@@ -4,6 +4,7 @@
 
 #include <cstring>
 #include <memory>
+#include <vector>
 
 #include "mopt_capi.h"
 #include "moptimizer/covariance/covariance.h"
@@ -68,6 +69,23 @@ class CostFunctionBase {
                                 nullptr, nullptr, &stats),
                   "mopt_evaluate");
     return stats;
+  }
+
+  /// New: exact quantiles of e = r^T r over all residuals of this cost term at x (mopt_residual_quantiles) for the
+  /// levels qs (at most MOPT_MAX_QUANTILES), plus the median and the robust scale sqrt(median / chi2_median(O)).
+  /// sqrt of a value is the quantile of the residual norm |r|.  Correspondences are not re-associated: call
+  /// update(x) first for fresh ones.
+  mopt_quantiles residualQuantiles(const Scalar* x, const std::vector<double>& qs) const {
+    mopt_problem p;
+    device::Store::Ptr st;
+    deviceProblem(&p, &st);
+    double xd[MOPT_MAX_PARAMETERS] = {0};
+    for (int i = 0; i < p.num_parameters && x; ++i) xd[i] = double(x[i]);
+    mopt_quantiles out;
+    device::check(mopt_residual_quantiles(st->context()->get(), st->get(), &p, xd, 0, st->size(), int(qs.size()),
+                                          qs.empty() ? nullptr : qs.data(), &out),
+                  "mopt_residual_quantiles");
+    return out;
   }
 
   /// New: additive covariance terms of this cost at x (mopt_covariance_terms): H, b, sum r^T r of the linearization,

@@ -16,6 +16,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libmopt_b200.so")
 
 MAX_PARAMETERS, MAX_OUTPUTS, MAX_COSTS, MAX_TRACE, NCCL_ID_BYTES = 16, 4, 8, 1024, 128
+MAX_QUANTILES = 8
 OK = 0
 F32, F64 = 0, 1
 (MODEL_POINT2POINT, MODEL_EXP_CURVE, MODEL_MICHAELIS_MENTEN, MODEL_PINHOLE, MODEL_POWELL,
@@ -48,6 +49,7 @@ EXPORTS = [
     "mopt_ctx_peer_handle", "mopt_ctx_open_peers", "mopt_ctx_set_exchange_enabled",
     "mopt_user_model_compile", "mopt_user_model_release", "mopt_user_model_log",
     "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate", "mopt_covariance_terms", "mopt_covariance_from_terms",
+    "mopt_residual_quantiles",
 ]
 MODEL_USER_BASE = 1000
 PEER_HANDLE_BYTES = 64
@@ -106,6 +108,33 @@ class EvalStats(C.Structure):
 
 
 mopt_eval_stats = EvalStats  # the C name
+
+
+class QuantilesStruct(C.Structure):
+    _fields_ = [("n_ranked", C.c_int64), ("n_nan", C.c_int64), ("lo", C.c_double * MAX_QUANTILES),
+                ("hi", C.c_double * MAX_QUANTILES), ("value", C.c_double * MAX_QUANTILES), ("median", C.c_double),
+                ("robust_sigma", C.c_double), ("reserved", C.c_double * 4)]
+
+
+mopt_quantiles = QuantilesStruct  # the C name
+
+
+class Quantiles:
+    """Context.quantiles: order statistics of e = r^T r.  `lo`, `hi`, `values` (numpy, one per requested q), the
+    `median` of e, `robust_sigma` = sqrt(median / chi2_median(O)), the counts `n_ranked` / `n_nan`, and
+    `norm_values` = sqrt(values), the quantiles of the residual norm |r|."""
+
+    def __init__(self, raw: QuantilesStruct, n_q: int):
+        self.raw = raw
+        self.lo = np.array(raw.lo[:n_q], dtype=np.float64)
+        self.hi = np.array(raw.hi[:n_q], dtype=np.float64)
+        self.values = np.array(raw.value[:n_q], dtype=np.float64)
+        self.median, self.robust_sigma = raw.median, raw.robust_sigma
+        self.n_ranked, self.n_nan = raw.n_ranked, raw.n_nan
+
+    @property
+    def norm_values(self) -> np.ndarray:
+        return np.sqrt(self.values)
 
 
 class CovTermsStruct(C.Structure):
@@ -233,6 +262,8 @@ def lib():
         L.mopt_measure_peaks.argtypes = [vp, C.POINTER(Peaks)]
         L.mopt_evaluate.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_double, C.c_int, vp, vp,
                                     C.POINTER(EvalStats)]
+        L.mopt_residual_quantiles.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_int, dp,
+                                              C.POINTER(QuantilesStruct)]
         L.mopt_covariance_terms.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), dp,
                                             C.POINTER(CovTermsStruct)]
         L.mopt_covariance_from_terms.argtypes = [C.POINTER(CovTermsStruct), C.c_int, C.c_double, dp,
@@ -439,6 +470,21 @@ class Context:
                                   float(inlier_threshold), out_dtype, r_t.data_ptr() if r_t is not None else None,
                                   w_t.data_ptr() if w_t is not None else None, C.byref(st)))
         return EvalResult(st, count, r_t, w_t)
+
+    def quantiles(self, store: "Store", problem: Problem, x, q=(), first: int = 0,
+                  count: Optional[int] = None) -> Quantiles:
+        """mopt_residual_quantiles: exact quantiles (numpy's method="linear") of e = r^T r over the elements
+        [first, first + count) at x, for the levels q (at most MAX_QUANTILES), plus the median and the robust scale.
+        This context's store only; never re-associates."""
+        count = store.n - first if count is None else int(count)
+        qs = np.ascontiguousarray(np.asarray(q, dtype=np.float64).reshape(-1))
+        if qs.size > MAX_QUANTILES:
+            raise ValueError(f"at most {MAX_QUANTILES} quantile levels, got {qs.size}")
+        xs = np.ascontiguousarray(np.asarray(x if len(x) else [0.0], dtype=np.float64))
+        out = QuantilesStruct()
+        check(lib().mopt_residual_quantiles(self._h, store.handle, C.byref(problem), _dp(xs), int(first), count,
+                                            int(qs.size), _dp(qs) if qs.size else None, C.byref(out)))
+        return Quantiles(out, int(qs.size))
 
     def covariance_terms(self, stores: Sequence["Store"], problems: Sequence[Problem], x) -> CovTerms:
         """mopt_covariance_terms: additive covariance terms (H, G, b, wsse, sum_sq, n_valid, m) of the cost terms at x,

@@ -9,6 +9,7 @@
 #include <mutex>
 
 #include "mopt_internal.h"
+#include "mopt_quant_rule.h"
 
 using namespace mopt;
 
@@ -344,6 +345,15 @@ int launch_eval(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int 
   return launch_evaluate(L, p->model, st->dtype, p->compute_dtype, out_dtype, a, ev);
 }
 
+// One radix-select sweep (mopt_residual_quantiles) of the builtin or run-time compiled model, on set 0 of slot 0.
+int launch_quant_sweep(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, const QuantArgs& qa) {
+  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
+  if (p->model >= MOPT_MODEL_USER_BASE)
+    return launch_user_quantile_sweep(L, ctx->device, p->model, st->dtype, p->compute_dtype, a, qa);
+  return launch_quantile_sweep(L, p->model, st->dtype, p->compute_dtype, a, qa);
+}
+
 // An output of mopt_evaluate must be device memory the context's device can write.
 int check_device_output(const mopt_ctx* ctx, const void* ptr, const char* what) {
   if (!ptr) return MOPT_OK;
@@ -518,6 +528,7 @@ int ctx_alloc(mopt_ctx* ctx) {
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_eval_stats, sizeof(double) * (kEvalSums + 1)));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw));
   MOPT_CUDA_TRY(cudaHostAlloc(&ctx->h_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw, cudaHostAllocDefault));
+  MOPT_CUDA_TRY(cudaMalloc(&ctx->d_quant, sizeof(QuantState)));
   ctx->flags_capacity = 4096;
   if (const char* e = getenv("MOPT_LM_FLAG_RING")) {  // test knob: a small ring makes an ordinary solve wrap it
     const int v = atoi(e);
@@ -619,6 +630,7 @@ int mopt_ctx_destroy(mopt_ctx* ctx) try {
   cudaFree(ctx->d_gen);
   cudaFree(ctx->d_eval_stats);
   cudaFree(ctx->d_cov_sums);
+  cudaFree(ctx->d_quant);
   if (ctx->h_cov_sums) cudaFreeHost(ctx->h_cov_sums);
   if (ctx->h_xerr) cudaFreeHost(ctx->h_xerr);
   cudaFree(ctx->d_partials); cudaFree(ctx->d_ticket); cudaFree(ctx->d_trial);
@@ -764,6 +776,89 @@ int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem,
     stats->inlier_sum_sq = h[3];
     stats->max_sq = h[4];
   }
+  return MOPT_OK;
+}
+MOPT_ABI_CATCH
+
+int mopt_residual_quantiles(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x,
+                            int64_t first, int64_t count, int n_q, const double* q, mopt_quantiles* out) try {
+  MOPT_REQUIRE(ctx && store && store->ctx == ctx, "store does not belong to this context");
+  MOPT_TRY(validate_problem(store, problem, false));
+  MOPT_REQUIRE(first >= 0 && count >= 0 && first <= store->n && count <= store->n - first,
+               "the range [first, first + count) must lie inside the store");
+  MOPT_REQUIRE(n_q >= 0 && n_q <= MOPT_MAX_QUANTILES, "n_q must lie in [0, MOPT_MAX_QUANTILES]");
+  MOPT_REQUIRE(n_q == 0 || q, "null q");
+  for (int k = 0; k < n_q; ++k) MOPT_REQUIRE(q[k] >= 0.0 && q[k] <= 1.0, "every q must lie in [0, 1]");
+  MOPT_REQUIRE(out, "null out");
+  MOPT_REQUIRE(problem->num_parameters == 0 || x, "null parameter vector");
+  MOPT_CUDA_TRY(cudaSetDevice(ctx->device));
+  QuantLevels lv;
+  for (int k = 0; k < n_q; ++k) lv.q[k] = q[k];
+  lv.q[n_q] = 0.5;  // the median
+  // the head of the state: counts, target ranks and their keys (the histogram is zeroed by the steps)
+  constexpr size_t kHead = offsetof(QuantState, rem);
+  static_assert(kHead <= sizeof(PassResult), "the quantile result must fit the pinned bounce buffer");
+  unsigned char* h = reinterpret_cast<unsigned char*>(ctx->h_result->v);
+  if (count > 0) {
+    MOPT_TRY(setup_slot(ctx, 0, problem, x));
+    MOPT_CUDA_TRY(cudaMemsetAsync(ctx->d_quant, 0, sizeof(QuantState), ctx->stream));
+    const int sweeps = problem->compute_dtype == MOPT_F32 ? 4 : 8;
+    QuantArgs qa;
+    qa.first = first;
+    qa.count = count;
+    qa.st = ctx->d_quant;
+    for (int d = 0; d < sweeps; ++d) {
+      qa.sweep = d;
+      MOPT_TRY(launch_quant_sweep(ctx, store, problem, qa));
+      MOPT_TRY(launch_quantile_step(ctx->stream, ctx->d_quant, d, n_q + 1, lv));
+    }
+    MOPT_CUDA_TRY(cudaMemcpyAsync(h, ctx->d_quant, kHead, cudaMemcpyDeviceToHost, ctx->stream));
+    MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  } else {
+    std::memset(h, 0, kHead);
+  }
+  QuantState head;
+  std::memcpy(&head, h, kHead);
+  mopt_quantiles r;
+  std::memset(&r, 0, sizeof(r));
+  r.n_ranked = int64_t(head.n_ranked);
+  r.n_nan = int64_t(head.n_nan);
+  // the selected key of rank j, as the fp64 value numpy ranks (the fp32 keys widen exactly)
+  auto value_of = [&](int64_t j) -> double {
+    for (int k = 0; k < head.n_rank; ++k)
+      if (head.rank[k] == j) {
+        if (problem->compute_dtype == MOPT_F32) {
+          const uint32_t b = uint32_t(head.key[k]);
+          float f;
+          std::memcpy(&f, &b, sizeof(f));
+          return double(f);
+        }
+        double v;
+        std::memcpy(&v, &head.key[k], sizeof(v));
+        return v;
+      }
+    return NAN;
+  };
+  for (int k = 0; k <= n_q; ++k) {
+    double lo = NAN, hi = NAN, v = NAN;
+    if (r.n_ranked > 0) {
+      const QuantRank qr = quantile_rank(r.n_ranked, lv.q[k]);
+      lo = value_of(qr.j);
+      hi = value_of(qr.j1);
+      MOPT_REQUIRE(!std::isnan(lo) && !std::isnan(hi), "internal error: a quantile rank was not selected");
+      v = quantile_lerp(lo, hi, qr.t);
+    }
+    if (k < n_q) {
+      r.lo[k] = lo;
+      r.hi[k] = hi;
+      r.value[k] = v;
+    } else {
+      r.median = v;
+    }
+  }
+  for (int k = n_q; k < MOPT_MAX_QUANTILES; ++k) r.lo[k] = r.hi[k] = r.value[k] = NAN;
+  r.robust_sigma = std::sqrt(r.median / chi2_median(problem->num_outputs));
+  *out = r;
   return MOPT_OK;
 }
 MOPT_ABI_CATCH

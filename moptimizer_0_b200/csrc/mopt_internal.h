@@ -10,6 +10,7 @@
 #include "mopt_lm_mono.cuh"
 #include "mopt_models.cuh"
 #include "mopt_pass.cuh"
+#include "mopt_quant.cuh"
 
 struct mopt_ctx {
   int device = 0;
@@ -59,6 +60,7 @@ struct mopt_ctx {
   double* d_eval_stats = nullptr;                // mopt_evaluate: the statistics written by the evaluation kernel's last CTA
   double* d_cov_sums = nullptr;                  // mopt_covariance_terms: [MOPT_MAX_COSTS][kMaxRaw] score Gram totals
   double* h_cov_sums = nullptr;                  // pinned host copy of the same
+  mopt::QuantState* d_quant = nullptr;           // mopt_residual_quantiles: histogram, prefixes and selected keys
 };
 
 struct mopt_store {
@@ -110,6 +112,11 @@ int launch_evaluate(const PassLaunch& L, int model, int store_dtype, int compute
 int launch_cov(const PassLaunch& L, int model, int form, int store_dtype, int compute_dtype, const PassArgs& a,
                const CovArgs& cv);
 
+// mopt_quant.cu: one radix-select sweep of a builtin model, and the step between sweeps (mopt_residual_quantiles)
+int launch_quantile_sweep(const PassLaunch& L, int model, int store_dtype, int compute_dtype, const PassArgs& a,
+                          const QuantArgs& qa);
+int launch_quantile_step(cudaStream_t stream, QuantState* st, int sweep, int n_q, const QuantLevels& lv);
+
 // mopt_rtc.cu: run-time compiled user models (ids >= MOPT_MODEL_USER_BASE)
 int launch_user(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
                 const PassArgs& a);
@@ -117,6 +124,8 @@ int launch_user_evaluate(const PassLaunch& L, int device, int model, int store_d
                          const PassArgs& a, const EvalArgs& ev);
 int launch_user_cov(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
                     const PassArgs& a, const CovArgs& cv);
+int launch_user_quantile_sweep(const PassLaunch& L, int device, int model, int store_dtype, int compute_dtype,
+                               const PassArgs& a, const QuantArgs& qa);
 int launch_user_setup(cudaStream_t stream, int device, int model, CostSlot* slot, const double* x_dev,
                       const double* x_host, int P);
 int user_model_rot_offset(int model);
