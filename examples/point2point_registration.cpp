@@ -59,6 +59,12 @@ int main(int argc, char** argv) {
     const mopt_quantiles qd = cost.residualQuantiles(x0, {0.5, 0.9});
     std::printf("correspondence distance: median %.5f, 90th percentile %.5f, robust sigma %.5f\n", std::sqrt(qd.value[0]),
                 std::sqrt(qd.value[1]), qd.robust_sigma);
+    // hypothesis scoring (the RANSAC step): the solution against the start, scored in one pass over the data
+    double hyps[12] = {0, 0, 0, 0, 0, 0};
+    for (int i = 0; i < 6; ++i) hyps[6 + i] = x0[i];
+    const std::vector<mopt_eval_stats> sc = cost.scoreHypotheses(hyps, 2, 0.03);
+    std::printf("inliers within 0.03: %lld at x = 0, %lld at the solution\n", (long long)sc[0].n_inliers,
+                (long long)sc[1].n_inliers);
     // how certain the pose is: standard deviations from s^2 H^-1, s^2 estimated from the fit
     double cov[36];
     mopt_cov_report rep;

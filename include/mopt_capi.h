@@ -300,6 +300,32 @@ MOPT_API int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem*
                            int64_t first, int64_t count, double inlier_threshold, int out_dtype,
                            void* residuals, void* weights, mopt_eval_stats* stats);
 
+/* ---- hypothesis scoring ----------------------------------------------------------------------- */
+#define MOPT_MAX_HYPOTHESES 1024
+/* mopt_evaluate's statistics (no per-element outputs) at n_hyp parameter vectors in one call: out[k] is what
+ * mopt_evaluate(ctx, store, problem, xs + k * P, first, count, inlier_threshold, ..., &stats) returns.  The store is
+ * read once per 32 hypotheses instead of once per hypothesis, so from 32 hypotheses on a call costs arithmetic rather
+ * than memory traffic: the scoring step of RANSAC (minimal-sample hypotheses against all putative correspondences)
+ * and of multi-start fits.  Returns after the context stream is synchronised.
+ *   - Exact parts.  n_valid, n_inliers and max_sq of out[k] equal mopt_evaluate's at xs[k] bit for bit, for every
+ *     builtin and user model and dtype pair: the same set-up (x rounded to the compute Scalar, then model setup),
+ *     the same residual, the same key e2 = sum fma(r_o, r_o) in the compute dtype and the same test
+ *     double(e2) <= inlier_threshold^2.  They do not depend on n_hyp, on k's place in the batch or on
+ *     mopt_ctx_set_launch, so a caller with more than MOPT_MAX_HYPOTHESES hypotheses splits them over calls.
+ *   - Sums.  sum_sq and inlier_sum_sq accumulate double(e2) in fp64 like mopt_evaluate's, in another order: they
+ *     agree with its sums to rounding, and are identical from run to run for the same inputs and launch settings.
+ *   - As mopt_evaluate: masked elements (no correspondence) enter no statistic, correspondences are never
+ *     re-associated, count = 0 gives all-zero statistics, and the covariance, loss, jacobian, variant and manifold
+ *     fields have no effect.  A non-finite hypothesis gets what mopt_evaluate gives at that x and does not affect
+ *     the others.
+ *   - Sharded contexts: this rank's store only, no collective (see mopt_eval_stats).
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for n_hyp outside [1, MOPT_MAX_HYPOTHESES], a null xs or out, a
+ * model without parameters, a store of another context, a problem the store does not accept, a range outside the
+ * store or a negative inlier_threshold. */
+MOPT_API int mopt_score_hypotheses(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, int n_hyp,
+                                   const double* xs /* n_hyp x P, row-major, host */, int64_t first, int64_t count,
+                                   double inlier_threshold, mopt_eval_stats* out /* n_hyp, host */);
+
 /* ---- residual quantiles ----------------------------------------------------------------------- */
 #define MOPT_MAX_QUANTILES 8
 /* Exact order statistics of the keys e_i = r_i^T r_i of one cost term over a range of its store

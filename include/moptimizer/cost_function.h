@@ -71,6 +71,22 @@ class CostFunctionBase {
     return stats;
   }
 
+  /// New: evaluateStatistics at n_hyp parameter vectors xs (n_hyp x P, row-major) in one pass over the data
+  /// (mopt_score_hypotheses, at most MOPT_MAX_HYPOTHESES per call): the scoring step of RANSAC and of multi-start
+  /// fits.  Counts and max_sq equal evaluateStatistics' at each row exactly.  Correspondences are not re-associated.
+  std::vector<mopt_eval_stats> scoreHypotheses(const Scalar* xs, int n_hyp, double inlier_threshold) const {
+    mopt_problem p;
+    device::Store::Ptr st;
+    deviceProblem(&p, &st);
+    std::vector<double> xd(size_t(n_hyp > 0 ? n_hyp : 0) * size_t(p.num_parameters));
+    for (size_t i = 0; i < xd.size(); ++i) xd[i] = double(xs[i]);
+    std::vector<mopt_eval_stats> out(size_t(n_hyp > 0 ? n_hyp : 0));
+    device::check(mopt_score_hypotheses(st->context()->get(), st->get(), &p, n_hyp, xd.data(), 0, st->size(),
+                                        inlier_threshold, out.data()),
+                  "mopt_score_hypotheses");
+    return out;
+  }
+
   /// New: exact quantiles of e = r^T r over all residuals of this cost term at x (mopt_residual_quantiles) for the
   /// levels qs (at most MOPT_MAX_QUANTILES), plus the median and the robust scale sqrt(median / chi2_median(O)).
   /// sqrt of a value is the quantile of the residual norm |r|.  Correspondences are not re-associated: call

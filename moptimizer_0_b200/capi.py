@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_PKG, "libmopt_b200.so")
 
 MAX_PARAMETERS, MAX_OUTPUTS, MAX_COSTS, MAX_TRACE, NCCL_ID_BYTES = 16, 4, 8, 1024, 128
 MAX_QUANTILES = 8
+MAX_HYPOTHESES = 1024
 OK = 0
 F32, F64 = 0, 1
 (MODEL_POINT2POINT, MODEL_EXP_CURVE, MODEL_MICHAELIS_MENTEN, MODEL_PINHOLE, MODEL_POWELL,
@@ -49,7 +50,7 @@ EXPORTS = [
     "mopt_ctx_peer_handle", "mopt_ctx_open_peers", "mopt_ctx_set_exchange_enabled",
     "mopt_user_model_compile", "mopt_user_model_release", "mopt_user_model_log",
     "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate", "mopt_covariance_terms", "mopt_covariance_from_terms",
-    "mopt_residual_quantiles",
+    "mopt_residual_quantiles", "mopt_score_hypotheses",
 ]
 MODEL_USER_BASE = 1000
 PEER_HANDLE_BYTES = 64
@@ -108,6 +109,25 @@ class EvalStats(C.Structure):
 
 
 mopt_eval_stats = EvalStats  # the C name
+
+
+class HypothesisScores:
+    """Context.score_hypotheses: mopt_eval_stats of K hypotheses as numpy arrays of shape (K,) -- `n_valid`,
+    `n_inliers`, `sum_sq`, `inlier_sum_sq`, `max_sq` -- and `msac`, the truncated-quadratic (MSAC) score."""
+
+    def __init__(self, raw, inlier_threshold: float):
+        st = np.ctypeslib.as_array(raw)
+        self.n_valid = np.array(st["n_valid"], dtype=np.int64)
+        self.n_inliers = np.array(st["n_inliers"], dtype=np.int64)
+        self.sum_sq = np.array(st["sum_sq"], dtype=np.float64)
+        self.inlier_sum_sq = np.array(st["inlier_sum_sq"], dtype=np.float64)
+        self.max_sq = np.array(st["max_sq"], dtype=np.float64)
+        self.inlier_threshold = float(inlier_threshold)
+
+    @property
+    def msac(self) -> np.ndarray:
+        """inlier_sum_sq + (n_valid - n_inliers) thr^2: every outlier costs thr^2 (lower is better)."""
+        return self.inlier_sum_sq + (self.n_valid - self.n_inliers) * self.inlier_threshold ** 2
 
 
 class QuantilesStruct(C.Structure):
@@ -262,6 +282,8 @@ def lib():
         L.mopt_measure_peaks.argtypes = [vp, C.POINTER(Peaks)]
         L.mopt_evaluate.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_double, C.c_int, vp, vp,
                                     C.POINTER(EvalStats)]
+        L.mopt_score_hypotheses.argtypes = [vp, vp, C.POINTER(Problem), C.c_int, dp, i64, i64, C.c_double,
+                                            C.POINTER(EvalStats)]
         L.mopt_residual_quantiles.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_int, dp,
                                               C.POINTER(QuantilesStruct)]
         L.mopt_covariance_terms.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), dp,
@@ -470,6 +492,25 @@ class Context:
                                   float(inlier_threshold), out_dtype, r_t.data_ptr() if r_t is not None else None,
                                   w_t.data_ptr() if w_t is not None else None, C.byref(st)))
         return EvalResult(st, count, r_t, w_t)
+
+    def score_hypotheses(self, store: "Store", problem: Problem, xs, inlier_threshold: float, first: int = 0,
+                         count: Optional[int] = None) -> HypothesisScores:
+        """mopt_score_hypotheses: mopt_evaluate's statistics of the elements [first, first + count) at each row of xs
+        (shape (K, P)), the store read once per 32 rows.  More than MAX_HYPOTHESES rows take several calls, which
+        changes no count.  This context's store only; never re-associates."""
+        P = problem.num_parameters
+        xs = np.asarray(xs, dtype=np.float64)
+        if xs.ndim != 2 or xs.shape[0] < 1 or xs.shape[1] != P:
+            raise ValueError(f"xs must have shape (K, {P}) with K >= 1, got {xs.shape}")
+        xs = np.ascontiguousarray(xs)
+        count = store.n - first if count is None else int(count)
+        out = (EvalStats * xs.shape[0])()
+        for k0 in range(0, xs.shape[0], MAX_HYPOTHESES):
+            k = min(MAX_HYPOTHESES, xs.shape[0] - k0)
+            check(lib().mopt_score_hypotheses(self._h, store.handle, C.byref(problem), k, _dp(xs[k0:]), int(first),
+                                              count, float(inlier_threshold),
+                                              C.cast(C.addressof(out) + k0 * C.sizeof(EvalStats), C.POINTER(EvalStats))))
+        return HypothesisScores(out, inlier_threshold)
 
     def quantiles(self, store: "Store", problem: Problem, x, q=(), first: int = 0,
                   count: Optional[int] = None) -> Quantiles:

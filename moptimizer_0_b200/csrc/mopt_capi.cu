@@ -8,6 +8,7 @@
 #include <cstring>
 #include <mutex>
 
+#include "mopt_hyp_rule.h"
 #include "mopt_internal.h"
 #include "mopt_quant_rule.h"
 
@@ -354,6 +355,38 @@ int launch_quant_sweep(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* 
   return launch_quantile_sweep(L, p->model, st->dtype, p->compute_dtype, a, qa);
 }
 
+// Hypothesis scores (mopt_score_hypotheses) of the builtin or run-time compiled model, from the sets in h.sets.
+int launch_hyp_score(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, const HypArgs& h) {
+  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
+  if (p->model >= MOPT_MODEL_USER_BASE)
+    return launch_user_hypothesis_score(L, ctx->device, p->model, st->dtype, p->compute_dtype, a, h);
+  return launch_hypothesis_score(L, p->model, st->dtype, p->compute_dtype, a, h);
+}
+
+// The buffers of mopt_score_hypotheses, on its first call on this context (the partials take 48 MB).
+int hyp_alloc(mopt_ctx* ctx) {
+  // each buffer on its own: after a failed allocation the next call allocates only what is missing
+  constexpr size_t kTiles = MOPT_MAX_HYPOTHESES / kHypTile;
+  if (!ctx->h_hyp)
+    MOPT_CUDA_TRY(cudaHostAlloc(&ctx->h_hyp, sizeof(double) * MOPT_MAX_HYPOTHESES * kMaxP, cudaHostAllocDefault));
+  if (!ctx->d_hyp_x) MOPT_CUDA_TRY(cudaMalloc(&ctx->d_hyp_x, sizeof(double) * MOPT_MAX_HYPOTHESES * kMaxP));
+  if (!ctx->d_hyp_sets) MOPT_CUDA_TRY(cudaMalloc(&ctx->d_hyp_sets, sizeof(double) * MOPT_MAX_HYPOTHESES * kSetSize));
+  if (!ctx->d_hyp_partials)
+    MOPT_CUDA_TRY(cudaMalloc(&ctx->d_hyp_partials, sizeof(double) * kTiles * kHypRows * kMaxGrid));
+  if (!ctx->d_hyp_out) MOPT_CUDA_TRY(cudaMalloc(&ctx->d_hyp_out, sizeof(double) * MOPT_MAX_HYPOTHESES * kHypStats));
+  if (!ctx->d_hyp_tickets) {
+    // zeroed on the context stream, ahead of the first score kernel (the stream does not wait for the default one)
+    unsigned int* t = nullptr;
+    MOPT_CUDA_TRY(cudaMalloc(&t, sizeof(unsigned int) * kTiles));
+    const cudaError_t e = cudaMemsetAsync(t, 0, sizeof(unsigned int) * kTiles, ctx->stream);
+    if (e != cudaSuccess) cudaFree(t);
+    MOPT_CUDA_TRY(e);
+    ctx->d_hyp_tickets = t;
+  }
+  return MOPT_OK;
+}
+
 // An output of mopt_evaluate must be device memory the context's device can write.
 int check_device_output(const mopt_ctx* ctx, const void* ptr, const char* what) {
   if (!ptr) return MOPT_OK;
@@ -631,6 +664,12 @@ int mopt_ctx_destroy(mopt_ctx* ctx) try {
   cudaFree(ctx->d_eval_stats);
   cudaFree(ctx->d_cov_sums);
   cudaFree(ctx->d_quant);
+  cudaFree(ctx->d_hyp_x);
+  cudaFree(ctx->d_hyp_sets);
+  cudaFree(ctx->d_hyp_partials);
+  cudaFree(ctx->d_hyp_tickets);
+  cudaFree(ctx->d_hyp_out);
+  if (ctx->h_hyp) cudaFreeHost(ctx->h_hyp);
   if (ctx->h_cov_sums) cudaFreeHost(ctx->h_cov_sums);
   if (ctx->h_xerr) cudaFreeHost(ctx->h_xerr);
   cudaFree(ctx->d_partials); cudaFree(ctx->d_ticket); cudaFree(ctx->d_trial);
@@ -775,6 +814,64 @@ int mopt_evaluate(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem,
     stats->sum_sq = h[2];
     stats->inlier_sum_sq = h[3];
     stats->max_sq = h[4];
+  }
+  return MOPT_OK;
+}
+MOPT_ABI_CATCH
+
+int mopt_score_hypotheses(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, int n_hyp, const double* xs,
+                          int64_t first, int64_t count, double inlier_threshold, mopt_eval_stats* out) try {
+  MOPT_REQUIRE(ctx && store && store->ctx == ctx, "store does not belong to this context");
+  MOPT_TRY(validate_problem(store, problem, false));
+  MOPT_REQUIRE(problem->num_parameters > 0, "a model without parameters has no hypotheses to score");
+  MOPT_REQUIRE(n_hyp >= 1 && n_hyp <= MOPT_MAX_HYPOTHESES, "n_hyp must lie in [1, MOPT_MAX_HYPOTHESES]");
+  MOPT_REQUIRE(xs && out, "null xs or out");
+  MOPT_REQUIRE(first >= 0 && count >= 0 && first <= store->n && count <= store->n - first,
+               "the range [first, first + count) must lie inside the store");
+  MOPT_REQUIRE(!(inlier_threshold < 0.0), "inlier_threshold must not be negative");
+  if (count == 0) {
+    std::memset(out, 0, sizeof(*out) * size_t(n_hyp));
+    return MOPT_OK;
+  }
+  MOPT_CUDA_TRY(cudaSetDevice(ctx->device));
+  MOPT_TRY(hyp_alloc(ctx));
+  MOPT_TRY(stage_cost(ctx, 0, problem));
+  const int P = problem->num_parameters;
+  double* h = ctx->h_hyp;  // pinned; idle between calls (each call returns after synchronising)
+  std::memset(h, 0, sizeof(double) * size_t(n_hyp) * kMaxP);
+  for (int k = 0; k < n_hyp; ++k)
+    for (int i = 0; i < P; ++i) h[size_t(k) * kMaxP + i] = xs[size_t(k) * P + i];
+  MOPT_CUDA_TRY(cudaMemcpyAsync(ctx->d_hyp_x, h, sizeof(double) * size_t(n_hyp) * kMaxP, cudaMemcpyHostToDevice,
+                                ctx->stream));
+  const CostDev* cost = &ctx->d_slots[0].cost;
+  if (user_model_has_setup(problem->model))
+    MOPT_TRY(launch_user_hypothesis_setup(ctx->stream, ctx->device, problem->model, cost, ctx->d_hyp_x, n_hyp,
+                                          ctx->d_hyp_sets));
+  else
+    MOPT_TRY(launch_hypothesis_setup(ctx->stream, cost, ctx->d_hyp_x, n_hyp, ctx->d_hyp_sets));
+  HypArgs ha;
+  ha.first = first;
+  ha.count = count;
+  ha.n_hyp = n_hyp;
+  ha.thr2 = inlier_threshold * inlier_threshold;  // as mopt_evaluate forms it
+  ha.thr2f = largest_float_le(ha.thr2);
+  ha.sets = ctx->d_hyp_sets;
+  ha.partials = ctx->d_hyp_partials;
+  ha.tickets = ctx->d_hyp_tickets;
+  ha.out = ctx->d_hyp_out;
+  MOPT_TRY(launch_hyp_score(ctx, store, problem, ha));
+  MOPT_CUDA_TRY(cudaMemcpyAsync(h, ctx->d_hyp_out, sizeof(double) * size_t(n_hyp) * kHypStats, cudaMemcpyDeviceToHost,
+                                ctx->stream));
+  MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  for (int k = 0; k < n_hyp; ++k) {
+    const double* v = h + size_t(k) * kHypStats;
+    mopt_eval_stats& o = out[k];
+    std::memset(&o, 0, sizeof(o));
+    o.n_valid = int64_t(v[0]);
+    o.n_inliers = int64_t(v[1]);
+    o.sum_sq = v[2];
+    o.inlier_sum_sq = v[3];
+    o.max_sq = v[4];
   }
   return MOPT_OK;
 }

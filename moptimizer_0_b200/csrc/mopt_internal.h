@@ -6,6 +6,7 @@
 #include "mopt_common.cuh"
 #include "mopt_cov.cuh"
 #include "mopt_eval.cuh"
+#include "mopt_hyp.cuh"
 #include "mopt_lm.cuh"
 #include "mopt_lm_mono.cuh"
 #include "mopt_models.cuh"
@@ -61,6 +62,15 @@ struct mopt_ctx {
   double* d_cov_sums = nullptr;                  // mopt_covariance_terms: [MOPT_MAX_COSTS][kMaxRaw] score Gram totals
   double* h_cov_sums = nullptr;                  // pinned host copy of the same
   mopt::QuantState* d_quant = nullptr;           // mopt_residual_quantiles: histogram, prefixes and selected keys
+  // mopt_score_hypotheses, allocated on first use: the hypotheses ([MOPT_MAX_HYPOTHESES][kMaxP], uploaded through the
+  // pinned h_hyp, which also takes the results back), their sets, the per-CTA partials of every tile, the tickets
+  // and the per-hypothesis statistics
+  double* h_hyp = nullptr;
+  double* d_hyp_x = nullptr;
+  double* d_hyp_sets = nullptr;
+  double* d_hyp_partials = nullptr;
+  unsigned int* d_hyp_tickets = nullptr;
+  double* d_hyp_out = nullptr;
 };
 
 struct mopt_store {
@@ -117,6 +127,11 @@ int launch_quantile_sweep(const PassLaunch& L, int model, int store_dtype, int c
                           const QuantArgs& qa);
 int launch_quantile_step(cudaStream_t stream, QuantState* st, int sweep, int n_q, const QuantLevels& lv);
 
+// mopt_hyp.cu: set 0 of n hypotheses (xs [n][kMaxP] -> sets [n][kSetSize]) and their scores (mopt_score_hypotheses)
+int launch_hypothesis_setup(cudaStream_t stream, const CostDev* c, const double* xs, int n, double* sets);
+int launch_hypothesis_score(const PassLaunch& L, int model, int store_dtype, int compute_dtype, const PassArgs& a,
+                            const HypArgs& h);
+
 // mopt_rtc.cu: run-time compiled user models (ids >= MOPT_MODEL_USER_BASE)
 int launch_user(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
                 const PassArgs& a);
@@ -126,6 +141,10 @@ int launch_user_cov(const PassLaunch& L, int device, int model, bool numeric, in
                     const PassArgs& a, const CovArgs& cv);
 int launch_user_quantile_sweep(const PassLaunch& L, int device, int model, int store_dtype, int compute_dtype,
                                const PassArgs& a, const QuantArgs& qa);
+int launch_user_hypothesis_score(const PassLaunch& L, int device, int model, int store_dtype, int compute_dtype,
+                                 const PassArgs& a, const HypArgs& h);
+int launch_user_hypothesis_setup(cudaStream_t stream, int device, int model, const CostDev* c, const double* xs, int n,
+                                 double* sets);
 int launch_user_setup(cudaStream_t stream, int device, int model, CostSlot* slot, const double* x_dev,
                       const double* x_host, int P);
 int user_model_rot_offset(int model);

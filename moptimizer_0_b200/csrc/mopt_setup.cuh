@@ -234,6 +234,25 @@ __device__ inline void setup_one_set(const CostDev& c, const double* xs, double*
   }
 }
 
+// x as the compute Scalar holds it (linearization.h:78-89 with a float Scalar rounds every coordinate).
+__device__ inline void scalar_x(const CostDev& c, const double* x, double* xs) {
+  const bool f32 = (c.compute_dtype == MOPT_F32);
+  for (int i = 0; i < c.P; ++i) xs[i] = f32 ? double(float(x[i])) : x[i];
+}
+
+// Set 0 of setup_cost at x: the set every residual of a cost evaluation (mopt_evaluate) is formed from.
+__device__ inline void setup_base_set(const CostDev& c, const double* x, double* set) {
+  double xs[kMaxP];
+  scalar_x(c, x, xs);
+  setup_one_set(c, xs, set);
+}
+
+// Set 0 of n parameter vectors (mopt_score_hypotheses), one thread each: xs is [n][kMaxP], sets is [n][kSetSize].
+__device__ inline void setup_hypotheses(const CostDev& c, const double* xs, int n, double* sets) {
+  const int k = int(blockIdx.x * blockDim.x + threadIdx.x);
+  if (k < n) setup_base_set(c, xs + size_t(k) * kMaxP, sets + size_t(k) * kSetSize);
+}
+
 // Affine decomposition of the point2point analytical Jacobian, J(q) = J0 + q_x J1 + q_y J2 + q_z J3
 // (each 3x6 row-major), for the three variants of mopt_p2p_variant.
 __device__ inline void setup_p2p_affine(const CostDev& c, const double* x, double jaff[4][18]) {
@@ -293,47 +312,49 @@ __device__ inline void setup_cost(const CostDev& c, const double* x, ParamBlock*
   const bool f32 = (c.compute_dtype == MOPT_F32);
   const int nsets = (c.jacobian == MOPT_JAC_ANALYTICAL) ? 1 : (c.jacobian == MOPT_JAC_FORWARD ? 1 + P : 1 + 2 * P);
   for (int s = lane; s < nsets; s += nlanes) {
+    if (s == 0) {  // the unperturbed set: the one every cost evaluation and hypothesis score reads
+      setup_base_set(c, x, pb->sets[0]);
+      continue;
+    }
     double xs[kMaxP];
-    for (int i = 0; i < P; ++i) xs[i] = f32 ? double(float(x[i])) : x[i];
-    if (s > 0) {
-      const int j = (s - 1) % P;
-      const bool minus = (s - 1) >= P;
-      double h;
-      double step_fwd, step_cen;  // the steps actually taken (see ParamBlock::hstep_*)
-      if (f32) {
-        const float ms = sqrtf(1.1920928955078125e-07f);
-        float hf = ms * fabsf(float(x[j]));
-        if (hf == 0.0f) hf = ms;
-        h = double(hf);
-        const float xpl = float(x[j]) + hf, xmi = float(x[j]) - hf;
-        xs[j] = double(minus ? xmi : xpl);
-        step_fwd = double(xpl) - double(float(x[j]));
-        step_cen = double(xpl) - double(xmi);
-      } else {
-        const double ms = sqrt(2.220446049250313e-16);
-        h = ms * fabs(x[j]);
-        if (h == 0.0) h = ms;
-        xs[j] = minus ? x[j] - h : x[j] + h;
-        step_fwd = (x[j] + h) - x[j];
-        step_cen = (x[j] + h) - (x[j] - h);
-      }
-      if (c.manifold == MOPT_MANIFOLD_SO3_LEFT && c.rot_offset >= 0 && j >= c.rot_offset && j < c.rot_offset + 3) {
-        // tangent coordinate of the rotation block is 0 at x, so the reference's rule (:85-87) gives h = sqrt(eps)
-        h = f32 ? double(sqrtf(1.1920928955078125e-07f)) : sqrt(2.220446049250313e-16);
-        double d[kMaxP];
-        for (int i = 0; i < P; ++i) d[i] = 0.0;
-        d[j] = minus ? -h : h;
-        double base[kMaxP];
-        for (int i = 0; i < P; ++i) base[i] = f32 ? double(float(x[i])) : x[i];
-        retract_dev(c, base, d, xs, f32);
-        step_fwd = h;  // the tangent-space step is not a coordinate difference of x
-        step_cen = 2.0 * h;
-      }
-      if (!minus) {
-        pb->h[j] = h;
-        pb->hstep_fwd[j] = step_fwd;
-        pb->hstep_cen[j] = step_cen;
-      }
+    scalar_x(c, x, xs);
+    const int j = (s - 1) % P;
+    const bool minus = (s - 1) >= P;
+    double h;
+    double step_fwd, step_cen;  // the steps actually taken (see ParamBlock::hstep_*)
+    if (f32) {
+      const float ms = sqrtf(1.1920928955078125e-07f);
+      float hf = ms * fabsf(float(x[j]));
+      if (hf == 0.0f) hf = ms;
+      h = double(hf);
+      const float xpl = float(x[j]) + hf, xmi = float(x[j]) - hf;
+      xs[j] = double(minus ? xmi : xpl);
+      step_fwd = double(xpl) - double(float(x[j]));
+      step_cen = double(xpl) - double(xmi);
+    } else {
+      const double ms = sqrt(2.220446049250313e-16);
+      h = ms * fabs(x[j]);
+      if (h == 0.0) h = ms;
+      xs[j] = minus ? x[j] - h : x[j] + h;
+      step_fwd = (x[j] + h) - x[j];
+      step_cen = (x[j] + h) - (x[j] - h);
+    }
+    if (c.manifold == MOPT_MANIFOLD_SO3_LEFT && c.rot_offset >= 0 && j >= c.rot_offset && j < c.rot_offset + 3) {
+      // tangent coordinate of the rotation block is 0 at x, so the reference's rule (:85-87) gives h = sqrt(eps)
+      h = f32 ? double(sqrtf(1.1920928955078125e-07f)) : sqrt(2.220446049250313e-16);
+      double d[kMaxP];
+      for (int i = 0; i < P; ++i) d[i] = 0.0;
+      d[j] = minus ? -h : h;
+      double base[kMaxP];
+      for (int i = 0; i < P; ++i) base[i] = f32 ? double(float(x[i])) : x[i];
+      retract_dev(c, base, d, xs, f32);
+      step_fwd = h;  // the tangent-space step is not a coordinate difference of x
+      step_cen = 2.0 * h;
+    }
+    if (!minus) {
+      pb->h[j] = h;
+      pb->hstep_fwd[j] = step_fwd;
+      pb->hstep_cen[j] = step_cen;
     }
     setup_one_set(c, xs, pb->sets[s]);
   }
