@@ -79,6 +79,7 @@ __global__ void __launch_bounds__(THREADS, MINB) dense_f2_kernel(const PassArgs 
   for (int i = 0; i < NRAW; ++i) acc[i] = F2(0.f);
   double dacc[1] = {0.0};
 
+  // All 32 lanes of the warp must call flush() together: warp_reduce_transpose is a full-mask shuffle.
   auto flush = [&]() {
     float s[V];
 #pragma unroll
@@ -232,7 +233,9 @@ __global__ void __launch_bounds__(THREADS, MINB) dense_f2_kernel(const PassArgs 
       buf ^= 1;
     }
     do_group(v);
-    if (++since_flush >= FLUSH_ROUNDS) {
+    // a warp's lanes hold g = 32 w .. 32 w + 31, so (g | 31) is its last lane's: where that lane has no group this is
+    // the warp's last iteration and only some of its lanes are here, so the flush after the loop takes this one
+    if (++since_flush >= FLUSH_ROUNDS && (g | 31) < ngroups) {
       flush();
       since_flush = 0;
     }

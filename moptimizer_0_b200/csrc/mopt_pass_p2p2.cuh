@@ -196,6 +196,7 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
   for (int i = 0; i < kP2PRaw; ++i) acc[i] = make_float2(0.f, 0.f);
   double dacc[1] = {0.0};
 
+  // All 32 lanes of the warp must call flush() together: warp_reduce_transpose is a full-mask shuffle.
   auto flush = [&]() {
     float s[32];
 #pragma unroll
@@ -264,7 +265,9 @@ __global__ void __launch_bounds__(THREADS, MINB) p2p_moment2_kernel(const PassAr
     for (int64_t g = full_rounds * stride + int64_t(blockIdx.x) * THREADS + threadIdx.x; g < ngroups;
          g += int64_t(gridDim.x) * THREADS) {
       direct_group(g);
-      if (++since_flush >= FLUSH_ROUNDS) {
+      // a warp's lanes hold g = 32 w .. 32 w + 31, so (g | 31) is its last lane's: where that lane has no group this is
+      // the warp's last iteration and only some of its lanes are here, so the flush after the loop takes this one
+      if (++since_flush >= FLUSH_ROUNDS && (g | 31) < ngroups) {
         flush();
         since_flush = 0;
       }
