@@ -455,7 +455,14 @@ MOPT_API int mopt_ldlt_solve(int n, const double* A_colmajor, const double* rhs,
  * (src/levenberg_marquadt_dyn.cpp:54; include/moptimizer/model.h:24-26 "i.e registration correspondences") but
  * ships no implementation.  A mopt_nn_index holds a fixed TARGET cloud in a device uniform grid; attached to a
  * point2point store it makes update(x) mean: tgt_i <- nearest target point of T(x) src_i within `max_distance`,
- * source points without one being skipped by later passes (model f returning false, linearization.h:102,144). */
+ * source points without one being skipped by later passes (model f returning false, linearization.h:102,144).
+ * The match is the brute-force nearest neighbour:
+ *   - ties go to the lowest original index of the target cloud;
+ *   - the radius is inclusive: a target at exactly max_distance matches;
+ *   - an fp32 index (index_dtype = MOPT_F32) forms the query and the distances in fp32 from fp32-rounded data and
+ *     writes fp32-rounded target coordinates;
+ *   - a target point with a non-finite coordinate is kept but never matches (it does not size the grid either).
+ * max_distance must be positive and finite. */
 typedef struct mopt_nn_index mopt_nn_index;
 MOPT_API int mopt_nn_index_create(mopt_ctx* ctx, const void* host_xyz, int host_dtype, int index_dtype, int64_t m,
                                   double max_distance, mopt_nn_index** out);

@@ -8,6 +8,11 @@
 // surrounding cells and rewrites the store's target streams in place.  Source points with no target within
 // the distance get a NaN marker and are skipped by every later pass, which is what `f` returning false
 // means in the reference (linearization.h:102,144).
+//
+// Contract (the brute-force oracle::Point2PointICP restated): ties go to the lowest original index, the radius is
+// inclusive (|q - p|^2 <= max_dist^2, in the index dtype), the fp32 index forms the query and the distances in fp32
+// from fp32-rounded data and writes fp32-rounded target coordinates, and a target point with a non-finite
+// coordinate never matches: it is kept in the index, in one extra cell behind the grid that no query scans.
 #include <cmath>
 #include <cstring>
 #include <vector>
@@ -26,7 +31,8 @@ struct mopt_nn_index {
   int64_t ncells = 1;
   void* d_pts = nullptr;        // sorted by cell: x[m], y[m], z[m] (planar, index dtype)
   int* d_orig = nullptr;        // original index of each sorted point (tie-break => deterministic matches)
-  unsigned int* d_start = nullptr;  // [ncells + 1] exclusive prefix of the per-cell counts
+  unsigned int* d_start = nullptr;  // [ncells + 2] exclusive prefix of the per-cell counts; cell ncells holds the
+                                    // non-finite points
   long long* d_matched = nullptr;
 };
 
@@ -38,21 +44,30 @@ struct GridDesc {
   int dims[3];
 };
 
+// Cell of a coordinate along one axis, -1 / dim outside the grid; NaN gives -1 (never int(NaN)).
 template <typename T>
 __device__ __forceinline__ int cell_coord(T v, double origin, double inv_cell, int dim) {
   const double c = floor((double(v) - origin) * inv_cell);
-  return c < 0.0 ? -1 : (c >= double(dim) ? dim : int(c));
+  return c >= 0.0 ? (c < double(dim) ? int(c) : dim) : -1;
+}
+
+template <typename T>
+__device__ __forceinline__ bool finite3(const T* p) {
+  return isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]);
 }
 
 template <typename T>
 __global__ void bbox_kernel(const T* __restrict__ aos, int64_t m, double* __restrict__ partial /*[grid][6]*/) {
-  double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < m; i += int64_t(gridDim.x) * blockDim.x)
+  // the box of the points whose three coordinates are finite (lo > hi when there is none)
+  double lo[3] = {HUGE_VAL, HUGE_VAL, HUGE_VAL}, hi[3] = {-HUGE_VAL, -HUGE_VAL, -HUGE_VAL};
+  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < m; i += int64_t(gridDim.x) * blockDim.x) {
+    if (!finite3(aos + i * 3)) continue;
     for (int k = 0; k < 3; ++k) {
       const double v = double(aos[i * 3 + k]);
       lo[k] = fmin(lo[k], v);
       hi[k] = fmax(hi[k], v);
     }
+  }
   __shared__ double s[6][256];
   for (int k = 0; k < 3; ++k) { s[k][threadIdx.x] = lo[k]; s[3 + k][threadIdx.x] = hi[k]; }
   __syncthreads();
@@ -68,16 +83,20 @@ __global__ void bbox_kernel(const T* __restrict__ aos, int64_t m, double* __rest
     for (int k = 0; k < 6; ++k) partial[blockIdx.x * 6 + k] = s[k][0];
 }
 
+// Cell of each target point: the clamped grid cell, or `ncells` (behind the grid, never scanned) for a point with a
+// non-finite coordinate.
 template <typename T>
-__global__ void count_kernel(const T* __restrict__ aos, int64_t m, GridDesc g, unsigned int* __restrict__ counts,
-                             unsigned int* __restrict__ cell_of) {
+__global__ void count_kernel(const T* __restrict__ aos, int64_t m, GridDesc g, unsigned int ncells,
+                             unsigned int* __restrict__ counts, unsigned int* __restrict__ cell_of) {
   for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < m; i += int64_t(gridDim.x) * blockDim.x) {
     int c[3];
     for (int k = 0; k < 3; ++k) {
       c[k] = cell_coord(aos[i * 3 + k], g.origin[k], g.inv_cell, g.dims[k]);
       c[k] = c[k] < 0 ? 0 : (c[k] >= g.dims[k] ? g.dims[k] - 1 : c[k]);
     }
-    const unsigned int cell = (unsigned(c[2]) * g.dims[1] + unsigned(c[1])) * g.dims[0] + unsigned(c[0]);
+    const unsigned int cell = finite3(aos + i * 3)
+                                  ? (unsigned(c[2]) * g.dims[1] + unsigned(c[1])) * g.dims[0] + unsigned(c[0])
+                                  : ncells;
     cell_of[i] = cell;
     atomicAdd(&counts[cell], 1u);
   }
@@ -110,7 +129,7 @@ __global__ void scan_tiles_kernel(unsigned int* __restrict__ data, int64_t n, un
   if (threadIdx.x == kScanThreads - 1) tile_sums[blockIdx.x] = s[threadIdx.x];
 }
 
-__global__ void scan_sums_kernel(unsigned int* __restrict__ tile_sums, int ntiles) {  // one thread: ntiles <= 8192
+__global__ void scan_sums_kernel(unsigned int* __restrict__ tile_sums, int ntiles) {  // one thread: ntiles <= 8193
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     unsigned int run = 0;
     for (int i = 0; i < ntiles; ++i) {
@@ -236,19 +255,25 @@ int build_index(mopt_nn_index* ix, const void* host, int host_dtype) {
   MOPT_CUDA_TRY(cudaMemcpyAsync(part.data(), d_part, sizeof(double) * part.size(), cudaMemcpyDeviceToHost, ctx->stream));
   MOPT_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   cudaFree(d_part);
-  double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
+  double lo[3] = {HUGE_VAL, HUGE_VAL, HUGE_VAL}, hi[3] = {-HUGE_VAL, -HUGE_VAL, -HUGE_VAL};
   for (int b = 0; b < bb_blocks; ++b)
     for (int k = 0; k < 3; ++k) {
       lo[k] = std::fmin(lo[k], part[b * 6 + k]);
       hi[k] = std::fmax(hi[k], part[b * 6 + 3 + k]);
     }
-  if (m == 0) for (int k = 0; k < 3; ++k) lo[k] = hi[k] = 0.0;
-  // cell edge: the search radius, grown until the grid has at most 2^24 cells
+  if (!(lo[0] <= hi[0])) for (int k = 0; k < 3; ++k) lo[k] = hi[k] = 0.0;  // no finite point (or m == 0)
+  // An axis whose points span more than DBL_MAX (e.g. -1e308 and 1e308): hi - lo is inf, and the axis becomes one
+  // slab that every query scans whole.
+  double ext[3];
+  for (int k = 0; k < 3; ++k) ext[k] = hi[k] - lo[k];
+  // cell edge: the search radius, grown until the grid has at most 2^24 cells.  The extents are finite (or one slab)
+  // and the radius is finite: a radius of at least every extent fits on the first pass, and otherwise the edge grows
+  // until it exceeds every extent / 255 (< DBL_MAX / 200), so the loop ends.
   double cell = ix->max_dist;
   for (;;) {
     double dims[3], total = 1.0;  // in double until the total is known to be small: a tiny radius over a wide
     for (int k = 0; k < 3; ++k) {  // cloud gives per-axis counts far beyond INT_MAX
-      dims[k] = std::floor((hi[k] - lo[k]) / cell) + 1.0;
+      dims[k] = std::isfinite(ext[k]) ? std::floor(ext[k] / cell) + 1.0 : 1.0;
       total *= dims[k];
     }
     if (total <= double(1 << 24)) {
@@ -265,20 +290,21 @@ int build_index(mopt_nn_index* ix, const void* host, int host_dtype) {
   g.inv_cell = 1.0 / cell;
 
   unsigned int *d_cell_of = nullptr, *d_cursor = nullptr, *d_tiles = nullptr;
-  const int ntiles = int((ix->ncells + 1 + kScanTile - 1) / kScanTile);
-  MOPT_CUDA_TRY(cudaMalloc(&ix->d_start, sizeof(unsigned int) * size_t(ix->ncells + 1)));
-  MOPT_CUDA_TRY(cudaMalloc(&d_cursor, sizeof(unsigned int) * size_t(ix->ncells)));
+  const int64_t nstart = ix->ncells + 2;  // the grid's cells, the cell of the non-finite points, the end
+  const int ntiles = int((nstart + kScanTile - 1) / kScanTile);
+  MOPT_CUDA_TRY(cudaMalloc(&ix->d_start, sizeof(unsigned int) * size_t(nstart)));
+  MOPT_CUDA_TRY(cudaMalloc(&d_cursor, sizeof(unsigned int) * size_t(ix->ncells + 1)));
   MOPT_CUDA_TRY(cudaMalloc(&d_cell_of, sizeof(unsigned int) * size_t(m > 0 ? m : 1)));
   MOPT_CUDA_TRY(cudaMalloc(&d_tiles, sizeof(unsigned int) * size_t(ntiles)));
-  MOPT_CUDA_TRY(cudaMemsetAsync(ix->d_start, 0, sizeof(unsigned int) * size_t(ix->ncells + 1), ctx->stream));
-  MOPT_CUDA_TRY(cudaMemsetAsync(d_cursor, 0, sizeof(unsigned int) * size_t(ix->ncells), ctx->stream));
+  MOPT_CUDA_TRY(cudaMemsetAsync(ix->d_start, 0, sizeof(unsigned int) * size_t(nstart), ctx->stream));
+  MOPT_CUDA_TRY(cudaMemsetAsync(d_cursor, 0, sizeof(unsigned int) * size_t(ix->ncells + 1), ctx->stream));
   int blocks = int(std::min<int64_t>((m + 255) / 256, 148 * 16));
   if (blocks < 1) blocks = 1;
-  count_kernel<T><<<blocks, 256, 0, ctx->stream>>>(d_aos, m, g, ix->d_start, d_cell_of);
+  count_kernel<T><<<blocks, 256, 0, ctx->stream>>>(d_aos, m, g, unsigned(ix->ncells), ix->d_start, d_cell_of);
   MOPT_CUDA_TRY(cudaGetLastError());
-  scan_tiles_kernel<<<ntiles, kScanThreads, 0, ctx->stream>>>(ix->d_start, ix->ncells + 1, d_tiles);
+  scan_tiles_kernel<<<ntiles, kScanThreads, 0, ctx->stream>>>(ix->d_start, nstart, d_tiles);
   scan_sums_kernel<<<1, 32, 0, ctx->stream>>>(d_tiles, ntiles);
-  scan_add_kernel<<<ntiles, kScanThreads, 0, ctx->stream>>>(ix->d_start, ix->ncells + 1, d_tiles);
+  scan_add_kernel<<<ntiles, kScanThreads, 0, ctx->stream>>>(ix->d_start, nstart, d_tiles);
   MOPT_CUDA_TRY(cudaGetLastError());
   T* pts = nullptr;
   MOPT_CUDA_TRY(cudaMalloc(&pts, esz * 3 * size_t(m > 0 ? m : 1)));
