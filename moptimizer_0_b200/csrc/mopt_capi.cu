@@ -166,6 +166,14 @@ __global__ void ldlt_test_kernel(int n, double* A, const double* rhs, double* ou
 // ----------------------------------------------------------------------------- helpers ----
 namespace {
 
+// Where x holds a rotation vector (x[3..5] for the builtin point2point and camera models, the declared offset for a
+// user model), or -1.
+int rot_offset(int model) {
+  if (model >= MOPT_MODEL_USER_BASE) return user_model_rot_offset(model);
+  return (model == MOPT_MODEL_POINT2POINT || model == MOPT_MODEL_PINHOLE || model == MOPT_MODEL_PINHOLE_DISTORT) ? 3
+                                                                                                               : -1;
+}
+
 int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_linearize) {
   MOPT_REQUIRE(st && p, "null store/problem");
   MOPT_REQUIRE(p->model == st->model, "problem.model differs from the store's model");
@@ -188,10 +196,7 @@ int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_line
     MOPT_REQUIRE(p->variant >= MOPT_P2P_EXACT && p->variant <= MOPT_P2P_LEFT, "unknown point2point variant");
   MOPT_REQUIRE(p->manifold == MOPT_MANIFOLD_ADDITIVE || p->manifold == MOPT_MANIFOLD_SO3_LEFT, "unknown manifold");
   if (p->manifold == MOPT_MANIFOLD_SO3_LEFT)
-    MOPT_REQUIRE(p->model == MOPT_MODEL_POINT2POINT || p->model == MOPT_MODEL_PINHOLE ||
-                     p->model == MOPT_MODEL_PINHOLE_DISTORT ||
-                     (p->model >= MOPT_MODEL_USER_BASE && user_model_rot_offset(p->model) >= 0),
-                 "MOPT_MANIFOLD_SO3_LEFT needs a model whose x[3..5] is a rotation vector");
+    MOPT_REQUIRE(rot_offset(p->model) >= 0, "MOPT_MANIFOLD_SO3_LEFT needs a model whose x[3..5] is a rotation vector");
   if (p->has_covariance) {
     const int O = sh.O;
     for (int r = 0; r < O; ++r)
@@ -200,6 +205,11 @@ int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_line
           set_last_error("covariance must be symmetric (only the upper triangle of H is accumulated)");
           return MOPT_ERR_UNSUPPORTED;
         }
+  }
+  // no kernel reads an fp64 store into fp32 arithmetic (with_dtypes)
+  if (st->dtype == MOPT_F64 && p->compute_dtype == MOPT_F32) {
+    set_last_error("store dtype f64 with compute dtype f32 is not supported");
+    return MOPT_ERR_UNSUPPORTED;
   }
   return MOPT_OK;
 }
@@ -210,9 +220,7 @@ void fill_cost(const mopt_problem* p, CostDev* c) {
   c->jacobian = p->jacobian; c->loss = p->loss; c->has_cov = p->has_covariance ? 1 : 0;
   c->compute_dtype = p->compute_dtype; c->loss_param = p->loss_param;
   c->manifold = p->manifold;
-  c->rot_offset = (p->model == MOPT_MODEL_POINT2POINT || p->model == MOPT_MODEL_PINHOLE ||
-                   p->model == MOPT_MODEL_PINHOLE_DISTORT) ? 3 : -1;
-  if (p->model >= MOPT_MODEL_USER_BASE) c->rot_offset = user_model_rot_offset(p->model);
+  c->rot_offset = rot_offset(p->model);
   c->so3_guard = ((p->flags & MOPT_FLAG_REFERENCE_FLOAT_GUARD) && p->compute_dtype == MOPT_F32) ? kSo3GuardF32 : kSo3GuardF64;
   const int O = p->num_outputs;
   for (int i = 0; i < O * O; ++i) c->cov[i] = p->has_covariance ? p->covariance[i] : ((i % (O + 1) == 0) ? 1.0 : 0.0);
@@ -310,58 +318,95 @@ int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int 
                              p->variant == MOPT_P2P_EXACT || p->variant == MOPT_P2P_LEFT, a);
   // finite differences of an affine residual are affine in the source point: moment kernel with q = p
   // (mopt_setup.cuh fills the affine pieces); cost-only passes of this model take the same kernel
-  if (p->model == MOPT_MODEL_POINT2POINT && !(p->flags & MOPT_FLAG_GENERIC_KERNEL) &&
-      !(st->dtype == MOPT_F64 && p->compute_dtype == MOPT_F32))
+  if (p->model == MOPT_MODEL_POINT2POINT && !(p->flags & MOPT_FLAG_GENERIC_KERNEL))
     return launch_p2p_moment(L, st->dtype, p->compute_dtype, p->loss, false, a);
-  if (p->model == MOPT_MODEL_PINHOLE_DISTORT) return launch_wide(L, p->model, st->dtype, p->compute_dtype, a);
+  if (is_wide(p->num_parameters)) return launch_wide(L, p->model, st->dtype, p->compute_dtype, a);
   return launch_dense(L, p->model, p->jacobian != MOPT_JAC_ANALYTICAL, st->dtype, p->compute_dtype, a);
 }
 
+// The analysis kernels below (score Gram, evaluation, quantile sweep, hypothesis scores) have one launcher each for
+// builtin and run-time compiled models alike: the kernel resolves to a KernelDesc, and its grid follows from the same
+// work items by the same rule (persistent_grid) whichever model it is.
+
 // Score Gram sums (mopt_covariance_terms) of cost term `slot`, staged by setup_slot, into `out`: the Jacobian form
-// launch_pass selects for the same problem (launch_cov picks the common-denominator differences where
+// launch_pass selects for the same problem (score_gram_kernel_desc picks the common-denominator differences where
 // pass_launch's affine_fd and the model allow them, as launch_dense / launch_wide do).
 int launch_cov_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int slot, double* out) {
-  const PassArgs a = make_args(ctx, st, slot, 0, PASS_LINEARIZE);
-  const PassLaunch L = pass_launch(ctx, p);
+  PassLaunch L = pass_launch(ctx, p);
   const bool numeric = p->jacobian != MOPT_JAC_ANALYTICAL;
+  int form = numeric ? COV_JAC_FD : COV_JAC_ANALYTICAL;
+  if (p->model == MOPT_MODEL_POINT2POINT && (!numeric || !(p->flags & MOPT_FLAG_GENERIC_KERNEL)))
+    form = COV_JAC_P2P_AFFINE;
+  KernelDesc k;
+  MOPT_TRY(p->model >= MOPT_MODEL_USER_BASE
+               ? user_kernel(ctx->device, p->model, KIND_COV, st->dtype, p->compute_dtype, numeric, &k)
+               : score_gram_kernel_desc(p->model, form, L.affine_fd, st->dtype, p->compute_dtype, &k));
+  // work items as the pass kernels count them: 16-byte groups (P <= 6), residuals (wide tier); like the builtin dense
+  // and wide passes, the kernel keeps its full occupancy whatever mopt_ctx_set_launch asks
+  const ModelShape sh = model_shape(p->model);
+  const int64_t items = sh.NS == 0 ? 1 : (sh.P <= 6 ? st->n / store_vec(st->dtype) : st->n);
+  L.ctas_per_sm = 0;
+  const int grid = persistent_grid(k.occupancy, k.threads, L, items);
+  PassArgs a = make_args(ctx, st, slot, 0, PASS_LINEARIZE);
   CovArgs cv;
   cv.out = out;
   cv.qrot = (!numeric && (p->variant == MOPT_P2P_EXACT || p->variant == MOPT_P2P_LEFT)) ? 1 : 0;
-  if (p->model >= MOPT_MODEL_USER_BASE)
-    return launch_user_cov(L, ctx->device, p->model, numeric, st->dtype, p->compute_dtype, a, cv);
-  int form = numeric ? COV_JAC_FD : COV_JAC_ANALYTICAL;
-  if (p->model == MOPT_MODEL_POINT2POINT &&
-      (!numeric || (!(p->flags & MOPT_FLAG_GENERIC_KERNEL) && !(st->dtype == MOPT_F64 && p->compute_dtype == MOPT_F32))))
-    form = COV_JAC_P2P_AFFINE;
-  return launch_cov(L, p->model, form, st->dtype, p->compute_dtype, a, cv);
+  void* params[] = {&a, &cv};
+  MOPT_CUDA_TRY(cudaLaunchKernel(k.fn, dim3(unsigned(grid)), dim3(unsigned(k.threads)), params, 0, ctx->stream));
+  return MOPT_OK;
 }
 
-// Per-residual evaluation (mopt_evaluate): the builtin or run-time compiled evaluate_kernel of the model, on set 0 of
-// slot 0 (staged by setup_slot), reducing its statistics through the same partials / ticket as the passes.
+// Per-residual evaluation (mopt_evaluate): evaluate_kernel of the model on set 0 of slot 0 (staged by setup_slot),
+// reducing its statistics through the same partials / ticket as the passes.
 int launch_eval(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int out_dtype, const EvalArgs& ev) {
-  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
-  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
-  if (p->model >= MOPT_MODEL_USER_BASE)
-    return launch_user_evaluate(L, ctx->device, p->model, st->dtype, p->compute_dtype, out_dtype, a, ev);
-  return launch_evaluate(L, p->model, st->dtype, p->compute_dtype, out_dtype, a, ev);
+  KernelDesc k[2];  // fp32, fp64 outputs
+  for (int o = 0; o < 2; ++o)
+    MOPT_TRY(p->model >= MOPT_MODEL_USER_BASE
+                 ? user_kernel(ctx->device, p->model, KIND_EVAL, st->dtype, p->compute_dtype, o == 1, &k[o])
+                 : evaluate_kernel_desc(p->model, st->dtype, p->compute_dtype, o == 1, &k[o]));
+  // One grid for both output dtypes (the smaller of their persistent grids), so that the statistics -- whose
+  // summation order follows the grid -- do not depend on which outputs are written or in which dtype.
+  const PassLaunch L = pass_launch(ctx, p);
+  const int64_t groups = ev.count / store_vec(st->dtype) + 1;
+  const int g0 = persistent_grid(k[0].occupancy, k[0].threads, L, groups);
+  const int g1 = persistent_grid(k[1].occupancy, k[1].threads, L, groups);
+  const KernelDesc& kern = k[out_dtype == MOPT_F64 ? 1 : 0];
+  PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  EvalArgs e = ev;
+  void* params[] = {&a, &e};
+  MOPT_CUDA_TRY(cudaLaunchKernel(kern.fn, dim3(unsigned(g0 < g1 ? g0 : g1)), dim3(unsigned(kern.threads)), params, 0,
+                                 ctx->stream));
+  return MOPT_OK;
 }
 
-// One radix-select sweep (mopt_residual_quantiles) of the builtin or run-time compiled model, on set 0 of slot 0.
+// One radix-select sweep (mopt_residual_quantiles) of the model, on set 0 of slot 0.
 int launch_quant_sweep(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, const QuantArgs& qa) {
-  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
-  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
-  if (p->model >= MOPT_MODEL_USER_BASE)
-    return launch_user_quantile_sweep(L, ctx->device, p->model, st->dtype, p->compute_dtype, a, qa);
-  return launch_quantile_sweep(L, p->model, st->dtype, p->compute_dtype, a, qa);
+  KernelDesc k;
+  MOPT_TRY(p->model >= MOPT_MODEL_USER_BASE
+               ? user_kernel(ctx->device, p->model, KIND_QUANT, st->dtype, p->compute_dtype, false, &k)
+               : quantile_sweep_kernel_desc(p->model, st->dtype, p->compute_dtype, &k));
+  const int grid = persistent_grid(k.occupancy, k.threads, pass_launch(ctx, p), qa.count / store_vec(st->dtype) + 1);
+  PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  QuantArgs q = qa;
+  void* params[] = {&a, &q};
+  MOPT_CUDA_TRY(cudaLaunchKernel(k.fn, dim3(unsigned(grid)), dim3(unsigned(k.threads)), params, 0, ctx->stream));
+  return MOPT_OK;
 }
 
-// Hypothesis scores (mopt_score_hypotheses) of the builtin or run-time compiled model, from the sets in h.sets.
+// Hypothesis scores (mopt_score_hypotheses) of the model, from the sets in h.sets.  The grid follows the elements
+// only: the CTA partition of the data, and with it every per-CTA partial, is the same whatever the batch.
 int launch_hyp_score(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, const HypArgs& h) {
-  const PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
-  PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
-  if (p->model >= MOPT_MODEL_USER_BASE)
-    return launch_user_hypothesis_score(L, ctx->device, p->model, st->dtype, p->compute_dtype, a, h);
-  return launch_hypothesis_score(L, p->model, st->dtype, p->compute_dtype, a, h);
+  KernelDesc k;
+  MOPT_TRY(p->model >= MOPT_MODEL_USER_BASE
+               ? user_kernel(ctx->device, p->model, KIND_HYP, st->dtype, p->compute_dtype, false, &k)
+               : hypothesis_score_kernel_desc(p->model, st->dtype, p->compute_dtype, &k));
+  const int grid = persistent_grid(k.occupancy, k.threads, pass_launch(ctx, p), h.count / store_vec(st->dtype) + 1);
+  PassArgs a = make_args(ctx, st, 0, 0, PASS_COST);
+  HypArgs ha = h;
+  void* params[] = {&a, &ha};
+  MOPT_CUDA_TRY(cudaLaunchKernel(k.fn, dim3(unsigned(grid), unsigned((h.n_hyp + kHypTile - 1) / kHypTile)),
+                                 dim3(unsigned(k.threads)), params, 0, ctx->stream));
+  return MOPT_OK;
 }
 
 // The buffers of mopt_score_hypotheses, on its first call on this context (the partials take 48 MB).
@@ -1128,10 +1173,8 @@ int mopt_lm_minimize(mopt_ctx* ctx, int n_costs, mopt_store* const* stores, cons
     }();
     const mopt_problem& p0 = problems[0];
     const bool moment_path = p0.model == MOPT_MODEL_POINT2POINT &&
-                             (p0.jacobian == MOPT_JAC_ANALYTICAL ||
-                              (!(p0.flags & MOPT_FLAG_GENERIC_KERNEL) && !(stores[0]->dtype == MOPT_F64 && p0.compute_dtype == MOPT_F32)));
-    if (n_costs == 1 && ctx->world == 1 && !has_update && !any_user_setup && moment_path && stores[0]->n <= mono_max &&
-        !(stores[0]->dtype == MOPT_F64 && p0.compute_dtype == MOPT_F32)) {
+                             (p0.jacobian == MOPT_JAC_ANALYTICAL || !(p0.flags & MOPT_FLAG_GENERIC_KERNEL));
+    if (n_costs == 1 && ctx->world == 1 && !has_update && !any_user_setup && moment_path && stores[0]->n <= mono_max) {
       PassArgs a = make_args(ctx, stores[0], 0, 0, -1);
       PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
       MonoArgs m;

@@ -1,8 +1,9 @@
-// Parameter covariance: instantiations + dispatch of the score Gram kernel (mopt_cov.cuh) for the builtin models,
-// and mopt_covariance_from_terms, the host-only fp64 finish (Jacobi eigensolver, truncated pseudo-inverse,
-// estimators).  mopt_covariance_terms itself lives in mopt_capi.cu next to the pass launcher it mirrors.
+// Parameter covariance: instantiations of the score Gram kernel (mopt_cov.cuh) for the builtin models, and
+// mopt_covariance_from_terms, the host-only fp64 finish (Jacobi eigensolver, truncated pseudo-inverse, estimators).
+// mopt_covariance_terms itself lives in mopt_capi.cu next to the pass launcher it mirrors.
 #include <cmath>
 #include <cstring>
+#include <type_traits>
 
 #include "mopt_cov.cuh"
 #include "mopt_internal.h"
@@ -10,69 +11,43 @@
 namespace mopt {
 namespace {
 
-// Does model M declare an affine first stage (NAFF / affine / finish / finish_diff)?  (as mopt_pass_dense.cu)
-template <class M, class = void>
-struct HasAffineStage { static constexpr bool value = false; };
-template <class M>
-struct HasAffineStage<M, decltype(void(M::NAFF))> { static constexpr bool value = true; };
-
 template <class M, typename ST, typename CT, int JAC>
-int launch_one(const PassLaunch& L, const PassArgs& a, const CovArgs& cv) {
-  auto kern = score_gram_kernel<M, ST, CT, JAC>;
-  // work items as the pass kernels count them: 16-byte groups (P <= 6), residuals (wide tier)
-  const int64_t items = (M::NS == 0) ? 1 : (M::P <= 6 ? a.n / VecOf<ST>::N : a.n);
-  PassLaunch L2 = L;
-  L2.ctas_per_sm = 0;
-  const int grid = pick_grid(reinterpret_cast<const void*>(kern), kCovThreads, L2, items);
-  kern<<<grid, kCovThreads, 0, L.stream>>>(a, cv);
-  MOPT_CUDA_TRY(cudaGetLastError());
+int gram_kernel(KernelDesc* k) {
+  *k = builtin_kernel(reinterpret_cast<const void*>(score_gram_kernel<M, ST, CT, JAC>), kCovThreads);
   return MOPT_OK;
 }
 
 // The Jacobian form of the linearization pass of the same problem (launch_pass, launch_dense, launch_wide).
 template <class M, typename ST, typename CT>
-int launch_form(const PassLaunch& L, int form, const PassArgs& a, const CovArgs& cv) {
-  if constexpr (M::P == 6 && M::O == 3 && M::NS == 6 && !M::HAS_JAC) {  // point2point
-    if (form == COV_JAC_P2P_AFFINE) return launch_one<M, ST, CT, COV_JAC_P2P_AFFINE>(L, a, cv);
+int gram_form(int form, bool affine_fd, KernelDesc* k) {
+  if constexpr (std::is_same_v<M, P2PModel>) {
+    if (form == COV_JAC_P2P_AFFINE) return gram_kernel<M, ST, CT, COV_JAC_P2P_AFFINE>(k);
   }
   if (form == COV_JAC_ANALYTICAL) {
-    if constexpr (M::HAS_JAC) return launch_one<M, ST, CT, COV_JAC_ANALYTICAL>(L, a, cv);
+    if constexpr (M::HAS_JAC) return gram_kernel<M, ST, CT, COV_JAC_ANALYTICAL>(k);
     set_last_error("this model has no analytical Jacobian");
     return MOPT_ERR_UNSUPPORTED;
   }
   if constexpr (HasAffineStage<M>::value) {
-    if (L.affine_fd) return launch_one<M, ST, CT, COV_JAC_AFFINE_FD>(L, a, cv);
+    if (affine_fd) return gram_kernel<M, ST, CT, COV_JAC_AFFINE_FD>(k);
   }
-  return launch_one<M, ST, CT, COV_JAC_FD>(L, a, cv);
-}
-
-template <class M>
-int launch_types(const PassLaunch& L, int form, int store_dtype, int compute_dtype, const PassArgs& a,
-                 const CovArgs& cv) {
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32) return launch_form<M, float, float>(L, form, a, cv);
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64) return launch_form<M, float, double>(L, form, a, cv);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64) return launch_form<M, double, double>(L, form, a, cv);
-  set_last_error("store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
+  return gram_kernel<M, ST, CT, COV_JAC_FD>(k);
 }
 
 }  // namespace
 
-int launch_cov(const PassLaunch& L, int model, int form, int store_dtype, int compute_dtype, const PassArgs& a,
-               const CovArgs& cv) {
-  switch (model) {
-    case MOPT_MODEL_POINT2POINT: return launch_types<P2PModel>(L, form, store_dtype, compute_dtype, a, cv);
-    case MOPT_MODEL_EXP_CURVE: return launch_types<ExpCurveModel>(L, form, store_dtype, compute_dtype, a, cv);
-    case MOPT_MODEL_MICHAELIS_MENTEN:
-      return launch_types<MichaelisMentenModel>(L, form, store_dtype, compute_dtype, a, cv);
-    case MOPT_MODEL_PINHOLE: return launch_types<PinholeModel>(L, form, store_dtype, compute_dtype, a, cv);
-    case MOPT_MODEL_POWELL: return launch_types<PowellModel>(L, form, store_dtype, compute_dtype, a, cv);
-    case MOPT_MODEL_PINHOLE_DISTORT:
-      return launch_types<PinholeDistortModel>(L, form, store_dtype, compute_dtype, a, cv);
-    default:
-      set_last_error("this model has no parameters: no covariance");
-      return MOPT_ERR_INVALID_ARGUMENT;
-  }
+int score_gram_kernel_desc(int model, int form, bool affine_fd, int store_dtype, int compute_dtype, KernelDesc* k) {
+  return with_builtin_model(model, [&](auto m) {
+    using M = decltype(m);
+    if constexpr (M::P == 0) {
+      set_last_error("internal error: no covariance for a model without parameters");
+      return MOPT_ERR_CUDA;
+    } else {
+      return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+        return gram_form<M, decltype(st), decltype(ct)>(form, affine_fd, k);
+      });
+    }
+  });
 }
 
 }  // namespace mopt

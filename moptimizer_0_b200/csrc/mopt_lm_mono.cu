@@ -52,11 +52,9 @@ int launch_mono_loss(const PassLaunch& L, int loss, bool qrot, const PassArgs& a
 
 int launch_p2p_lm_mono(const PassLaunch& L, int store_dtype, int compute_dtype, int loss, bool qrot, const PassArgs& a,
                        const MonoArgs& m) {
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32) return launch_mono_loss<float, float>(L, loss, qrot, a, m);
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64) return launch_mono_loss<float, double>(L, loss, qrot, a, m);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64) return launch_mono_loss<double, double>(L, loss, qrot, a, m);
-  set_last_error("point2point: store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
+  return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+    return launch_mono_loss<decltype(st), decltype(ct)>(L, loss, qrot, a, m);
+  });
 }
 
 

@@ -1,4 +1,4 @@
-// Instantiations + dispatch of the generic dense pass kernel (mopt_pass.cuh).
+// Instantiations + dispatch of the generic dense pass kernel (mopt_pass.cuh): models with at most 32 packed sums.
 #include "mopt_internal.h"
 #include "mopt_pass_dense_f2.cuh"
 
@@ -6,12 +6,6 @@ namespace mopt {
 namespace {
 
 constexpr int kThreads = 256;
-
-// Does model M declare an affine first stage (NAFF / affine / finish / finish_diff)?
-template <class M, class = void>
-struct HasAffineStage { static constexpr bool value = false; };
-template <class M>
-struct HasAffineStage<M, decltype(void(M::NAFF))> { static constexpr bool value = true; };
 
 template <class M, typename ST, typename CT, bool NUMERIC, int THREADS, int MINB, bool AFFINE_FD = false>
 int launch_shape(const PassLaunch& L, const PassArgs& a) {
@@ -70,39 +64,24 @@ int launch_one(const PassLaunch& L, const PassArgs& a) {
   return launch_shape<M, ST, CT, NUMERIC, kThreads, kMinB>(L, a);
 }
 
-template <class M, bool NUMERIC>
-int launch_types(const PassLaunch& L, int store_dtype, int compute_dtype, const PassArgs& a) {
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32) return launch_one<M, float, float, NUMERIC>(L, a);
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64) return launch_one<M, float, double, NUMERIC>(L, a);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64) return launch_one<M, double, double, NUMERIC>(L, a);
-  set_last_error("store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
-}
-
-template <class M>
-int launch_model(const PassLaunch& L, bool numeric, int store_dtype, int compute_dtype, const PassArgs& a) {
-  if (numeric) return launch_types<M, true>(L, store_dtype, compute_dtype, a);
-  if (!M::HAS_JAC) {
-    // cost-only passes of Jacobian-free models still come through here with numeric == false
-    return launch_types<M, true>(L, store_dtype, compute_dtype, a);
-  }
-  return launch_types<M, false>(L, store_dtype, compute_dtype, a);
-}
-
 }  // namespace
 
 int launch_dense(const PassLaunch& L, int model, bool numeric, int store_dtype, int compute_dtype, const PassArgs& a) {
-  switch (model) {
-    case MOPT_MODEL_POINT2POINT: return launch_model<P2PModel>(L, numeric, store_dtype, compute_dtype, a);
-    case MOPT_MODEL_EXP_CURVE: return launch_model<ExpCurveModel>(L, numeric, store_dtype, compute_dtype, a);
-    case MOPT_MODEL_MICHAELIS_MENTEN: return launch_model<MichaelisMentenModel>(L, numeric, store_dtype, compute_dtype, a);
-    case MOPT_MODEL_PINHOLE: return launch_model<PinholeModel>(L, numeric, store_dtype, compute_dtype, a);
-    case MOPT_MODEL_POWELL: return launch_model<PowellModel>(L, numeric, store_dtype, compute_dtype, a);
-    case MOPT_MODEL_POINT_DIST: return launch_model<PointDistModel>(L, true, store_dtype, compute_dtype, a);
-    default:
-      set_last_error("unknown model kind");
-      return MOPT_ERR_INVALID_ARGUMENT;
-  }
+  return with_builtin_model(model, [&](auto m) {
+    using M = decltype(m);
+    if constexpr (is_wide(M::P)) {
+      set_last_error("internal error: a wide model on the dense pass");
+      return MOPT_ERR_CUDA;
+    } else {
+      return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+        using ST = decltype(st);
+        using CT = decltype(ct);
+        // cost-only passes of Jacobian-free models still come through here with numeric == false
+        if (numeric || !M::HAS_JAC) return launch_one<M, ST, CT, true>(L, a);
+        return launch_one<M, ST, CT, false>(L, a);
+      });
+    }
+  });
 }
 
 }  // namespace mopt

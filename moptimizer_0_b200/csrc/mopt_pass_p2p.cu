@@ -53,14 +53,16 @@ int launch_loss(const PassLaunch& L, int loss, bool qrot, const PassArgs& a) {
 }  // namespace
 
 int launch_p2p_moment(const PassLaunch& L, int store_dtype, int compute_dtype, int loss, bool qrot, const PassArgs& a) {
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32) {
-    if (L.threads == 1024) return launch_loss<float, float, ShapeF32>(L, loss, qrot, a);  // first generation (A/B)
-    return launch_p2p_moment_gen2(L, loss, qrot, a);  // mopt_pass_p2p2.cu
-  }
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64) return launch_loss<float, double, ShapeF64>(L, loss, qrot, a);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64) return launch_loss<double, double, ShapeF64>(L, loss, qrot, a);
-  set_last_error("point2point: store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
+  return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+    using ST = decltype(st);
+    using CT = decltype(ct);
+    if constexpr (sizeof(CT) == 4) {
+      if (L.threads == 1024) return launch_loss<ST, CT, ShapeF32>(L, loss, qrot, a);  // first generation (A/B)
+      return launch_p2p_moment_gen2(L, loss, qrot, a);  // mopt_pass_p2p2.cu
+    } else {
+      return launch_loss<ST, CT, ShapeF64>(L, loss, qrot, a);
+    }
+  });
 }
 
 }  // namespace mopt

@@ -1,4 +1,4 @@
-// Instantiations + dispatch of the wide pass kernel (mopt_pass.cuh): models with more than 32 packed sums.
+// Instantiations + dispatch of the wide pass kernel (mopt_pass.cuh): models with more than 32 packed sums (is_wide).
 #include "mopt_internal.h"
 #include "mopt_pass_wide_tc.cuh"
 
@@ -34,35 +34,30 @@ int launch_tc(const PassLaunch& L, const PassArgs& a) {
   return MOPT_OK;
 }
 
-template <class M>
-int launch_types(const PassLaunch& L, int store_dtype, int compute_dtype, const PassArgs& a) {
-  // fp32 store + fp32 compute, common-denominator finite differences, C = I: the tensor-core kernel
-  // (mopt_ctx_set_launch(.., 1024) keeps the first-generation kernel for A/B on the same box)
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32 && L.affine_fd && L.identity_cov && !a.masked &&
-      L.threads != 1024)
-    return launch_tc<M>(L, a);
-  // L.affine_fd (launch_pass): common-denominator finite differences (wide_pass_kernel AFFINE_FD) — the default
-  // with fp32 compute unless MOPT_FLAG_GENERIC_KERNEL asks for the per-residual form; fp64 compute is the literal
-  // restatement of the reference unless MOPT_FLAG_STABLE_FD opts in
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32)
-    return L.affine_fd ? launch_one<M, float, float, true>(L, a) : launch_one<M, float, float, false>(L, a);
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64)
-    return L.affine_fd ? launch_one<M, float, double, true>(L, a) : launch_one<M, float, double, false>(L, a);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64)
-    return L.affine_fd ? launch_one<M, double, double, true>(L, a) : launch_one<M, double, double, false>(L, a);
-  set_last_error("store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
-}
-
 }  // namespace
 
 int launch_wide(const PassLaunch& L, int model, int store_dtype, int compute_dtype, const PassArgs& a) {
-  switch (model) {
-    case MOPT_MODEL_PINHOLE_DISTORT: return launch_types<PinholeDistortModel>(L, store_dtype, compute_dtype, a);
-    default:
-      set_last_error("unknown wide model kind");
-      return MOPT_ERR_INVALID_ARGUMENT;
-  }
+  return with_builtin_model(model, [&](auto m) {
+    using M = decltype(m);
+    if constexpr (!is_wide(M::P)) {
+      set_last_error("internal error: a dense model on the wide pass");
+      return MOPT_ERR_CUDA;
+    } else {
+      return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+        using ST = decltype(st);
+        using CT = decltype(ct);
+        // fp32 store + fp32 compute, common-denominator finite differences, C = I: the tensor-core kernel
+        // (mopt_ctx_set_launch(.., 1024) keeps the first-generation kernel for A/B on the same box)
+        if constexpr (sizeof(ST) == 4 && sizeof(CT) == 4) {
+          if (L.affine_fd && L.identity_cov && !a.masked && L.threads != 1024) return launch_tc<M>(L, a);
+        }
+        // L.affine_fd (launch_pass): common-denominator finite differences (wide_pass_kernel AFFINE_FD) — the default
+        // with fp32 compute unless MOPT_FLAG_GENERIC_KERNEL asks for the per-residual form; fp64 compute is the
+        // literal restatement of the reference unless MOPT_FLAG_STABLE_FD opts in
+        return L.affine_fd ? launch_one<M, ST, CT, true>(L, a) : launch_one<M, ST, CT, false>(L, a);
+      });
+    }
+  });
 }
 
 }  // namespace mopt

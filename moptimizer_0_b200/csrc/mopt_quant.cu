@@ -1,4 +1,4 @@
-// Instantiations + dispatch of the radix-select sweep (mopt_quant.cuh) for the builtin models, and the one-CTA step
+// Instantiations of the radix-select sweep (mopt_quant.cuh) for the builtin models, and the one-CTA step
 // between sweeps, which is the same for every model.
 #include "mopt_internal.h"
 #include "mopt_quant.cuh"
@@ -95,40 +95,16 @@ __global__ void __launch_bounds__(256) quantile_step_kernel(QuantState* st, int 
   }
 }
 
-template <class M, typename ST, typename CT>
-int launch_sweep(const PassLaunch& L, const PassArgs& a, const QuantArgs& qa) {
-  auto k = quantile_sweep_kernel<M, ST, CT>;
-  const int grid = pick_grid(reinterpret_cast<const void*>(k), kQuantThreads, L, qa.count / VecOf<ST>::N + 1);
-  k<<<grid, kQuantThreads, 0, L.stream>>>(a, qa);
-  MOPT_CUDA_TRY(cudaGetLastError());
-  return MOPT_OK;
-}
-
-template <class M>
-int launch_types(const PassLaunch& L, int store_dtype, int compute_dtype, const PassArgs& a, const QuantArgs& qa) {
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F32) return launch_sweep<M, float, float>(L, a, qa);
-  if (store_dtype == MOPT_F32 && compute_dtype == MOPT_F64) return launch_sweep<M, float, double>(L, a, qa);
-  if (store_dtype == MOPT_F64 && compute_dtype == MOPT_F64) return launch_sweep<M, double, double>(L, a, qa);
-  set_last_error("store dtype f64 with compute dtype f32 is not supported");
-  return MOPT_ERR_UNSUPPORTED;
-}
-
 }  // namespace
 
-int launch_quantile_sweep(const PassLaunch& L, int model, int store_dtype, int compute_dtype, const PassArgs& a,
-                          const QuantArgs& qa) {
-  switch (model) {
-    case MOPT_MODEL_POINT2POINT: return launch_types<P2PModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_EXP_CURVE: return launch_types<ExpCurveModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_MICHAELIS_MENTEN: return launch_types<MichaelisMentenModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_PINHOLE: return launch_types<PinholeModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_POWELL: return launch_types<PowellModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_POINT_DIST: return launch_types<PointDistModel>(L, store_dtype, compute_dtype, a, qa);
-    case MOPT_MODEL_PINHOLE_DISTORT: return launch_types<PinholeDistortModel>(L, store_dtype, compute_dtype, a, qa);
-    default:
-      set_last_error("unknown model kind");
-      return MOPT_ERR_INVALID_ARGUMENT;
-  }
+int quantile_sweep_kernel_desc(int model, int store_dtype, int compute_dtype, KernelDesc* k) {
+  return with_builtin_model(model, [&](auto m) {
+    return with_dtypes(store_dtype, compute_dtype, [&](auto st, auto ct) {
+      *k = builtin_kernel(
+          reinterpret_cast<const void*>(quantile_sweep_kernel<decltype(m), decltype(st), decltype(ct)>), kQuantThreads);
+      return MOPT_OK;
+    });
+  });
 }
 
 int launch_quantile_step(cudaStream_t stream, QuantState* st, int sweep, int n_q, const QuantLevels& lv) {
