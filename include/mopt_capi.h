@@ -433,6 +433,73 @@ MOPT_API int mopt_covariance_terms(mopt_ctx* ctx, int n_costs, mopt_store* const
 MOPT_API int mopt_covariance_from_terms(const mopt_cov_terms* terms, int estimator, double rcond, double* cov,
                                         mopt_cov_report* report);
 
+/* ---- closed-form rigid alignment -------------------------------------------------------------- */
+/* The best rigid transform for the correspondences a point2point store holds: the weighted Kabsch / Horn solution.
+ * Two calls, as for the covariance: mopt_align_terms streams the store once on the device and returns the weighted
+ * first and second moments of the pairs it uses; mopt_align_from_terms (host only) solves for x = [t, omega].  Terms
+ * of several ranges or of the ranks of a sharded problem combine with mopt_align_terms_merge, not field by field. */
+typedef struct mopt_align_moments { /* the terms: combine with mopt_align_terms_merge, NOT by adding fields */
+  int64_t n_valid;     /* elements of the range with a correspondence: mopt_evaluate's n_valid */
+  int64_t n_used;      /* valid elements with double(e2(x)) <= thr^2: mopt_evaluate's n_inliers; they enter the moments */
+  double w;            /* sum of w_i over used elements */
+  double mean_src[3];  /* weighted mean of p (group A) */
+  double mean_tgt[3];  /* weighted mean of q (group B) */
+  double cross[9];     /* cross[3a+b] = sum w (p_a - mean_src_a)(q_b - mean_tgt_b) */
+  double var_src;      /* sum w |p - mean_src|^2 */
+  double var_tgt;      /* sum w |q - mean_tgt|^2 */
+  double reserved[4];
+} mopt_align_moments;
+
+typedef struct mopt_align_report {
+  double cost;         /* sum w |R p + t - q|^2 at the solution = max(0, var_src + var_tgt - 2 eig[0]) */
+  double rms;          /* sqrt(cost / w) */
+  double eig[4];       /* eigenvalues of Horn's 4x4 matrix N, descending */
+  int32_t degenerate;  /* eig[0] - eig[1] <= 1e-12 * |eig[0]|: rotation not unique (collinear / < 3 distinct points) */
+  int32_t reserved0;
+  double reserved[3];
+} mopt_align_report;
+
+/* Alignment terms of the elements [first, first + count) of a MOPT_MODEL_POINT2POINT store at x (host pointer), on
+ * the device.  Returns after the context stream is synchronised.
+ *   - Which elements enter.  Element i is used when it has a correspondence and double(e2_i) <= inlier_threshold^2,
+ *     e2_i = sum fma(r_o, r_o) of the residual on set 0 in problem.compute_dtype at x: mopt_evaluate's inlier test,
+ *     so n_valid and n_used equal mopt_evaluate's n_valid and n_inliers bit for bit.  NaN data and NaN keys never
+ *     enter.  inlier_threshold = +inf takes every valid element.
+ *   - Weights.  w_i is the loss weight of e2_i in the compute dtype (what mopt_evaluate writes to `weights` with
+ *     out_dtype = compute_dtype), converted to fp64; MOPT_LOSS_NONE gives w = 1.  With a robust loss one call and one
+ *     solve are one IRLS step of the robust closed-form fit.
+ *   - Moments of the store values p_i, q_i (converted exactly to fp64), not of T(x) p_i, accumulated in fp64 in
+ *     centred form and combined in a fixed order: identical bits from run to run for the same launch settings, equal
+ *     to rounding under another mopt_ctx_set_launch.  They stay accurate on clouds far from the origin.
+ *   - The covariance, jacobian, variant and manifold fields have no effect.  Correspondences are never re-associated:
+ *     call mopt_store_reassociate(store, x) first for fresh ones.
+ *   - Sharded contexts: this rank's store only, no collective (merge the ranks' terms with mopt_align_terms_merge).
+ *   - count = 0 gives all-zero terms.
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for a store whose model is not point2point, a store of another
+ * context, a problem the store does not accept, a range outside the store, a NaN or negative inlier_threshold, or a
+ * null x or out. */
+MOPT_API int mopt_align_terms(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const double* x,
+                              int64_t first, int64_t count, double inlier_threshold, mopt_align_moments* out);
+/* Host only: the terms of the union of two disjoint sets of pairs (Chan's pairwise rule: counts and w add, means
+ * combine by weight, cross and var gain Wa Wb / W d_src d_tgt^T with d the difference of the means).  merge(a, b) and
+ * merge(b, a) are identical bits; an operand with w = 0 leaves the other's moments unchanged (its counts still add).
+ * `out` may alias `a` or `b`.  Accuracy: each mean of the struct is one double, so far from the origin it carries up to
+ * half an ulp of rounding (6e-11 at 1e6), which the merge takes into cross and var at first order.  For a cloud 1e6 from
+ * the origin with unit spread, merged terms agree with one-shot moments to about 1e-12 of the largest moment after one
+ * merge and 8e-12 after 63 (1e-15 near the origin), so fold few terms, such as one per rank.  mopt_align_terms itself
+ * carries each mean's rounding error through its device reduction and does not have this loss.
+ * MOPT_ERR_INVALID_ARGUMENT for a null argument. */
+MOPT_API int mopt_align_terms_merge(const mopt_align_moments* a, const mopt_align_moments* b,
+                                   mopt_align_moments* out);
+/* Host only, needs no GPU: Horn's quaternion solution of min sum w |R p + t - q|^2 from terms.  N (4x4 symmetric) is
+ * built from `cross`, the eigenvector of its largest eigenvalue (cyclic Jacobi in fp64) is the rotation as a unit
+ * quaternion (w >= 0), t = mean_tgt - R mean_src and omega = 2 atan2(|v|, w) v / |v| (|omega| <= pi).  x_out = [t, omega]
+ * (6 doubles) is the point2point parameter vector: a start for mopt_lm_minimize or a hypothesis for
+ * mopt_score_hypotheses.  R is always a proper rotation.  `report` may be NULL.  A degenerate configuration returns
+ * MOPT_OK with one of the minimisers and report->degenerate = 1.
+ * MOPT_ERR_INVALID_ARGUMENT, with nothing written, for a null terms or x_out, w <= 0 or non-finite terms. */
+MOPT_API int mopt_align_from_terms(const mopt_align_moments* terms, double* x_out, mopt_align_report* report);
+
 /* End-to-end convenience: upload host AoS data (group A and B) into `store` and linearize, with the
  * host->device copies chunked and overlapped with the device work. */
 MOPT_API int mopt_upload_and_linearize(mopt_ctx* ctx, mopt_store* store, const mopt_problem* problem, const void* host_a,

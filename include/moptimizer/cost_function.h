@@ -119,6 +119,22 @@ class CostFunctionBase {
     return terms;
   }
 
+  /// New: closed-form rigid alignment terms of this point2point cost at x (mopt_align_terms): the weighted moments of
+  /// the source and target points of every residual with r^T r <= inlier_threshold^2, weighted by the loss weight at
+  /// x.  Fold terms with mopt_align_terms_merge and solve with mopt_align_from_terms, which returns x = [t, omega].
+  /// Correspondences are not re-associated: call update(x) first for fresh ones.
+  mopt_align_moments alignmentTerms(const Scalar* x, double inlier_threshold) const {
+    mopt_problem p;
+    device::Store::Ptr st;
+    deviceProblem(&p, &st);
+    double xd[MOPT_MAX_PARAMETERS] = {0};
+    for (int i = 0; i < p.num_parameters && x; ++i) xd[i] = double(x[i]);
+    mopt_align_moments terms;
+    device::check(mopt_align_terms(st->context()->get(), st->get(), &p, xd, 0, st->size(), inlier_threshold, &terms),
+                  "mopt_align_terms");
+    return terms;
+  }
+
  protected:
   void fillDeviceProblem(int num_parameters, int num_outputs, int jacobian, mopt_problem* p,
                          device::Store::Ptr* store) const {

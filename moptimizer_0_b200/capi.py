@@ -50,7 +50,8 @@ EXPORTS = [
     "mopt_ctx_peer_handle", "mopt_ctx_open_peers", "mopt_ctx_set_exchange_enabled",
     "mopt_user_model_compile", "mopt_user_model_release", "mopt_user_model_log",
     "mopt_measure_peaks", "mopt_measure_h2d", "mopt_evaluate", "mopt_covariance_terms", "mopt_covariance_from_terms",
-    "mopt_residual_quantiles", "mopt_score_hypotheses",
+    "mopt_residual_quantiles", "mopt_score_hypotheses", "mopt_align_terms", "mopt_align_terms_merge",
+    "mopt_align_from_terms",
 ]
 MODEL_USER_BASE = 1000
 PEER_HANDLE_BYTES = 64
@@ -242,6 +243,62 @@ def covariance_from_terms(terms: CovTerms, estimator: int = COV_SCALED, rcond: f
     return Covariance(cov[:P * P].reshape(P, P).T.copy(), rep)
 
 
+class AlignMomentsStruct(C.Structure):
+    _fields_ = [("n_valid", C.c_int64), ("n_used", C.c_int64), ("w", C.c_double), ("mean_src", C.c_double * 3),
+                ("mean_tgt", C.c_double * 3), ("cross", C.c_double * 9), ("var_src", C.c_double),
+                ("var_tgt", C.c_double), ("reserved", C.c_double * 4)]
+
+
+class AlignReport(C.Structure):
+    _fields_ = [("cost", C.c_double), ("rms", C.c_double), ("eig", C.c_double * 4), ("degenerate", C.c_int32),
+                ("reserved0", C.c_int32), ("reserved", C.c_double * 3)]
+
+
+mopt_align_moments, mopt_align_report = AlignMomentsStruct, AlignReport  # the C names
+
+
+class AlignTerms:
+    """mopt_align_moments with numpy views: `mean_src`, `mean_tgt` (3), `cross` (3 x 3, source rows, target columns)
+    and the scalars.  Terms of disjoint ranges or of the ranks of a sharded problem combine with `+`
+    (mopt_align_terms_merge), in a fixed order for identical bits."""
+
+    def __init__(self, raw: Optional[AlignMomentsStruct] = None):
+        self.raw = raw if raw is not None else AlignMomentsStruct()
+
+    n_valid = property(lambda self: self.raw.n_valid)
+    n_used = property(lambda self: self.raw.n_used)
+    w = property(lambda self: self.raw.w)
+    mean_src = property(lambda self: np.ctypeslib.as_array(self.raw.mean_src))
+    mean_tgt = property(lambda self: np.ctypeslib.as_array(self.raw.mean_tgt))
+    cross = property(lambda self: np.ctypeslib.as_array(self.raw.cross).reshape(3, 3))
+    var_src = property(lambda self: self.raw.var_src)
+    var_tgt = property(lambda self: self.raw.var_tgt)
+
+    def __add__(self, other: "AlignTerms") -> "AlignTerms":
+        out = AlignMomentsStruct()
+        check(lib().mopt_align_terms_merge(C.byref(self.raw), C.byref(other.raw), C.byref(out)))
+        return AlignTerms(out)
+
+
+class Alignment:
+    """align_from_terms / Context.align: `x` = [t, omega] (the point2point parameter vector), `cost` = sum w |R p + t - q|^2
+    at x, `rms`, `eig` (Horn's N, descending) and `degenerate`."""
+
+    def __init__(self, x: np.ndarray, rep: AlignReport):
+        self.x = x
+        self.cost, self.rms = rep.cost, rep.rms
+        self.eig = np.array(rep.eig[:], dtype=np.float64)
+        self.degenerate = bool(rep.degenerate)
+
+
+def align_from_terms(terms: AlignTerms) -> Alignment:
+    """mopt_align_from_terms (host only): Horn's closed-form rigid transform from (merged) terms."""
+    x = np.zeros(6, dtype=np.float64)
+    rep = AlignReport()
+    check(lib().mopt_align_from_terms(C.byref(terms.raw), _dp(x), C.byref(rep)))
+    return Alignment(x, rep)
+
+
 class MoptError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"mopt error {code}: {msg}")
@@ -290,6 +347,11 @@ def lib():
                                             C.POINTER(CovTermsStruct)]
         L.mopt_covariance_from_terms.argtypes = [C.POINTER(CovTermsStruct), C.c_int, C.c_double, dp,
                                                  C.POINTER(CovReport)]
+        L.mopt_align_terms.argtypes = [vp, vp, C.POINTER(Problem), dp, i64, i64, C.c_double,
+                                       C.POINTER(AlignMomentsStruct)]
+        L.mopt_align_terms_merge.argtypes = [C.POINTER(AlignMomentsStruct), C.POINTER(AlignMomentsStruct),
+                                             C.POINTER(AlignMomentsStruct)]
+        L.mopt_align_from_terms.argtypes = [C.POINTER(AlignMomentsStruct), dp, C.POINTER(AlignReport)]
         L.mopt_measure_h2d.argtypes = [vp, C.c_uint64, C.c_double, dp]
         L.mopt_upload_and_linearize.argtypes = [vp, vp, C.POINTER(Problem), vp, vp, C.c_int, i64, dp, dp, dp, dp]
         L.mopt_lm_minimize.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(Problem), C.POINTER(LmOptions), dp,
@@ -543,6 +605,24 @@ class Context:
         """Covariance of x (`.cov`, `.std`, `.rank`, `.dof`, `.sigma2`) from this context's stores: the terms on the
         device, then mopt_covariance_from_terms."""
         return covariance_from_terms(self.covariance_terms(stores, problems, x), estimator, rcond)
+
+    def align_terms(self, store: "Store", problem: Problem, x, inlier_threshold: float = np.inf, first: int = 0,
+                    count: Optional[int] = None) -> AlignTerms:
+        """mopt_align_terms: weighted moments of the source and target points of the elements [first, first + count)
+        of a point2point store that mopt_evaluate counts as inliers at x, each weighted by its loss weight at x.  This
+        context's store only; never re-associates."""
+        count = store.n - first if count is None else int(count)
+        xs = np.ascontiguousarray(np.asarray(x, dtype=np.float64))
+        out = AlignMomentsStruct()
+        check(lib().mopt_align_terms(self._h, store.handle, C.byref(problem), _dp(xs), int(first), count,
+                                     float(inlier_threshold), C.byref(out)))
+        return AlignTerms(out)
+
+    def align(self, store: "Store", problem: Problem, x, inlier_threshold: float = np.inf, first: int = 0,
+              count: Optional[int] = None) -> Alignment:
+        """The closed-form rigid transform (`.x`, `.cost`, `.rms`) of the pairs align_terms selects: the terms on the
+        device, then mopt_align_from_terms."""
+        return align_from_terms(self.align_terms(store, problem, x, inlier_threshold, first, count))
 
     def linearize_async(self, store: "Store", problem: Problem, xs: np.ndarray):
         check(lib().mopt_linearize_async(self._h, store.handle, C.byref(problem), _dp(xs)))

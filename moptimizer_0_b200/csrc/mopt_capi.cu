@@ -174,6 +174,10 @@ int rot_offset(int model) {
                                                                                                                : -1;
 }
 
+}  // namespace
+
+namespace mopt {
+
 int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_linearize) {
   MOPT_REQUIRE(st && p, "null store/problem");
   MOPT_REQUIRE(p->model == st->model, "problem.model differs from the store's model");
@@ -214,6 +218,10 @@ int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_line
   return MOPT_OK;
 }
 
+}  // namespace mopt
+
+namespace {
+
 void fill_cost(const mopt_problem* p, CostDev* c) {
   std::memset(c, 0, sizeof(*c));
   c->model = p->model; c->variant = p->variant; c->P = p->num_parameters; c->O = p->num_outputs;
@@ -242,6 +250,10 @@ int stage_cost(mopt_ctx* ctx, int i, const mopt_problem* p) {
   return MOPT_OK;
 }
 
+}  // namespace
+
+namespace mopt {
+
 PassArgs make_args(mopt_ctx* ctx, const mopt_store* st, int slot, int accumulate, int mode_override) {
   PassArgs a;
   std::memset(&a, 0, sizeof(a));
@@ -258,6 +270,10 @@ PassArgs make_args(mopt_ctx* ctx, const mopt_store* st, int slot, int accumulate
   a.masked = st->may_have_invalid ? 1 : 0;
   return a;
 }
+
+}  // namespace mopt
+
+namespace {
 
 // `push`: this pass completes the rank-local result (last cost term), so its last CTA also pushes the packed
 // result to every peer when the NVLink exchange is open.
@@ -284,6 +300,10 @@ bool can_fuse_setup(const mopt_ctx* ctx, const mopt_problem* p, const mopt_store
          p->manifold == MOPT_MANIFOLD_ADDITIVE;
 }
 
+}  // namespace
+
+namespace mopt {
+
 PassLaunch pass_launch(const mopt_ctx* ctx, const mopt_problem* p) {
   PassLaunch L{ctx->stream, ctx->num_sms, ctx->ctas_per_sm, ctx->threads};
   // finite differences over a common denominator (AFFINE_FD): the default with fp32 compute, opt-in with fp64
@@ -292,6 +312,10 @@ PassLaunch pass_launch(const mopt_ctx* ctx, const mopt_problem* p) {
   L.identity_cov = !p->has_covariance;
   return L;
 }
+
+}  // namespace mopt
+
+namespace {
 
 int launch_pass(mopt_ctx* ctx, const mopt_store* st, const mopt_problem* p, int slot, int accumulate, int mode_override,
                 bool push, const XArg* fused_x = nullptr) {
@@ -604,6 +628,7 @@ int ctx_alloc(mopt_ctx* ctx) {
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_xerr_dev, sizeof(int)));
   MOPT_CUDA_TRY(cudaMemset(ctx->d_xerr_dev, 0, sizeof(int)));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_eval_stats, sizeof(double) * (kEvalSums + 1)));
+  MOPT_CUDA_TRY(cudaMalloc(&ctx->d_align, sizeof(AlignAcc)));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw));
   MOPT_CUDA_TRY(cudaHostAlloc(&ctx->h_cov_sums, sizeof(double) * MOPT_MAX_COSTS * kMaxRaw, cudaHostAllocDefault));
   MOPT_CUDA_TRY(cudaMalloc(&ctx->d_quant, sizeof(QuantState)));
@@ -707,6 +732,7 @@ int mopt_ctx_destroy(mopt_ctx* ctx) try {
   cudaFree(ctx->d_xerr_dev);
   cudaFree(ctx->d_gen);
   cudaFree(ctx->d_eval_stats);
+  cudaFree(ctx->d_align);
   cudaFree(ctx->d_cov_sums);
   cudaFree(ctx->d_quant);
   cudaFree(ctx->d_hyp_x);

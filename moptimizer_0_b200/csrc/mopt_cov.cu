@@ -50,13 +50,9 @@ int score_gram_kernel_desc(int model, int form, bool affine_fd, int store_dtype,
   });
 }
 
-}  // namespace mopt
-
-namespace {
-
 // Cyclic Jacobi eigendecomposition of the symmetric n x n matrix A (column-major, overwritten): on return the
 // diagonal of A holds the eigenvalues and the columns of V the eigenvectors.  Sweeps until the off-diagonal mass is
-// below 1e-30 of the total (fp64 rounding level), at most 100 sweeps.
+// below 1e-30 of the total (fp64 rounding level), at most 100 sweeps.  Also Horn's solve (mopt_align.cu).
 void jacobi_eigen(int n, double* A, double* V) {
   auto a = [&](int r, int c) -> double& { return A[r + c * n]; };
   for (int i = 0; i < n * n; ++i) V[i] = (i % (n + 1) == 0) ? 1.0 : 0.0;
@@ -94,7 +90,7 @@ void jacobi_eigen(int n, double* A, double* V) {
   }
 }
 
-}  // namespace
+}  // namespace mopt
 
 extern "C" {
 
@@ -122,7 +118,7 @@ int mopt_covariance_from_terms(const mopt_cov_terms* terms, int estimator, doubl
   }
   for (int c = 0; c < P; ++c)
     for (int r = 0; r < P; ++r) S[r + c * P] = d[r] * (0.5 * (terms->H[r + c * P] + terms->H[c + r * P])) * d[c];
-  jacobi_eigen(P, S, V);
+  mopt::jacobi_eigen(P, S, V);
   double lmax = 0.0;
   for (int i = 0; i < P; ++i) lmax = std::fmax(lmax, S[i + i * P]);
   int rank = 0;

@@ -3,6 +3,7 @@
 
 #include <cuda_runtime.h>
 
+#include "mopt_align.cuh"
 #include "mopt_common.cuh"
 #include "mopt_cov.cuh"
 #include "mopt_eval.cuh"
@@ -59,6 +60,7 @@ struct mopt_ctx {
   unsigned long long mono_gen = 0;               // barrier targets handed out so far (monotonic over the context's life)
   int* d_xerr_dev = nullptr;                     // device-resident copy, read by the kernels that follow a failed exchange
   double* d_eval_stats = nullptr;                // mopt_evaluate: the statistics written by the evaluation kernel's last CTA
+  double* d_align = nullptr;                     // mopt_align_terms: the terms (an AlignAcc) written by its last CTA
   double* d_cov_sums = nullptr;                  // mopt_covariance_terms: [MOPT_MAX_COSTS][kMaxRaw] score Gram totals
   double* h_cov_sums = nullptr;                  // pinned host copy of the same
   mopt::QuantState* d_quant = nullptr;           // mopt_residual_quantiles: histogram, prefixes and selected keys
@@ -188,6 +190,12 @@ int launch_dense(const PassLaunch& L, int model, bool numeric, int store_dtype, 
 
 // mopt_capi.cu: copy the cost constants of `problem` into slot `slot` and run model setup at x on the device
 int setup_slot(mopt_ctx* ctx, int slot, const mopt_problem* problem, const double* x);
+// mopt_capi.cu: does `st` accept `p` (and, with need_linearize, can it be linearized)?  Sets the last error if not.
+int validate_problem(const mopt_store* st, const mopt_problem* p, bool need_linearize);
+// mopt_capi.cu: the kernel arguments of a pass over `st` with the constants of cost slot `slot`
+PassArgs make_args(mopt_ctx* ctx, const mopt_store* st, int slot, int accumulate, int mode_override);
+// mopt_capi.cu: the launch settings of the context for problem `p`
+PassLaunch pass_launch(const mopt_ctx* ctx, const mopt_problem* p);
 // mopt_icp.cu: enqueue model->update(x) for a store with a target index (no-op without one)
 int enqueue_reassociate(mopt_store* st, const ParamBlock* pb, const LmState* gate);
 
@@ -205,6 +213,12 @@ int launch_quantile_step(cudaStream_t stream, QuantState* st, int sweep, int n_q
 // mopt_hyp.cu: set 0 of n hypotheses (xs [n][kMaxP] -> sets [n][kSetSize]) and their scores (mopt_score_hypotheses)
 int launch_hypothesis_setup(cudaStream_t stream, const CostDev* c, const double* xs, int n, double* sets);
 int hypothesis_score_kernel_desc(int model, int store_dtype, int compute_dtype, KernelDesc* k);
+// mopt_align.cu: the moments of a point2point store (mopt_align_terms); no other model has them
+int align_kernel_desc(int store_dtype, int compute_dtype, KernelDesc* k);
+
+// mopt_cov.cu: cyclic Jacobi eigendecomposition of the symmetric n x n column-major A (overwritten): on return the
+// diagonal of A holds the eigenvalues (unsorted) and the columns of V the eigenvectors
+void jacobi_eigen(int n, double* A, double* V);
 
 // mopt_rtc.cu: run-time compiled user models (ids >= MOPT_MODEL_USER_BASE)
 int launch_user(const PassLaunch& L, int device, int model, bool numeric, int store_dtype, int compute_dtype,
